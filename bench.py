@@ -5,6 +5,7 @@ iterations/s and E0 time-to-solution ride along as extra keys).
   python bench.py --gpus 1 --steps K --warmup W                       our arm, one GPU
   torchrun ... bench.py --gpus N --steps K --warmup W                  our arm, H row-sharded over N GPUs (strong scaling)
   python bench.py --impl reference --gpus N --steps K --warmup W       the reference's CPU implementation (oracle/_ref)
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    also write what the last timed step computed (dump_outputs)
 
 A step is one product y = H x (csr_mat::MultMv) on the workload named in config.workload.  Default workload =
 BASELINE config 3, Fermi-Hubbard 4x4, N_up = N_dn = 8 (dim 165,636,900; 5.82e9 stored entries), generated directly in
@@ -24,6 +25,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                  # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 if os.environ.get("NCCL_DEBUG", "VERSION").upper() == "VERSION":
     os.environ["NCCL_DEBUG"] = "WARN"          # keep NCCL's version banner off stdout: rank 0 prints ONE JSON line
 
@@ -153,6 +155,24 @@ class ClockSampler:
 def algorithmic_bytes(nnz, nrows_local, n, s_val, s_vec):
     """B_spmv = Z*(S_val+4) + 8*(rows+1) + (n + rows)*S_vec  (SURVEY section 8d; one compulsory read of x, one write of y)."""
     return nnz * (s_val + 4) + 8 * (nrows_local + 1) + (n + nrows_local) * s_vec
+
+
+DUMP_ROWS = 1 << 21                 # rows of y written by --dump-outputs: 3 float64 arrays of at most 2 M entries = 48 MB
+DUMP_SEED = 20261020
+
+
+def dump_outputs(dirpath, y):
+    """What a caller of the timed step receives: y = H x (complex128, the reference's order).  Written as DIR/y_rows.npy (row
+    indices), DIR/y_real.npy and DIR/y_imag.npy, all float64: every row when dim <= DUMP_ROWS, else the rows drawn with the fixed
+    seed DUMP_SEED (the same rows for every build of the same workload), so two builds can be compared output for output."""
+    import numpy as np
+    n = y.n
+    rows = np.arange(n) if n <= DUMP_ROWS else np.unique(np.random.default_rng(DUMP_SEED).integers(0, n, size=DUMP_ROWS, dtype=np.int64))
+    ys = y.to_numpy()[rows]
+    os.makedirs(dirpath, exist_ok=True)
+    np.save(os.path.join(dirpath, "y_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(dirpath, "y_real.npy"), np.ascontiguousarray(ys.real))
+    np.save(os.path.join(dirpath, "y_imag.npy"), np.ascontiguousarray(ys.imag))
 
 
 # ------------------------------------------------------------------------------------------------ reference arm
@@ -518,13 +538,20 @@ def main():
                          "QBGPU_SPECIES_ORDER handle: same entries, same 12 bytes each, two passes); ordinary = the one-pass "
                          "sliced-jagged handle in the reference's order; species-matfree = nothing stored.  Same operator, same "
                          "calling convention everywhere: complex128 device vectors in the reference's order through MultMv")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one GPU, our arm: after the timed steps write y = H x of the last one to DIR as .npy (float64; a fixed, "
+                         "seeded sample of rows when the workload has more than %d)" % DUMP_ROWS)
     ap.add_argument("--species-probe", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.species_probe:
         return species_probe(args)
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs writes the products of our arm on one GPU")
 
     if args.impl == "reference":
         if rank == 0:
@@ -598,6 +625,8 @@ def main():
     per_step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = sum(per_step_ms)
     clocks = sampler.stop()
+    if args.dump_outputs:                                   # before any later leg reuses y
+        dump_outputs(args.dump_outputs, y)
     ms_per_step = total_ms / args.steps
     value = 1e3 / ms_per_step
     peak, peak_src = measured_peak()

@@ -18,7 +18,7 @@ def _run(args, timeout=900):
 
 def test_reference_arm_prints_one_contract_line(oracle):
     if not oracle.have_qb_ref():
-        pytest.skip("oracle/_ref/qb_ref is not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/qb_ref is not built (needs the reference's sources at build time)")
     r = _run(["--impl", "reference", "--steps", "2", "--warmup", "1", "--workload", "heis_chain20"])
     assert r.returncode == 0, r.stderr[-500:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
@@ -39,6 +39,42 @@ def test_our_arm_needs_a_device_and_has_no_fallback():
     assert r.returncode != 0
     assert "CUDA" in (r.stderr + r.stdout)
     assert not any(ln.startswith("{") for ln in r.stdout.splitlines())   # no number is printed
+
+
+def test_steps_below_one_are_refused():
+    r = _run(["--steps", "0", "--warmup", "1", "--workload", "heis_chain20", "--no-cpu", "--no-lanczos"], timeout=300)
+    assert r.returncode != 0 and "--steps" in r.stderr
+    assert not any(ln.startswith("{") for ln in r.stdout.splitlines())
+
+
+def test_dump_outputs_writes_a_fixed_bounded_sample_of_y(tmp_path, monkeypatch):
+    """--dump-outputs: y of the last timed step as float64 .npy files, every row of a small workload, a seeded sample of a large
+    one (the same rows on every run), at most 64 MB in all."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    assert 3 * 8 * bench.DUMP_ROWS <= 64 << 20
+
+    class HostY:                                                       # the two members of DeviceVector the dump reads
+        def __init__(self, n):
+            self.n = n
+            self.v = np.arange(n) * (1.0 - 0.5j)
+
+        def to_numpy(self):
+            return self.v.copy()
+
+    def dump(d, n):
+        bench.dump_outputs(str(d), HostY(n))
+        z = {k: np.load(str(d / f"y_{k}.npy")) for k in ("rows", "real", "imag")}
+        assert all(a.dtype == np.float64 and a.shape == z["rows"].shape for a in z.values())
+        assert np.array_equal(z["real"], z["rows"]) and np.array_equal(z["imag"], -0.5 * z["rows"])
+        return z["rows"]
+
+    assert np.array_equal(dump(tmp_path / "small", 1000), np.arange(1000))
+    monkeypatch.setattr(bench, "DUMP_ROWS", 500)
+    rows = dump(tmp_path / "a", 100000)
+    assert 400 < rows.size <= 500 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(rows, dump(tmp_path / "b", 100000))
 
 
 def test_byte_formulas_match_the_survey():
@@ -65,8 +101,10 @@ def test_cpu_baseline_sample_is_the_same_lattice_and_bounded(oracle):
     args, desc = bench.cpu_baseline_sample("hubbard4x3")
     assert args == ["hubbard_direct", 4, 3, 6, 6, 1.0, 1.1] and "fewer" not in desc
     assert bench.cpu_baseline_sample("heis_chain32_k0")[0] == ["heis_chain_k", 20, 0, 0]
-    if not oracle.have_qb_ref():
-        pytest.skip("oracle/_ref/qb_ref is not built (needs /root/reference at build time)")
+    if not oracle.have_qb_ref():                                       # no reference build: the leg says so instead of raising
+        r = bench.cpu_baseline_leg("hubbard4x3", reps=2, warm=1)
+        assert r["value"] is None and r["kind"] == "reference" and "not built" in r["sample"]
+        return
     r = bench.cpu_baseline_leg("hubbard4x3", reps=2, warm=1)          # its own sample: nothing scaled
     assert r["kind"] == "reference" and r["value"] > 0 and r["scaled_by_stored_entries"] == 1.0 and "scaled x" not in r["sample"]
     assert abs(r["value"] - 1e3 / r["sample_ms_per_product"]) < 1e-9 * r["value"]

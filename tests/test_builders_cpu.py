@@ -19,7 +19,7 @@ def test_hubbard4x2_is_bit_identical_to_reference(oracle):
 ])
 def test_against_live_reference(oracle, args, mk, tmp_path):
     if not oracle.have_qb_ref():
-        pytest.skip("oracle/_ref/qb_ref not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/qb_ref not built (needs the reference's sources at build time)")
     f = str(tmp_path / "H.qbcsr")
     oracle.run_qb_ref(args + ["--dump", f], workdir=str(tmp_path))
     A = oracle.read_qbcsr(f)

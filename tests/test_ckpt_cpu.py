@@ -21,10 +21,13 @@ MAXIT = 200
 PREC = 2e-12
 
 
+def _needs_qb_ref(oracle):
+    if not oracle.have_qb_ref():
+        pytest.skip("oracle/_ref/qb_ref is not built (needs the reference's sources at build time)")
+
+
 @pytest.fixture(scope="module")
 def case(oracle):
-    if not oracle.have_qb_ref():
-        pytest.skip("oracle/_ref/qb_ref is not built (needs /root/reference at build time)")
     A, meta, ex = oracle.load_golden("heis12_full")
     work = tempfile.mkdtemp(prefix="qb_ckpt_")
     path = os.path.join(work, "A.qbcsr")
@@ -61,6 +64,7 @@ def _numpy_resume(oracle, A, k, v, hess, state, maxit):
 
 
 def test_resume_from_a_checkpoint_written_by_the_reference(oracle, case):
+    _needs_qb_ref(oracle)
     A, meta, ex, work, path = case
     n = A.dim
     w = os.path.join(work, "ref_writes")
@@ -84,6 +88,7 @@ def test_resume_from_a_checkpoint_written_by_the_reference(oracle, case):
 
 
 def test_the_reference_resumes_from_a_checkpoint_written_here(oracle, case):
+    _needs_qb_ref(oracle)
     A, meta, ex, work, path = case
     n = A.dim
     k = 25
@@ -187,6 +192,7 @@ def _numpy_cg(oracle, A, E0, m, v, r, p, maxit):
 
 
 def test_cg_checkpoints_in_both_directions(oracle, case):
+    _needs_qb_ref(oracle)
     A, meta, ex, work, path = case
     n, E0 = A.dim, meta["lanczos_E0"]
     # the reference stops at step 10 -> we load and continue to its own stopping step and vector

@@ -15,7 +15,7 @@ QB_AB = os.path.join(ROOT, "oracle", "_ref", "qb_ab")
 @pytest.mark.parametrize("name", ["tri4x4_k01", "hubbard4x2", "heis16_full"])
 def test_reference_templates_over_the_gpu_adaptor(oracle, name, tmp_path):
     if not os.path.exists(QB_AB):
-        pytest.skip("oracle/_ref/qb_ab not built (make -C oracle ab; needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/qb_ab not built (make -C oracle ab; needs the reference's sources at build time)")
     A, meta, ex = oracle.load_golden(name)
     f = str(tmp_path / "H.qbcsr")
     out = str(tmp_path / "ab.json")
