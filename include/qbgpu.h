@@ -421,10 +421,6 @@ int qbgpu_build_heisenberg_orbit(qbgpu_matrix_t *A, int nsites, int ndown, int n
 int64_t qbgpu_dim_heisenberg(int nsites, int nup);
 int64_t qbgpu_dim_hubbard(int nsites, int nup, int ndn);
 
-/* tuning hook used by scripts/kbench.py: selects an experimental instantiation of the sliced-jagged kernel
- * (only in builds with -DQBGPU_TUNING_VARIANTS; otherwise a no-op).  id 0 = production configuration.
- * id 1000 + v selects pass 1 of the matrix-free species-order product instead: v = 0 grid-stride rows (default),
- * 1 contiguous row ranges with one 1024-thread CTA per SM, 2 block x[iu, :] staged in shared memory. */
 /* ---------------------------------------------------------------------------- multi-GPU drivers (csrc/dist.cu)
  * One process per GPU; everything a rank needs from its peers travels through peer memory (CUDA IPC over NVLink): copy-engine
  * pulls of the vector slices and a push-based, deterministic all-reduce kernel for the scalars -- no MPI / NCCL inside, so a
@@ -474,6 +470,8 @@ int qbgpu_dist_kpm_moments(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matr
 int qbgpu_dist_eigenvec_cg(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, int64_t maxit, int64_t *m, const double E0[2],
                            double *accu, void *v_dev, void *r_dev, void *p_dev, void *pp_dev);
 
+/* pass 1 of the matrix-free species-order product: id = 1000 + v, v = 0 grid-stride rows (default), 1 contiguous row ranges
+ * with one 1024-thread CTA per SM, 2 block x[iu, :] staged in shared memory.  Any other id: QBGPU_ERR_ARG. */
 int qbgpu_debug_set_variant(int id);
 /* Rows of a full-basis Heisenberg (kind 0, n0 = down spins) or Hubbard (kind 1, n0/n1 = N_up/N_dn) operator recomputed on the
  * HOST in long double from the Lin tables (reference src/basis.cc:1144-1190) and the generators' own row function: the
@@ -481,9 +479,6 @@ int qbgpu_debug_set_variant(int id);
  * full vector (x_complex: re,im pairs); y_out: 2 doubles per listed row.  No device involved. */
 int qbgpu_debug_rows_host(int kind, int nsites, int n0, int n1, int nbonds, const int32_t *bonds, double J, double t, double U,
                           int64_t nrows, const int64_t *rows, const void *x_host, int x_complex, double *y_out);
-/* |col - row| beyond which a gathered entry is loaded with the L2 evict-first policy (kernels with the per-entry
- * gather policy only) */
-int qbgpu_debug_set_far_rows(int64_t rows);
 
 /* counters for bench.py's `gpu_launches` (kernels launched by this library since the last reset) */
 int64_t qbgpu_kernel_launches(int reset);

@@ -70,7 +70,7 @@ _SIGS = {
     "qbgpu_trlan_largest": [vp, C.c_int, C.c_int, C.c_int, dbl, C.POINTER(C.c_int), C.POINTER(C.c_int), vp, vp, C.c_int],
     "qbgpu_spmv_fused": [vp, vp, vp, vp, vp, vp, vp, vp],
     "qbgpu_lanczos_step_a": [vp, vp, vp, vp], "qbgpu_lanczos_step_a_part": [vp, vp, vp, vp, C.c_int, C.c_int],
-    "qbgpu_split_columns": [vp, C.c_int, vp, vp, C.c_int], "qbgpu_debug_set_variant": [C.c_int], "qbgpu_debug_set_far_rows": [C.c_int64], "qbgpu_real_view": [vp, C.POINTER(vp)],
+    "qbgpu_split_columns": [vp, C.c_int, vp, vp, C.c_int], "qbgpu_debug_set_variant": [C.c_int], "qbgpu_real_view": [vp, C.POINTER(vp)],
     "qbgpu_ipc_export": [vp, vp], "qbgpu_ipc_open": [vp, C.POINTER(vp)], "qbgpu_ipc_close": [vp],
     "qbgpu_peer_pull_async": [C.c_int, C.c_int, vp, vp, C.c_size_t], "qbgpu_peer_wait": [C.c_int], "qbgpu_ring_prepare": [vp, C.c_int, C.c_int, i64, C.POINTER(vp)], "qbgpu_peer_ring_reset": [],
     "qbgpu_peer_pull_flag": [C.c_int, C.c_int, vp, vp, C.c_size_t, C.c_int], "qbgpu_peer_ring_status": [vp], "qbgpu_peer_pull_sm": [C.c_int, C.c_int, vp, vp, C.c_size_t, C.c_int], "qbgpu_lanczos_step_b": [vp, vp, vp, vp],

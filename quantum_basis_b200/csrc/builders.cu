@@ -607,12 +607,6 @@ struct TermTable {
     // branch-free decode for spmv_terms_kernel_v2: XOR masks on the two sublattice labels and "sites below" masks; the
     // padding code 255 has all-zero masks and amplitude 0, so it replays as "0 * x[own row]"
     uint32_t mask_a[256], mask_b[256], below_f[256], below_t[256];
-    // packed decode for spmv_terms_kernel_v3 (one 64-bit and one 32-bit shared-memory lookup per entry instead of six):
-    // masks[code] = mask_a | mask_b << 32;  meta[code] = f | t << 5 | spin << 10 | (f < t) << 11 | weight << 12;
-    // amp_of_weight[w] = the amplitude of a bond of multiplicity w (accumulated like the LIL assembly)
-    unsigned long long masks[256];
-    uint32_t meta[256];
-    double amp_of_weight[256];
 };
 
 __global__ void __launch_bounds__(kBBlock) matfree_states_kernel(SectorTables S, int64_t row_lo, int64_t nloc, uint2 *states)
@@ -858,116 +852,12 @@ spmv_terms_kernel_v2(SectorTables S, const ModelParams *Mp, const TermTable *Tp,
     }
 }
 
-
-// Experimental variant (QBGPU_TERMS_KERNEL=3): the six per-entry shared-memory lookups folded into one 64-bit and one 32-bit lookup; the "below" masks are
-// rebuilt with shifts and the amplitude comes from a table indexed by the bond multiplicity (almost always the same
-// address across a warp: a broadcast).  QBGPU_TERMS_KERNEL=3; not yet run on hardware.
-template <typename VecT, bool DOTS, int KIND>
-__global__ void __launch_bounds__(kMFBlock, 3)
-spmv_terms_kernel_v3(SectorTables S, const ModelParams *Mp, const TermTable *Tp, const uint2 *__restrict__ states, const int64_t *__restrict__ sliceptr,
-                     const uint32_t *__restrict__ codes, int64_t nrows, int64_t nslices, int64_t row_lo, int wbonds,
-                     const VecT *__restrict__ x, const VecT *z, VecT *y, double2 alpha, double2 gamma, double2 beta,
-                     int scal_mode, const double *__restrict__ sc, double *dots_out, double *partials, unsigned *ticket)
-{
-    using VT = VecTraits<VecT>;
-    __shared__ ModelParams M;
-    __shared__ unsigned long long masks[256];
-    __shared__ uint32_t meta[256];
-    __shared__ double ampw[256];
-    for (int k = threadIdx.x; k < 16; k += blockDim.x) ((int *)&M)[k] = ((const int *)Mp)[k];
-    for (int k = threadIdx.x; k < 256; k += blockDim.x) { masks[k] = Tp->masks[k]; meta[k] = Tp->meta[k]; ampw[k] = Tp->amp_of_weight[k]; }
-    __syncthreads();
-    double dot_scale = 1.0;
-    if (scal_mode != 0) {
-        const double sx = sc[0], sz = sc[1], bprev = sc[2];
-        alpha = make_double2(sx, 0.0);
-        gamma = make_double2(0.0, 0.0);
-        beta = scal_mode == 1 ? make_double2(-bprev * sz, 0.0) : make_double2(1.0, 0.0);
-        dot_scale = sx;
-    }
-    const bool use_beta = (beta.x != 0.0 || beta.y != 0.0);
-    double d[3] = {0.0, 0.0, 0.0};
-    const int lane = threadIdx.x & 31;
-    constexpr int WPB = kMFBlock / 32;
-    for (int64_t s = (int64_t)blockIdx.x * WPB + (threadIdx.x >> 5); s < nslices; s += (int64_t)gridDim.x * WPB) {
-        const int64_t base = sliceptr[s];
-        const int maxw = (int)((sliceptr[s + 1] - base) >> 5);
-        const int64_t row = s * 32 + lane;
-        const bool live = row < nrows;
-        const uint2 st = live ? states[row] : states[nrows - 1];
-        const uint32_t la = st.x, lb = st.y;
-        const uint32_t occ0 = (la & 0x55555555u) | ((lb & 0x55555555u) << 1);
-        const uint32_t occ1 = ((la >> 1) & 0x55555555u) | (lb & 0xAAAAAAAAu);
-        const uint32_t occ01 = occ0 ^ occ1;                      // parity of the fermions on a site (0, 1 or 2 electrons)
-        VecT acc = VT::zero();
-        int anti = 0;
-        uint32_t wnext = maxw > 0 ? codes[base + lane] : 0xFFFFFFFFu;
-        for (int k = 0; k < maxw; k++) {
-            const uint32_t w4 = wnext;
-            if (k + 1 < maxw) wnext = codes[base + (int64_t)(k + 1) * 32 + lane];
-            uint32_t na[4], nb[4];
-            double v[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-                const uint32_t code = (w4 >> (8 * u)) & 255u;
-                const unsigned long long mk = masks[code];
-                const uint32_t mt = meta[code];
-                na[u] = la ^ (uint32_t)mk;
-                nb[u] = lb ^ (uint32_t)(mk >> 32);
-                const double a = ampw[mt >> 12];
-                if (KIND == 0) {
-                    anti += (int)(mt >> 12);
-                    v[u] = a;
-                } else {
-                    const int f = mt & 31, t = (mt >> 5) & 31;
-                    // parity of the fermions below f plus below t = parity of (occ0 ^ occ1) over the sites strictly between
-                    // them and, when f < t, f itself...: popc(x & bf) + popc(x & bt) has the parity of popc(x & (bf ^ bt))
-                    const uint32_t between = ((1u << f) - 1u) ^ ((1u << t) - 1u);
-                    int sg = __popc(occ01 & between);
-                    sg += (int)((mt >> 10) & 1u) * ((int)((occ0 >> f) & 1u) + (int)((occ0 >> t) & 1u)) + (int)((mt >> 11) & 1u);
-                    v[u] = (sg & 1) ? -a : a;
-                }
-            }
-            int64_t jb[4];
-            int32_t ra[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) { jb[u] = __ldg(S.Jb + nb[u]); ra[u] = __ldg(S.rankA + na[u]); }
-            VecT xv[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) xv[u] = ld_vec(x + (jb[u] + ra[u]));
-#pragma unroll
-            for (int u = 0; u < 4; u++) mac(acc, v[u], xv[u]);
-        }
-        if (live) {
-            double diag;
-            if (KIND == 0) diag = 0.25 * M.J * (double)(wbonds - 2 * anti);
-            else { diag = 0.0; const int ndbl = __popc(occ0 & occ1); for (int r = 0; r < ndbl; r++) diag += M.U; }
-            const VecT xi = x[row_lo + row];
-            mac(acc, diag, xi);
-            VecT out = VT::scale(alpha, acc);
-            if (gamma.x != 0.0 || gamma.y != 0.0) out = VT::add(out, VT::scale(gamma, xi));
-            if (use_beta) out = VT::add(out, VT::scale(beta, z[row]));
-            y[row] = out;
-            if (DOTS) {
-                const double2 p = VT::conj_mul(xi, out);
-                d[0] += p.x; d[1] += p.y; d[2] += VT::abs2(out);
-            }
-        }
-    }
-    if (DOTS) {
-        d[0] *= dot_scale; d[1] *= dot_scale;
-        block_reduce_finalize<3, kMFBlock>(d, partials, ticket, dots_out);
-    }
-}
-
 template <typename VecT, bool DOTS>
 static int launch_terms_variant(const qbgpu_matrix *A, const FusedArgs &a)
 {
     Context &c = ctx();
     const MatFree *mf = (const MatFree *)A->mf;
-    static const int version = getenv("QBGPU_TERMS_KERNEL") ? atoi(getenv("QBGPU_TERMS_KERNEL")) : 2;
-    auto kern = version == 3 ? (mf->kind == 0 ? spmv_terms_kernel_v3<VecT, DOTS, 0> : spmv_terms_kernel_v3<VecT, DOTS, 1>)
-                             : (mf->kind == 0 ? spmv_terms_kernel_v2<VecT, DOTS, 0> : spmv_terms_kernel_v2<VecT, DOTS, 1>);
+    auto kern = mf->kind == 0 ? spmv_terms_kernel_v2<VecT, DOTS, 0> : spmv_terms_kernel_v2<VecT, DOTS, 1>;
     int blocks_per_sm = 0;
     QB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kern, kMFBlock, 0));
     if (blocks_per_sm < 1) blocks_per_sm = 1;
@@ -1115,16 +1005,6 @@ static int create_matfree(qbgpu_matrix_t *out, const HostTables &T, const ModelP
             TT.below_t[code] = (1u << t) - 1u;
         }
         TT.hop[255] = 0; TT.amp[255] = 0.0;                    // padding: no flip, no weight, zero amplitude
-        for (int code = 0; code < 256; code++) {
-            const uint32_t h = TT.hop[code];
-            const uint32_t f = h & 31u, t = (h >> 5) & 31u, sp = (h >> 10) & 1u, w = code < TT.ncodes ? (h >> 11) : 0u;
-            TT.masks[code] = (unsigned long long)TT.mask_a[code] | ((unsigned long long)TT.mask_b[code] << 32);
-            TT.meta[code] = f | (t << 5) | (sp << 10) | ((f < t ? 1u : 0u) << 11) | ((w & 255u) << 12);
-        }
-        for (int w = 0; w < 256; w++) {
-            if (M.kind == 0) TT.amp_of_weight[w] = 0.5 * M.J * w;
-            else { double amp = 0.0; for (int r = 0; r < w; r++) amp += -M.t; TT.amp_of_weight[w] = amp; }
-        }
         const int64_t nslices = (nloc + 31) / 32;
         int64_t *d_words = nullptr;
         void *d_tmp = nullptr;

@@ -59,25 +59,10 @@ int qbgpu_init(int device)
     cudaDeviceProp prop;
     QB_CUDA(cudaGetDeviceProperties(&prop, device));
     c.num_sms = prop.multiProcessorCount;
-    // L2 evict_last / persisting accesses only take effect inside the persisting set-aside, which defaults to 0 bytes
-    // (measured, profiles/r01_kbench_sweep3_l2_persist.txt: a set-aside does not help this kernel and the maximum one
-    // costs 7-13 %, so it stays off unless QBGPU_L2_PERSIST_MB asks for it)
-    // L2 fetch granularity hint (32, 64 or 128 bytes): the gathers of x are 8/16-byte reads scattered over the vector, so
-    // anything fetched beyond the 32-byte sector would be wasted DRAM traffic.  Measured on B200: no effect at all
-    // (profiles/r01_kbench_l2_fetch_granularity.txt), so nothing is set unless QBGPU_L2_FETCH_BYTES asks for it
-    if (const char *fg = getenv("QBGPU_L2_FETCH_BYTES")) {
-        const long v = atol(fg);
-        if (v == 32 || v == 64 || v == 128) {
-            cudaError_t le = cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)v);
-            if (le != cudaSuccess) cudaGetLastError();      // a hint: not every device accepts it
-        }
-    }
-    if (prop.persistingL2CacheMaxSize > 0 && getenv("QBGPU_L2_PERSIST_MB")) {
-        size_t want = (size_t)atol(getenv("QBGPU_L2_PERSIST_MB")) << 20;
-        if (want > (size_t)prop.persistingL2CacheMaxSize) want = (size_t)prop.persistingL2CacheMaxSize;
-        (void)cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want);
-        if (getenv("QBGPU_VERBOSE")) fprintf(stderr, "[qbgpu] L2 %d MB, persisting set-aside %zu MB (max %d MB)\n", prop.l2CacheSize >> 20, want >> 20, prop.persistingL2CacheMaxSize >> 20);
-    }
+    // No L2 limit is set.  L2 evict_last / persisting accesses only take effect inside the persisting set-aside, which
+    // defaults to 0 bytes; measured, a set-aside does not help the products and the maximum one costs 7-13 %
+    // (profiles/r01_kbench_sweep3_l2_persist.txt).  An L2 fetch granularity hint had no effect at all
+    // (profiles/r01_kbench_l2_fetch_granularity.txt).
     QB_CUDA(cudaStreamCreateWithFlags(&c.own_stream, cudaStreamNonBlocking));
     QB_CUDA(cudaStreamCreateWithFlags(&c.copy_stream, cudaStreamNonBlocking));
     c.stream = c.own_stream;
@@ -184,16 +169,8 @@ int qbgpu_host_unregister(void *ptr)
 
 int qbgpu_debug_set_variant(int id)
 {
-    if (id >= 1000 && id < 1010) { qb::set_kron_local_variant(id - 1000); return QBGPU_OK; }   // pass 1 of the matrix-free species product
-    if (id >= 2000 && id < 2020) { qb::set_sjds_bulk_mode(id - 2000); return QBGPU_OK; }       // bulk-streamed sliced-jagged product: 0 off, 1.. configuration
-    if (id >= 3000 && id < 3030) { qb::set_block_smem_variant(id - 3000); return QBGPU_OK; }   // block-local product (pass 1 of the stored species handle)
-    qb::set_sjds_variant(id);
-    return QBGPU_OK;
-}
-
-int qbgpu_debug_set_far_rows(int64_t rows)
-{
-    qb::set_sjds_far_rows(rows);
+    if (id < 1000 || id > 1002) return fail(QBGPU_ERR_ARG, "debug_set_variant: unknown id " + std::to_string(id) + " (1000, 1001 or 1002)");
+    qb::set_kron_local_variant(id - 1000);
     return QBGPU_OK;
 }
 

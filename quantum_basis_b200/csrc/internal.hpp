@@ -50,9 +50,6 @@ struct qbgpu_matrix {
     void    *sp = nullptr;
     qbgpu_matrix *second = nullptr;
     int32_t *slice_order = nullptr;
-    // per traversal item: x = the slice (= slice_order[it]), y = 0x80000000 | len when the slice's 32 rows all have `len` entries and
-    // rank = row (the producer of the bulk-streamed kernel then needs no rowinfo load: 8 bytes per slice instead of 4 + 128)
-    uint2   *ord_desc = nullptr;
     // > 0: rows [u*block_D, (u+1)*block_D) reference only columns of the same block (the local part of a species handle):
     // the product may stage the block of x in shared memory (sjds_bulk.cu: sjds_block_smem_kernel)
     int64_t  block_D = 0;
@@ -90,14 +87,10 @@ struct FusedArgs {
     int         scal_mode = 0;
     const double *sc = nullptr;    // device scalars for scal_mode != 0
     double     *dots = nullptr;    // device: out[0]=Re sum conj(x)y, out[1]=Im, out[2]=sum|y|^2 ; null = no dots
-    // species handles, real-content route of MultMv (species.cu: mv_species): the way in fused into pass 1.  When x_ref is set,
-    // x (fp64, internal order) is an OUTPUT of the block-local kernel: it stages the block from the complex vector in the
-    // reference's order through perm_inv, writes it to x for pass 2, and raises *imag_flag if an imaginary part is not zero.
-    const void *x_ref = nullptr;
+    // species handles, real-content route of MultMv (species.cu: mv_species): the way OUT fused into the closing pass (fp64
+    // vectors, y += H_cross x): instead of y[row] the bulk-streamed kernel writes y_ref[perm_inv[row]] = out_alpha * (y, 0)
+    // -- complex, in the reference's order -- and the separate permutation is skipped
     const int32_t *perm_inv = nullptr;
-    int        *imag_flag = nullptr;
-    // the way OUT fused into the closing pass (fp64 vectors, y += H_cross x): instead of y[row] the bulk-streamed kernel writes
-    // y_ref[perm_inv[row]] = out_alpha * (y, 0) -- complex, in the reference's order -- and the separate permutation is skipped
     void       *y_ref = nullptr;
     double2     out_alpha = {1.0, 0.0};
 };
@@ -108,24 +101,17 @@ int autotune(qbgpu_matrix *A, int flags = 0);
 int sjds_convert(qbgpu_matrix *A, bool forward);
 int value_dict_encode(qbgpu_matrix *A);               // matrix.cu: try to replace fp64 values by 1-byte codes
 int launch_spmv_sjds(const qbgpu_matrix *A, const FusedArgs &args);
-void set_sjds_variant(int v);
 // sjds_bulk.cu: the same product with the matrix stream moved by cp.async.bulk into per-warp shared-memory rings, and the
 // block-local product (rows of block u reference only columns of block u) with the block of x staged in shared memory
-int launch_spmv_sjds_bulk(const qbgpu_matrix *A, const FusedArgs &args);
-int sjds_bulk_mode();
-bool sjds_bulk_wanted(const qbgpu_matrix *A);
+int launch_spmv_sjds_bulk(const qbgpu_matrix *A, const FusedArgs &args);        // tile-ordered handles (slice_order set)
 bool sjds_bulk_out_fusable(const qbgpu_matrix *cross_part);      // the closing pass of this part can write the reference-order result itself
-void set_sjds_bulk_mode(int m);
 bool block_smem_applicable(const qbgpu_matrix *A, int64_t D);
-bool sjds_block_variant_ok();
 int launch_spmv_block_smem(const qbgpu_matrix *A, const FusedArgs &args, int64_t D);
-void set_block_smem_variant(int v);
 int launch_spmv_matfree(const qbgpu_matrix *A, const FusedArgs &args);     // builders.cu
 void matfree_destroy(qbgpu_matrix *A);
 int launch_spmv_sector_matfree(const qbgpu_matrix *A, const FusedArgs &a);      // sectors.cu
 void sector_matfree_destroy(qbgpu_matrix *A);
 int64_t matfree_bytes(const qbgpu_matrix *A);
-void set_sjds_far_rows(int64_t r);      // in-place CSR <-> sliced-jagged re-ordering of col/val
 int ring_prepare(qbgpu_matrix *A, int rank, int world, int64_t chunk, qbgpu_matrix **view);     // sjds.cu
 int peer_ring_flags(const int **flags, int **timeout_flag);                 // peer.cu: arrival flags by ring distance
 int peer_mark_fence();                                                      // peer.cu: pulls enqueued later are ordered after THIS point of the compute stream
@@ -134,7 +120,7 @@ int peer_record_on_lane(int lane, cudaEvent_t ev);                          // p
 // species.cu
 int launch_spmv_species(const qbgpu_matrix *A, const FusedArgs &args);      // the two-pass products of species-order handles
 void species_destroy(qbgpu_matrix *A);
-void set_kron_local_variant(int v);       // tuning hook (qbgpu_debug_set_variant(1000 + v)); default from QBGPU_KRON_LOCAL
+void set_kron_local_variant(int v);       // tuning hook (qbgpu_debug_set_variant(1000 + v)); default 0
 int64_t species_bytes(const qbgpu_matrix *A);
 // dst[perm[r]] = src[r]  (reference order -> internal order); complex -> real takes the real part, real -> complex sets imag = 0
 int vec_to_native(const qbgpu_matrix *A, bool src_cplx, bool dst_cplx, const void *src, void *dst);

@@ -474,7 +474,7 @@ int qbgpu_destroy(qbgpu_matrix_t A)
 {
     if (!A) return QBGPU_OK;                               // like mkl_sparse_destroy on csr_mat's empty objects
     if (!A->borrowed) { matfree_destroy(A); sector_matfree_destroy(A); species_destroy(A); }
-    if (!A->borrowed) { cudaFree(A->rowptr); cudaFree(A->col); cudaFree(A->val); cudaFree(A->rowinfo); cudaFree(A->vdict); cudaFree(A->slice_order); cudaFree(A->ord_desc);
+    if (!A->borrowed) { cudaFree(A->rowptr); cudaFree(A->col); cudaFree(A->val); cudaFree(A->rowinfo); cudaFree(A->vdict); cudaFree(A->slice_order);
                         cudaFree(A->perm_x); cudaFree(A->perm_y); }
     else if (A->owns_order) cudaFree(A->slice_order);
     delete A;

@@ -29,50 +29,21 @@ __device__ __forceinline__ uint64_t l2_policy_evict_last()  { uint64_t p; asm vo
 
 // All loads of the inner loop are volatile asm so that they are issued in program order -- first the U column and
 // value loads of a trip, then the U gathers -- instead of ptxas' register-frugal "load, gather, fma" chain per
-// diagonal, which leaves a warp with a single dependent pair of loads in flight.
-template <int POL> __device__ __forceinline__ int ld_i32(const int *p, uint64_t pol)
-{
-    int v;
-    if (POL == 0) asm volatile("ld.global.cs.b32 %0, [%1];" : "=r"(v) : "l"(p));
-    else if (POL == 1) asm volatile("ld.global.nc.b32 %0, [%1];" : "=r"(v) : "l"(p));
-    else if (POL == 2) asm volatile("ld.global.nc.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-    else asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-    return v;
-}
-template <int POL> __device__ __forceinline__ double ld_f64(const double *p, uint64_t pol)
-{
-    double v;
-    if (POL == 0) asm volatile("ld.global.cs.f64 %0, [%1];" : "=d"(v) : "l"(p));
-    else if (POL == 1) asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(v) : "l"(p));
-    else if (POL == 2) asm volatile("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol));
-    else asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol));
-    return v;
-}
-template <int POL> __device__ __forceinline__ uint8_t ld_f64(const uint8_t *p, uint64_t pol)      // dictionary codes
-{
-    unsigned v;
-    if (POL == 0) asm volatile("ld.global.cs.u8 %0, [%1];" : "=r"(v) : "l"(p));
-    else if (POL == 1) asm volatile("ld.global.nc.u8 %0, [%1];" : "=r"(v) : "l"(p));
-    else if (POL == 2) asm volatile("ld.global.nc.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-    else asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-    return (uint8_t)v;
-}
-template <int POL> __device__ __forceinline__ double2 ld_f64(const double2 *p, uint64_t pol)
-{
-    double2 v;
-    if (POL == 0) asm volatile("ld.global.cs.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
-    else if (POL == 1) asm volatile("ld.global.nc.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
-    else if (POL == 2) asm volatile("ld.global.nc.L2::cache_hint.v2.f64 {%0, %1}, [%2], %3;" : "=d"(v.x), "=d"(v.y) : "l"(p), "l"(pol));
-    else asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.f64 {%0, %1}, [%2], %3;" : "=d"(v.x), "=d"(v.y) : "l"(p), "l"(pol));
-    return v;
-}
-// gathered vector: XPOL 0 = read-only path, default policy; 1 = read-only path + L2 evict_last; 2 = per entry:
-// evict_last when the column is within `far_rows` of the row (it will be gathered again soon by a neighbouring
-// jagged diagonal), evict_first for the long-range terms, whose next use is further away than L2 can hold
+// diagonal, which leaves a warp with a single dependent pair of loads in flight.  The matrix stream is read through the
+// non-coherent path with an L2 evict_first policy operand.
+__device__ __forceinline__ int ld_i32(const int *p, uint64_t pol)
+{ int v; asm volatile("ld.global.nc.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol)); return v; }
+__device__ __forceinline__ double ld_f64(const double *p, uint64_t pol)
+{ double v; asm volatile("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol)); return v; }
+__device__ __forceinline__ uint8_t ld_f64(const uint8_t *p, uint64_t pol)      // dictionary codes
+{ unsigned v; asm volatile("ld.global.nc.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol)); return (uint8_t)v; }
+__device__ __forceinline__ double2 ld_f64(const double2 *p, uint64_t pol)
+{ double2 v; asm volatile("ld.global.nc.L2::cache_hint.v2.f64 {%0, %1}, [%2], %3;" : "=d"(v.x), "=d"(v.y) : "l"(p), "l"(pol)); return v; }
+// gathered vector: XPOL 0 = read-only path, default policy; 1 = read-only path + L2 evict_last
 template <int XPOL> __device__ __forceinline__ double ld_x(const double *p, uint64_t pol)
 {
     double v;
-    if (XPOL == 0) asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(v) : "l"(p));  // XPOL 1,2: policy operand
+    if (XPOL == 0) asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(v) : "l"(p));  // XPOL 1: policy operand
     else asm volatile("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol));
     return v;
 }
@@ -84,22 +55,19 @@ template <int XPOL> __device__ __forceinline__ double2 ld_x(const double2 *p, ui
     return v;
 }
 
-// U = jagged diagonals per trip (U independent col/val loads, then U gathers); SPOL/XPOL = cache policies above;
+// U = jagged diagonals per trip (U independent col/val loads, then U gathers); XPOL = cache policy of the gathers above;
 // UL = unconditional loads: lanes whose row has ended re-read the slice's first entry (always valid, L1-resident)
 // instead of branching around the loads, so that all 3U loads of a trip can be in flight together;
 // MINB = __launch_bounds__ min blocks/SM: without it ptxas schedules for 32 registers (full occupancy) and chains
 // "load column, load value, gather, fma" one diagonal at a time -- a single dependent pair of loads in flight per
 // warp; with MINB <= 4 it batches the U column loads, the U value loads and the U gathers (checked in the SASS).
-// ORD = the slices are visited in the order given by `order` (the cross part of a species-order handle: tiles of down
-// indices, so that the gathered columns of a tile stay in L2) instead of ascending; a template parameter for the same
-// reason as KEEP.
-template <typename ValT, typename VecT, bool DOTS, int U, int SPOL, int XPOL, bool UL, int MINB, bool KEEP = false, bool ORD = false>
+template <typename ValT, typename VecT, bool DOTS, int U, int XPOL, bool UL, int MINB, bool KEEP = false>
 __global__ void __launch_bounds__(kSBlock, MINB)
 spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *__restrict__ rowptr,
                  const uint32_t *__restrict__ rowinfo, const int32_t *__restrict__ col, const ValT *__restrict__ val,
                  const VecT *__restrict__ x, const VecT *z, VecT *y, double2 alpha, double2 gamma, double2 beta,
                  int scal_mode, const double *__restrict__ sc, double *dots_out, double *partials, unsigned *ticket,
-                 int64_t far_rows, const double *__restrict__ vdict, const int32_t *__restrict__ order)
+                 const double *__restrict__ vdict)
 {
     using VT = VecTraits<VecT>;
     constexpr bool kDict = sizeof(ValT) == 1;               // 1-byte codes into a <= 256-entry fp64 dictionary
@@ -108,7 +76,7 @@ spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *
     if (kDict) { sdict[threadIdx.x] = vdict[threadIdx.x]; __syncthreads(); }      // kSBlock == 256 threads
     constexpr int WPB = kSBlock / 32;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t pol_s = (SPOL >= 2 || XPOL == 2) ? l2_policy_evict_first() : 0, pol_x = XPOL >= 1 ? l2_policy_evict_last() : 0;
+    const uint64_t pol_s = l2_policy_evict_first(), pol_x = XPOL >= 1 ? l2_policy_evict_last() : 0;
     double dot_scale = 1.0;
     if (scal_mode != 0) {                                  // Lanczos step a: 1 = first column block, 2 = a later one
         const double sx = sc[0], sz = sc[1], bprev = sc[2];
@@ -125,9 +93,7 @@ spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *
     // well (a run-time flag here cost 15-25 % on the unsplit product).
     double d[3] = {0.0, 0.0, 0.0};
 
-    for (int64_t it = (int64_t)blockIdx.x * WPB + warp; it < nslices; it += (int64_t)gridDim.x * WPB) {
-        int64_t s = it;
-        if constexpr (ORD) s = order[it];
+    for (int64_t s = (int64_t)blockIdx.x * WPB + warp; s < nslices; s += (int64_t)gridDim.x * WPB) {
         const uint32_t info = rowinfo[s * 32 + lane];
         const int len = (int)(info & kLenMask);
         const int64_t row = s * 32 + (info >> 24);
@@ -150,11 +116,11 @@ spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *
             if (UL) {
                 VecT xv[U];
 #pragma unroll
-                for (int u = 0; u < U; u++) c[u] = ld_i32<SPOL>(col + o[u], pol_s);
+                for (int u = 0; u < U; u++) c[u] = ld_i32(col + o[u], pol_s);
 #pragma unroll
-                for (int u = 0; u < U; u++) v[u] = ld_f64<SPOL>(val + o[u], pol_s);
+                for (int u = 0; u < U; u++) v[u] = ld_f64(val + o[u], pol_s);
 #pragma unroll
-                for (int u = 0; u < U; u++) xv[u] = ld_x<XPOL>(x + c[u], (XPOL == 2 && llabs((long long)c[u] - (long long)(row_lo + row)) > far_rows) ? pol_s : pol_x);
+                for (int u = 0; u < U; u++) xv[u] = ld_x<XPOL>(x + c[u], pol_x);
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     VecT t = (u & 1) ? acc1 : acc0;
@@ -167,15 +133,14 @@ spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     c[u] = 0; v[u] = ValT{};
-                    if (a[u]) { c[u] = ld_i32<SPOL>(col + o[u], pol_s); v[u] = ld_f64<SPOL>(val + o[u], pol_s); }
+                    if (a[u]) { c[u] = ld_i32(col + o[u], pol_s); v[u] = ld_f64(val + o[u], pol_s); }
                 }
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     if (a[u]) {
-                        const uint64_t px = (XPOL == 2 && llabs((long long)c[u] - (long long)(row_lo + row)) > far_rows) ? pol_s : pol_x;
                         ArithT w;
                         if constexpr (kDict) w = sdict[v[u]]; else w = v[u];
-                        if (u & 1) mac(acc1, w, ld_x<XPOL>(x + c[u], px)); else mac(acc0, w, ld_x<XPOL>(x + c[u], px));
+                        if (u & 1) mac(acc1, w, ld_x<XPOL>(x + c[u], pol_x)); else mac(acc0, w, ld_x<XPOL>(x + c[u], pol_x));
                     }
                 }
             }
@@ -200,18 +165,11 @@ spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *
     }
 }
 
-// tuning hook (qbgpu_debug_set_variant): variant id = 1 + MINB_index*16 + UL*8 + U_index*4 + SPOL_index*2 + XPOL
-// (MINB_index 0 -> 2 blocks/SM, 1 -> 4; U_index 0 -> 4, 1 -> 8; SPOL_index 0 -> .cs, 1 -> L2 evict_first hint)
-static int g_sjds_variant = 0;
-static int64_t g_far_rows = 1 << 21;                      // rows; ~32 MB of complex vector either side
-void set_sjds_variant(int v) { g_sjds_variant = v; }
-void set_sjds_far_rows(int64_t r) { g_far_rows = r; }
-
-template <typename ValT, typename VecT, bool DOTS, int U, int SPOL, int XPOL, bool UL, int MINB, bool KEEP = false, bool ORD = false>
-static int launch_sjds_variant(const qbgpu_matrix *A, const FusedArgs &a)
+template <typename ValT, typename VecT, bool DOTS, int U, int XPOL, bool UL, int MINB, bool KEEP = false>
+static int launch_sjds_cfg(const qbgpu_matrix *A, const FusedArgs &a)
 {
     Context &c = ctx();
-    auto kern = spmv_sjds_kernel<ValT, VecT, DOTS, U, SPOL, XPOL, UL, MINB, KEEP, ORD>;
+    auto kern = spmv_sjds_kernel<ValT, VecT, DOTS, U, XPOL, UL, MINB, KEEP>;
     static int blocks_per_sm = 0;
     if (blocks_per_sm == 0) {
         QB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kern, kSBlock, 0));
@@ -227,65 +185,27 @@ static int launch_sjds_variant(const qbgpu_matrix *A, const FusedArgs &a)
     const int grid = (int)(want < cap ? want : cap);
     kern<<<grid, kSBlock, 0, c.stream>>>(nslices, nrows, A->row_lo, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val,
                                          (const VecT *)a.x, (const VecT *)a.z, (VecT *)a.y, a.alpha, a.gamma, a.beta,
-                                         a.scal_mode, a.sc, a.dots, c.partials, c.ticket, g_far_rows, A->vdict, A->slice_order);
+                                         a.scal_mode, a.sc, a.dots, c.partials, c.ticket, A->vdict);
     QB_LAUNCH_COUNT();
     QB_CUDA(cudaGetLastError());
     return QBGPU_OK;
 }
 
-// production configuration of the template (chosen from the measurements in profiles/)
-// complex vectors: 4 diagonals per trip, branchy tail, 4 blocks/SM; fp64 vectors: 8 per trip, unconditional loads
-// (scripts/kbench.py sweeps, profiles/r01_kbench_*.txt)
-template <typename VecT> struct Prod { static constexpr int U = 4, S = 2, X = 1, MinB = 4, DotsMinB = 4; static constexpr bool UL = false; };
-template <> struct Prod<double> { static constexpr int U = 8, S = 2, X = 0, MinB = 4, DotsMinB = 3; static constexpr bool UL = true; };
-
 template <typename ValT, typename VecT>
 static int launch_sjds_typed(const qbgpu_matrix *A, const FusedArgs &a)
 {
+    // configuration of the template, chosen from the measurements in profiles/r01_kbench_*.txt: complex vectors take 4
+    // diagonals per trip, a branchy tail, L2 evict_last on the gathers and 4 blocks/SM; fp64 vectors take 8 per trip with
+    // unconditional loads (with the epilogue of the dots that needs a few more registers: 3 blocks/SM keeps its loads batched)
+    constexpr bool kCplx = sizeof(VecT) == 16;
+    constexpr int U = kCplx ? 4 : 8, X = kCplx ? 1 : 0, MinB = 4, DotsMinB = kCplx ? 4 : 3;
+    constexpr bool UL = !kCplx;
     const bool dots = a.dots != nullptr;
-#ifdef QBGPU_TUNING_VARIANTS
-    if constexpr (sizeof(ValT) == 8) {                      // experimental instantiations only for fp64 values
-        if (dots && g_sjds_variant >= 45) {                 // configurations of the fused-epilogue (DOTS) kernel
-            switch (g_sjds_variant) {
-            case 45: return launch_sjds_variant<ValT, VecT, true, 8, 2, 0, true, 3>(A, a);
-            case 46: return launch_sjds_variant<ValT, VecT, true, 8, 2, 0, true, 2>(A, a);
-            case 47: return launch_sjds_variant<ValT, VecT, true, 4, 2, 1, false, 4>(A, a);
-            case 48: return launch_sjds_variant<ValT, VecT, true, 4, 2, 1, false, 3>(A, a);
-            case 49: return launch_sjds_variant<ValT, VecT, true, 6, 2, 0, true, 3>(A, a);
-            case 50: return launch_sjds_variant<ValT, VecT, true, 4, 2, 0, true, 4>(A, a);
-            default: break;
-            }
-        }
-        if (!dots && g_sjds_variant > 0) {
-            switch (g_sjds_variant - 1) {
-#define QB_V1(M, MI, L, U, UI, S, SI, X) case (MI * 16 + (L ? 8 : 0) + UI * 4 + SI * 2 + X): return launch_sjds_variant<ValT, VecT, false, U, S, X, L, M>(A, a);
-#define QB_V2(M, MI, L, U, UI) QB_V1(M, MI, L, U, UI, 0, 0, 0) QB_V1(M, MI, L, U, UI, 0, 0, 1) QB_V1(M, MI, L, U, UI, 2, 1, 0) QB_V1(M, MI, L, U, UI, 2, 1, 1)
-#define QB_V3(M, MI) QB_V2(M, MI, false, 4, 0) QB_V2(M, MI, false, 8, 1) QB_V2(M, MI, true, 4, 0) QB_V2(M, MI, true, 8, 1)
-                QB_V3(2, 0) QB_V3(4, 1)
-#undef QB_V1
-#undef QB_V2
-#undef QB_V3
-            case 34: return launch_sjds_variant<ValT, VecT, false, 4, 2, 1, false, 3>(A, a);
-            case 37: return launch_sjds_variant<ValT, VecT, false, 2, 2, 1, false, 6>(A, a);
-            case 40: return launch_sjds_variant<ValT, VecT, false, 8, 2, 0, true, 3>(A, a);
-            default: break;
-            }
-        }
-    }
-#endif
-    using P = Prod<VecT>;
-    if (A->slice_order) {                                   // cross part of a species-order handle: tile-ordered traversal
-        if (!dots && a.scal_mode == 0 && a.z == a.y && a.beta.x == 1.0 && a.beta.y == 0.0 && a.gamma.x == 0.0 && a.gamma.y == 0.0)
-            return launch_sjds_variant<ValT, VecT, false, P::U, P::S, P::X, P::UL, P::MinB, true, true>(A, a);
-        return dots ? launch_sjds_variant<ValT, VecT, true, P::U, P::S, P::X, P::UL, P::DotsMinB, false, true>(A, a)
-                    : launch_sjds_variant<ValT, VecT, false, P::U, P::S, P::X, P::UL, P::MinB, false, true>(A, a);
-    }
     // accumulating column block of a sharded product (y += H_p x, immediates only): skip the rows this block does not touch
     if (!dots && a.scal_mode == 0 && a.z == a.y && a.beta.x == 1.0 && a.beta.y == 0.0 && a.gamma.x == 0.0 && a.gamma.y == 0.0)
-        return launch_sjds_variant<ValT, VecT, false, P::U, P::S, P::X, P::UL, P::MinB, true>(A, a);
-    // (with fp64 vectors the epilogue variant needs a few more registers: 3 blocks/SM keeps its loads batched)
-    return dots ? launch_sjds_variant<ValT, VecT, true, P::U, P::S, P::X, P::UL, P::DotsMinB>(A, a)
-                : launch_sjds_variant<ValT, VecT, false, P::U, P::S, P::X, P::UL, P::MinB>(A, a);
+        return launch_sjds_cfg<ValT, VecT, false, U, X, UL, MinB, true>(A, a);
+    return dots ? launch_sjds_cfg<ValT, VecT, true, U, X, UL, DotsMinB>(A, a)
+                : launch_sjds_cfg<ValT, VecT, false, U, X, UL, MinB>(A, a);
 }
 
 
@@ -348,7 +268,7 @@ spmv_sjds_ring_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
 #pragma unroll
             for (int u = 0; u < U; u++) {
                 c[u] = 0; v[u] = ValT{};
-                if (a[u]) { c[u] = ld_i32<2>(col + o[u], pol_s); v[u] = ld_f64<2>(val + o[u], pol_s); }
+                if (a[u]) { c[u] = ld_i32(col + o[u], pol_s); v[u] = ld_f64(val + o[u], pol_s); }
             }
             // the furthest slice this trip needs (ring order inside a row: the distance never decreases)
             int need = 0;
@@ -438,10 +358,12 @@ static int launch_sjds_ring_typed(const qbgpu_matrix *A, const FusedArgs &a)
 
 int launch_spmv_sjds(const qbgpu_matrix *A, const FusedArgs &a)
 {
-    // tile-ordered cross parts (and, on request, every handle): the matrix stream through cp.async.bulk + mbarrier rings
-    // (sjds_bulk.cu); QBGPU_SJDS_BULK=0 or a tuning variant of the register-fed kernel selects the kernels below
-    if (A->block_D > 0 && !a.dots && A->ring_world <= 1 && g_sjds_variant == 0 && block_smem_applicable(A, A->block_D)) return launch_spmv_block_smem(A, a, A->block_D);
-    if (A->ring_world <= 1 && (g_sjds_variant == 0 || a.y_ref) && sjds_bulk_wanted(A)) return launch_spmv_sjds_bulk(A, a);
+    if (A->block_D > 0 && !a.dots && A->ring_world <= 1 && block_smem_applicable(A, A->block_D)) return launch_spmv_block_smem(A, a, A->block_D);
+    // tile-ordered cross parts: the matrix stream through cp.async.bulk + mbarrier rings (sjds_bulk.cu).  Measured on BASELINE
+    // config 3 (profiles/r02_bulk_sweep_*.txt): on the one-pass product in the reference's order the bulk-streamed kernel equals
+    // the register-fed one at best (the gathers need the L1 the rings take); on the tile-ordered cross part -- gathers in whole
+    // 512-byte segments that hit L2 -- it runs at 88 % of the copy peak.
+    if (A->ring_world <= 1 && A->slice_order) return launch_spmv_sjds_bulk(A, a);
     if (a.y_ref) return fail(QBGPU_ERR_STATE, "fused way out: only the bulk-streamed kernel writes the reference's order (internal)");
     if (A->ring_world > 1) {
         if (A->ndict) return A->api_complex ? launch_sjds_ring_typed<uint8_t, double2>(A, a) : launch_sjds_ring_typed<uint8_t, double>(A, a);

@@ -70,9 +70,6 @@ __device__ __forceinline__ double ldx_hint(const double *p, uint64_t pol)
 { double v; asm volatile("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol)); return v; }
 __device__ __forceinline__ double2 ldx_hint(const double2 *p, uint64_t pol)
 { double2 v; asm volatile("ld.global.nc.L2::cache_hint.v2.f64 {%0, %1}, [%2], %3;" : "=d"(v.x), "=d"(v.y) : "l"(p), "l"(pol)); return v; }
-__device__ __forceinline__ double ldx_plain(const double *p) { double v; asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(v) : "l"(p)); return v; }
-__device__ __forceinline__ double2 ldx_plain(const double2 *p)
-{ double2 v; asm volatile("ld.global.nc.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p)); return v; }
 
 // streaming loads of the matrix arrays for the register-fed path of kernel (2)
 __device__ __forceinline__ int lds_i32(const int *p, uint64_t pol)
@@ -110,30 +107,31 @@ template <typename VecT> struct SegState {
     VecT zv, xi;          // epilogue operands, requested together with the gathers
 };
 
-// PIPE: two segments are in the consumer at a time -- the gathers of segment j+1 are issued before the products of
-// segment j are accumulated (ping-pong register sets), so a warp always has up to 2*KSEG gathers in flight.
+// Two segments are in the consumer at a time -- the gathers of segment j+1 are issued before the products of segment j
+// are accumulated (ping-pong register sets), so a warp always has up to 2*KSEG gathers in flight.
 __device__ __forceinline__ double real_of(double v) { return v; }
 __device__ __forceinline__ double real_of(double2 v) { return v.x; }
 
 // OUT: the way out of a species handle fused into this (closing, accumulating) pass: y_ref[perm_inv[row]] = out_alpha * (y, 0)
 // instead of y[row] = y (fp64 vectors only; see FusedArgs::y_ref).  The rows of a tile that share a sector of y_ref are
 // closed within microseconds of each other (neighbouring up configurations of the same tile), so L2 merges the halves.
-template <typename ValT, typename VecT, bool DOTS, bool KEEP, bool ORD, int NW, int NST, int KSEG, int MINB, bool PIPE, bool OUT = false>
-__global__ void __launch_bounds__(NW * 32, MINB)
+// The 32-row slices are visited in the order given by `order` (the tiles of down indices of a cross part, so that the
+// gathered columns of a tile stay in L2).
+template <typename ValT, typename VecT, bool DOTS, bool KEEP, int NW, int NST, int KSEG, bool OUT = false>
+__global__ void __launch_bounds__(NW * 32, 2)
 spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *__restrict__ rowptr,
                       const uint32_t *__restrict__ rowinfo, const int32_t *__restrict__ col, const ValT *__restrict__ val,
                       const VecT *__restrict__ x, const VecT *z, VecT *y, double2 alpha, double2 gamma, double2 beta,
                       int scal_mode, const double *__restrict__ sc, double *dots_out, double *partials, unsigned *ticket,
                       const double *__restrict__ vdict, const int32_t *__restrict__ order,
-                      const int32_t *__restrict__ perm_inv = nullptr, double2 *y_ref = nullptr, double2 out_alpha = {1.0, 0.0},
-                      const uint2 *__restrict__ ord_desc = nullptr)
+                      const int32_t *__restrict__ perm_inv = nullptr, double2 *y_ref = nullptr, double2 out_alpha = {1.0, 0.0})
 {
     static_assert(!OUT || (sizeof(VecT) == 8 && !DOTS), "the fused way out serves the fp64 closing pass");
     using VT = VecTraits<VecT>;
     using ST = BulkStage<ValT, KSEG>;
     using Seg = SegState<VecT>;
     static_assert(KSEG % 2 == 0 && KSEG >= 2, "diagonal k accumulates into accumulator k & 1 (the order of sjds.cu)");
-    static_assert(!PIPE || NST >= 3, "the pipelined consumer holds two stages");
+    static_assert(NST >= 3, "the pipelined consumer holds two stages");
     constexpr bool kDict = sizeof(ValT) == 1;
     using ArithT = typename std::conditional<kDict, double, ValT>::type;
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -172,31 +170,21 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
     const int stride = (int)gridDim.x * NW;                // (slice counts are < 2^31: rows < 2^31 by the int32 columns)
     const int nsl = (int)nslices;
     int p_it = (int)blockIdx.x * NW + warp;
-    // traversal item -> (slice, descriptor).  With descriptors (qbgpu_matrix::ord_desc) one 8-byte load names the slice AND, for a
-    // slice whose 32 rows all have the same length in rank = row order (most of a cross part), replaces the 128-byte rowinfo load
-    auto item_of = [&](int it) -> uint2 {
-        if constexpr (ORD) {
-            if (it >= nsl) return make_uint2(0u, 0u);
-            if (ord_desc) return ord_desc[it];
-            return make_uint2((uint32_t)order[it], 0u);
-        } else return make_uint2((uint32_t)it, 0u);
-    };
-    auto info_of = [&](uint2 d) -> uint32_t {
-        return (d.y & 0x80000000u) ? (((uint32_t)lane << 24) | (d.y & kLenMaskB)) : rowinfo[(int64_t)d.x * 32 + lane];
-    };
+    auto slice_of = [&](int it) -> uint32_t { return it < nsl ? (uint32_t)order[it] : 0u; };      // traversal item -> slice
+    auto info_of = [&](uint32_t sl) -> uint32_t { return rowinfo[(int64_t)sl * 32 + lane]; };
     bool p_more = p_it < nsl;
-    const uint2 pd = item_of(p_it);
-    int ps = (int)pd.x;
+    const uint32_t pd = slice_of(p_it);
+    int ps = (int)pd;
     uint32_t pinfo = p_more ? info_of(pd) : 0u;
     int64_t pbase = p_more ? rowptr[(int64_t)ps * 32] : 0;
     int pk = 0, poff = 0;
     // one slice ahead: requested when the producer enters a slice, consumed when it enters the next (no exposed latency)
     int n_it = p_it + stride;
-    const uint2 nd0 = item_of(n_it);
-    int ns = (int)nd0.x;
+    const uint32_t nd0 = slice_of(n_it);
+    int ns = (int)nd0;
     uint32_t ninfo = n_it < nsl ? info_of(nd0) : 0u;
     int64_t nbase = n_it < nsl ? rowptr[(int64_t)ns * 32] : 0;
-    uint2 nn_d = item_of(n_it + stride);                                             // ORD: the item after that (a dependent load)
+    uint32_t nn_d = slice_of(n_it + stride);                                         // the slice after that (a dependent load)
 
     uint32_t phases = 0;                                   // bit s = parity the consumer waits for on stage s
     int n_issued = 0;                                      // segments issued so far; segment i lives in stage i % NST
@@ -235,11 +223,11 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
             p_more = p_it < nsl;
             ps = ns; pinfo = ninfo; pbase = nbase; pk = 0; poff = 0;
             n_it += stride;
-            ns = (int)nn_d.x;
+            ns = (int)nn_d;
             const bool nv = n_it < nsl;
             ninfo = nv ? info_of(nn_d) : 0u;
             nbase = nv ? rowptr[(int64_t)ns * 32] : 0;
-            nn_d = item_of(n_it + stride);
+            nn_d = slice_of(n_it + stride);
         }
     };
 
@@ -340,30 +328,20 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
     int n_gathered = 0;
     Seg ga, gb;
     VecT xa[KSEG], xb[KSEG];
-    if constexpr (PIPE) {
-        if (n_gathered < n_issued) {
-            gather(n_gathered, ga, xa); n_gathered++;
+    if (n_gathered < n_issued) {
+        gather(n_gathered, ga, xa); n_gathered++;
 #pragma unroll 1
-            while (true) {
-                const bool hb = n_gathered < n_issued;
-                if (hb) { gather(n_gathered, gb, xb); n_gathered++; }
-                fma_phase(n_gathered - (hb ? 2 : 1), ga, xa);
-                if (p_more) issue();
-                if (!hb) break;
-                const bool ha = n_gathered < n_issued;
-                if (ha) { gather(n_gathered, ga, xa); n_gathered++; }
-                fma_phase(n_gathered - (ha ? 2 : 1), gb, xb);
-                if (p_more) issue();
-                if (!ha) break;
-            }
-        }
-    } else {
-#pragma unroll 1
-        while (n_gathered < n_issued) {
-            gather(n_gathered, ga, xa);
-            fma_phase(n_gathered, ga, xa);
-            n_gathered++;
+        while (true) {
+            const bool hb = n_gathered < n_issued;
+            if (hb) { gather(n_gathered, gb, xb); n_gathered++; }
+            fma_phase(n_gathered - (hb ? 2 : 1), ga, xa);
             if (p_more) issue();
+            if (!hb) break;
+            const bool ha = n_gathered < n_issued;
+            if (ha) { gather(n_gathered, ga, xa); n_gathered++; }
+            fma_phase(n_gathered - (ha ? 2 : 1), gb, xb);
+            if (p_more) issue();
+            if (!ha) break;
         }
     }
     if (DOTS) {
@@ -372,46 +350,25 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
     }
 }
 
-// -1 unset (environment QBGPU_SJDS_BULK, else 10), 0 = off everywhere, 10 = production (tile-ordered "cross" parts only, ring
-// chosen by vector type), 11..19 = configuration 1..9 on the cross parts, 1..9 = configuration 1..9 on EVERY sliced-jagged handle
-static int g_bulk_mode = -1;
-void set_sjds_bulk_mode(int m) { g_bulk_mode = m; }
-int sjds_bulk_mode()
-{
-    if (g_bulk_mode < 0) { const char *e = getenv("QBGPU_SJDS_BULK"); g_bulk_mode = e ? atoi(e) : 10; }
-    return g_bulk_mode;
-}
-// Does the bulk-streamed kernel serve this handle?  Measured on BASELINE config 3 (profiles/r02_bulk_sweep_*.txt): on the
-// one-pass product in the reference's order it equals the register-fed kernel at best (the gathers need the L1 the rings
-// take), on the tile-ordered cross part -- gathers in whole 512-byte segments that hit L2 -- it runs at 88 % of the copy peak.
-bool sjds_bulk_wanted(const qbgpu_matrix *A)
-{
-    const int m = sjds_bulk_mode();
-    if (m <= 0) return false;
-    return m < 10 ? true : A->slice_order != nullptr;
-}
-
-// may the closing pass over this (cross) part write the reference-order result itself?  (environment QBGPU_FUSE_WAY_OUT=0: no)
+// may the closing pass over this (cross) part write the reference-order result itself?
 bool sjds_bulk_out_fusable(const qbgpu_matrix *A)
 {
-    static int allow = -1;
-    if (allow < 0) { const char *e = getenv("QBGPU_FUSE_WAY_OUT"); allow = e ? atoi(e) != 0 : 1; }
-    return allow && A && A->format == QBGPU_FORMAT_SELL && A->slice_order && A->ring_world <= 1 && sjds_bulk_mode() >= 10;
+    return A && A->format == QBGPU_FORMAT_SELL && A->slice_order && A->ring_world <= 1;
 }
 
-template <typename ValT, typename VecT, bool DOTS, bool KEEP, bool ORD, int NW, int NST, int KSEG, int MINB, bool PIPE, bool OUT = false>
+template <typename ValT, typename VecT, bool DOTS, bool KEEP, int NW, int NST, int KSEG, bool OUT = false>
 static int launch_bulk_cfg(const qbgpu_matrix *A, const FusedArgs &a)
 {
     Context &c = ctx();
     using ST = BulkStage<ValT, KSEG>;
-    auto kern = spmv_sjds_bulk_kernel<ValT, VecT, DOTS, KEEP, ORD, NW, NST, KSEG, MINB, PIPE, OUT>;
+    auto kern = spmv_sjds_bulk_kernel<ValT, VecT, DOTS, KEEP, NW, NST, KSEG, OUT>;
     constexpr size_t smem = 64 * NW + (size_t)NW * NST * ST::BYTES;
     static int blocks_per_sm = 0;
     if (blocks_per_sm == 0) {
         QB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         QB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kern, NW * 32, smem));
         if (blocks_per_sm < 1) return fail(QBGPU_ERR_STATE, "bulk-streamed product: the stage ring does not fit in shared memory");
-        if (getenv("QBGPU_VERBOSE")) fprintf(stderr, "[qbgpu] bulk kernel NW=%d NST=%d KSEG=%d MINB=%d PIPE=%d: %d CTAs/SM, %zu B smem\n", NW, NST, KSEG, MINB, (int)PIPE, blocks_per_sm, smem);
+        if (getenv("QBGPU_VERBOSE")) fprintf(stderr, "[qbgpu] bulk kernel NW=%d NST=%d KSEG=%d: %d CTAs/SM, %zu B smem\n", NW, NST, KSEG, blocks_per_sm, smem);
     }
     const int64_t nrows = A->nrows();
     if (nrows == 0) return QBGPU_OK;
@@ -423,66 +380,47 @@ static int launch_bulk_cfg(const qbgpu_matrix *A, const FusedArgs &a)
     kern<<<grid, NW * 32, smem, c.stream>>>(nslices, nrows, A->row_lo, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val,
                                             (const VecT *)a.x, (const VecT *)a.z, (VecT *)a.y, a.alpha, a.gamma, a.beta,
                                             a.scal_mode, a.sc, a.dots, c.partials, c.ticket, A->vdict, A->slice_order,
-                                            OUT ? a.perm_inv : nullptr, OUT ? (double2 *)a.y_ref : nullptr, a.out_alpha,
-                                            ORD ? A->ord_desc : nullptr);
+                                            OUT ? a.perm_inv : nullptr, OUT ? (double2 *)a.y_ref : nullptr, a.out_alpha);
     QB_LAUNCH_COUNT();
     QB_CUDA(cudaGetLastError());
     return QBGPU_OK;
 }
 
-template <typename ValT, typename VecT, bool DOTS, bool KEEP, bool ORD>
-static int launch_bulk_mode(const qbgpu_matrix *A, const FusedArgs &a, int mode)
+template <typename ValT, typename VecT, bool DOTS, bool KEEP>
+static int launch_bulk_ring(const qbgpu_matrix *A, const FusedArgs &a)
 {
-    // (warps per CTA, stages per warp, diagonals per segment, min CTAs/SM, pipelined).  What the stage rings take from the
-    // SM's 256 KB of SRAM is lost to L1, and L1 lines are what gathers in flight are tracked in: with fp64 vectors a fat
-    // ring (106 KB per CTA, two CTAs) is best; with complex vectors (twice the lines per gather) a leaner one
-    // (profiles/r02_bulk_sweep_*.txt: 8,4,8 is 2x slower than 8,3,6 there).
-    switch (mode) {
-#ifdef QBGPU_TUNING_VARIANTS
-    case 2: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 3, 4, 2, false>(A, a);      // lean ring: 41 KB per CTA
-    case 3: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 2, 10, 3, false>(A, a);
-    case 4: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 4, 4, 2, true>(A, a);       // lean ring, pipelined
-    case 5: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 3, 8, 2, true>(A, a);
-    case 6: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 16, 3, 4, 1, true>(A, a);      // one CTA of 16 warps, 82 KB
-    case 8: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 4, 6, 2, true>(A, a);
-    case 9: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 4, 8, 2, false>(A, a);
-#endif
-    case 7: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 3, 6, 2, true>(A, a);
-    case 1: return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 4, 8, 2, true>(A, a);
-    default:                                                // production choice by vector type
-        if (sizeof(VecT) == 16) return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 3, 6, 2, true>(A, a);
-        return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, ORD, 8, 4, 8, 2, true>(A, a);
-    }
+    // (warps per CTA, stages per warp, diagonals per segment).  What the stage rings take from the SM's 256 KB of SRAM is lost
+    // to L1, and L1 lines are what gathers in flight are tracked in: with fp64 vectors a fat ring (106 KB per CTA, two CTAs)
+    // is best; with complex vectors (twice the lines per gather) a leaner one (profiles/r02_bulk_sweep_*.txt: 8,4,8 is 2x
+    // slower than 8,3,6 there).
+    if constexpr (sizeof(VecT) == 16) return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, 8, 3, 6>(A, a);
+    else return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, 8, 4, 8>(A, a);
 }
 
 template <typename ValT, typename VecT>
-static int launch_bulk_typed(const qbgpu_matrix *A, const FusedArgs &a, int mode)
+static int launch_bulk_typed(const qbgpu_matrix *A, const FusedArgs &a)
 {
     const bool dots = a.dots != nullptr;
     const bool keep = !dots && a.scal_mode == 0 && a.z == a.y && a.beta.x == 1.0 && a.beta.y == 0.0 && a.gamma.x == 0.0 && a.gamma.y == 0.0;
     if (a.y_ref) {                                          // the closing pass of a species product writes the reference's order
         if constexpr (sizeof(VecT) == 8) {
-            if (keep && A->slice_order && a.perm_inv) return launch_bulk_cfg<ValT, VecT, false, true, true, 8, 4, 8, 2, true, true>(A, a);
+            if (keep && a.perm_inv) return launch_bulk_cfg<ValT, VecT, false, true, 8, 4, 8, true>(A, a);
         }
         return fail(QBGPU_ERR_STATE, "fused way out: not the closing pass of a species handle (internal)");
     }
-    if (A->slice_order) {
-        if (keep) return launch_bulk_mode<ValT, VecT, false, true, true>(A, a, mode);
-        return dots ? launch_bulk_mode<ValT, VecT, true, false, true>(A, a, mode) : launch_bulk_mode<ValT, VecT, false, false, true>(A, a, mode);
-    }
-    if (keep) return launch_bulk_mode<ValT, VecT, false, true, false>(A, a, mode);
-    return dots ? launch_bulk_mode<ValT, VecT, true, false, false>(A, a, mode) : launch_bulk_mode<ValT, VecT, false, false, false>(A, a, mode);
+    if (keep) return launch_bulk_ring<ValT, VecT, false, true>(A, a);
+    return dots ? launch_bulk_ring<ValT, VecT, true, false>(A, a) : launch_bulk_ring<ValT, VecT, false, false>(A, a);
 }
 
-// entry: sliced-jagged handle, not a ring view.  The bulk copies may read up to 15 bytes before/after a slice's range inside
-// col[] / val[]: always inside the arrays except at their very ends, where the allocations keep 64 bytes of slack.
+// entry: tile-ordered sliced-jagged handle (slice_order set), not a ring view.  The bulk copies may read up to 15 bytes
+// before/after a slice's range inside col[] / val[]: always inside the arrays except at their very ends, where the
+// allocations keep 64 bytes of slack.
 int launch_spmv_sjds_bulk(const qbgpu_matrix *A, const FusedArgs &a)
 {
-    const int mode = sjds_bulk_mode() % 10;
-    if (A->ndict) return A->api_complex ? launch_bulk_typed<uint8_t, double2>(A, a, mode) : launch_bulk_typed<uint8_t, double>(A, a, mode);
-    if (!A->api_complex) return launch_bulk_typed<double, double>(A, a, mode);
-    if (A->val_real) return launch_bulk_typed<double, double2>(A, a, mode);
-    return launch_bulk_typed<double2, double2>(A, a, mode);
+    if (A->ndict) return A->api_complex ? launch_bulk_typed<uint8_t, double2>(A, a) : launch_bulk_typed<uint8_t, double>(A, a);
+    if (!A->api_complex) return launch_bulk_typed<double, double>(A, a);
+    if (A->val_real) return launch_bulk_typed<double, double2>(A, a);
+    return launch_bulk_typed<double2, double2>(A, a);
 }
 
 // ------------------------------------------------------------------------------- (2) block-local product, x in smem
@@ -494,14 +432,12 @@ sjds_block_smem_kernel(int64_t nrows, int64_t row_lo, int64_t D, int64_t u_lo, i
                        const uint32_t *__restrict__ rowinfo, const int32_t *__restrict__ col, const ValT *__restrict__ val,
                        const VecT *__restrict__ x, const VecT *z, VecT *y, double2 alpha, double2 gamma, double2 beta,
                        int scal_mode, const double *__restrict__ sc, const double *__restrict__ vdict, int use_bulk,
-                       const double2 *__restrict__ x_ref, const int32_t *__restrict__ perm_inv, VecT *x_out, int *imag_flag,
                        int64_t P, int64_t EP)
 {
     using VT = VecTraits<VecT>;
     constexpr bool kDict = sizeof(ValT) == 1;
     using ArithT = typename std::conditional<kDict, double, ValT>::type;
     constexpr int NWARP = NT / 32;
-    bool any_imag = false;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ double sdict[kDict ? 256 : 1];
     __shared__ __align__(8) unsigned long long xbar_storage;
@@ -541,32 +477,8 @@ sjds_block_smem_kernel(int64_t nrows, int64_t row_lo, int64_t D, int64_t u_lo, i
         const int64_t c0 = (u_lo + ub) * D;                 // first column (= first global row) of the block
         const int64_t r0 = c0 - row_lo, r1 = r0 + D;        // local rows of the block
         __syncthreads();                                    // every warp has finished reading the previous block from xs
-        bool x_ready = true, staged = false;
-        if constexpr (sizeof(VecT) == 8) {
-            if (x_ref) {
-                // the way in, fused: this block of the internal order gathered from the complex vector in the reference's order
-                // (the rows of one odd-site label are a rectangle here: the neighbouring blocks read the other halves of the same
-                // sectors at about the same time, so L2 serves them); kept for pass 2 in x_out; loads of four rounds first
-                constexpr int R = 4;
-                for (int64_t j0 = threadIdx.x; j0 < D; j0 += (int64_t)R * NT) {
-                    int32_t r[R];
-                    double2 v[R];
-#pragma unroll
-                    for (int u = 0; u < R; u++) { const int64_t j = j0 + (int64_t)u * NT; if (j < D) r[u] = perm_inv[c0 + j]; }
-#pragma unroll
-                    for (int u = 0; u < R; u++) { const int64_t j = j0 + (int64_t)u * NT; if (j < D) v[u] = ldx_plain(x_ref + r[u]); }
-#pragma unroll
-                    for (int u = 0; u < R; u++) {
-                        const int64_t j = j0 + (int64_t)u * NT;
-                        if (j < D) { xs[j] = v[u].x; x_out[c0 + j] = v[u].x; any_imag = any_imag || (v[u].y != 0.0); }
-                    }
-                }
-                __syncthreads();
-                staged = true;
-            }
-        }
-        if (staged) {
-        } else if (use_bulk) {
+        bool x_ready = true;
+        if (use_bulk) {
             if (threadIdx.x == 0) {
                 fence_proxy_async_smem();
                 const uint32_t bytes = (uint32_t)(D * (int64_t)sizeof(VecT));
@@ -657,245 +569,7 @@ sjds_block_smem_kernel(int64_t nrows, int64_t row_lo, int64_t D, int64_t u_lo, i
         }
         if (!x_ready) { mbar_wait(xbar, xphase); xphase ^= 1u; }                           // (a warp without any slice in this block)
     }
-    if (any_imag && imag_flag) *(volatile int *)imag_flag = 1;
 }
-
-// ------------------------------------------------------------------- (3) block-local product, x in smem AND the stream in rings
-// Kernel (2) feeds the matrix stream through registers: 1024 threads x 4 diagonals = 48 KB in flight per SM is all its 64
-// registers per thread allow, just short of what 1/148 of the HBM bandwidth times the loaded DRAM latency asks for (5.3 TB/s,
-// long-scoreboard stalls 11.8 per issue: profiles/r02_ncu_full_mv_reference_order_hubbard4x4.csv).  Here the two halves of this
-// file meet: the block of x sits in shared memory (one bulk copy per block, its successor prefetched into L2), and the matrix
-// stream arrives through the per-warp stage rings of kernel (1) -- 24 stages = 79 KB in flight with 8 warps -- so nothing a warp
-// touches in its loop is further away than shared memory.  The producer cursor runs ahead across block boundaries (the stream
-// does not depend on x); the consumers meet at a CTA barrier per block.  Same accumulation order as kernels (1) and (2).
-template <typename ValT, typename VecT, int NW, int NST, int KSEG>
-__global__ void __launch_bounds__(NW * 32, 1)
-sjds_block_bulk_kernel(int64_t nrows, int64_t row_lo, int64_t D, int64_t u_lo, int64_t u_cnt, const int64_t *__restrict__ rowptr,
-                       const uint32_t *__restrict__ rowinfo, const int32_t *__restrict__ col, const ValT *__restrict__ val,
-                       const VecT *__restrict__ x, const VecT *z, VecT *y, double2 alpha, double2 gamma, double2 beta,
-                       int scal_mode, const double *__restrict__ sc, const double *__restrict__ vdict, uint32_t xs_off, uint32_t ring_off)
-{
-    using VT = VecTraits<VecT>;
-    using ST = BulkStage<ValT, KSEG>;
-    static_assert(KSEG % 2 == 0 && KSEG >= 2, "diagonal k accumulates into accumulator k & 1 (the order of sjds.cu)");
-    constexpr bool kDict = sizeof(ValT) == 1;
-    using ArithT = typename std::conditional<kDict, double, ValT>::type;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ double sdict[kDict ? 256 : 1];
-    if (kDict) { for (int i = threadIdx.x; i < 256; i += NW * 32) sdict[i] = vdict[i]; }
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const VecT *xs = (const VecT *)(smem_raw + xs_off);
-    unsigned char *wbase = smem_raw + ring_off + (size_t)warp * NST * ST::BYTES;
-    const uint32_t bar0 = smem_u32(smem_raw + 64 * warp);       // [NW][8] stage barriers, then the barrier of the x block
-    const uint32_t xbar = smem_u32(smem_raw + 64 * NW);
-    if (lane == 0) {
-#pragma unroll
-        for (int st = 0; st < NST; st++) mbar_init(bar0 + 8 * st, 1);
-        if (warp == 0) mbar_init(xbar, 1);
-        mbar_fence_init();
-    }
-    if (scal_mode != 0) {
-        const double sx = sc[0], sz = sc[1], bprev = sc[2];
-        alpha = make_double2(sx, 0.0);
-        gamma = make_double2(0.0, 0.0);
-        beta = scal_mode == 1 ? make_double2(-bprev * sz, 0.0) : make_double2(1.0, 0.0);
-    }
-    __shared__ double2 s_scal[3];
-    if (threadIdx.x == 0) { s_scal[0] = alpha; s_scal[1] = gamma; s_scal[2] = beta; }
-    __syncthreads();
-    const bool use_gamma = (s_scal[1].x != 0.0 || s_scal[1].y != 0.0);
-    const bool use_beta = (s_scal[2].x != 0.0 || s_scal[2].y != 0.0);
-    const uint64_t pol_s = pol_evict_first();
-    const uint32_t xbytes = (uint32_t)(D * (int64_t)sizeof(VecT));
-
-    auto s_first = [&](int64_t ub) -> int { return (int)(((u_lo + ub) * D - row_lo) >> 5); };
-    auto s_last = [&](int64_t ub) -> int { return (int)(((u_lo + ub + 1) * D - row_lo - 1) >> 5); };
-    // successor of (ub, s) in this warp's sequence: the slices s_first(ub) + warp, + NW, ... of the CTA's blocks ub, ub + grid, ...
-    auto next_slice = [&](int64_t &ub, int &s) -> bool {
-        s += NW;
-        while (ub < u_cnt) {
-            if (s <= s_last(ub)) return true;
-            ub += gridDim.x;
-            if (ub < u_cnt) s = s_first(ub) + warp;
-        }
-        return false;
-    };
-    // ---- producer cursor (current slice) and the slice after it, whose row metadata is requested one slice ahead
-    int64_t pub = blockIdx.x;
-    int ps = (pub < u_cnt ? s_first(pub) : 0) + warp - NW;
-    bool p_more = next_slice(pub, ps);
-    uint32_t pinfo = p_more ? rowinfo[(int64_t)ps * 32 + lane] : 0u;
-    int64_t pbase = p_more ? rowptr[(int64_t)ps * 32] : 0;
-    int pk = 0, poff = 0;
-    int64_t nub = pub;
-    int ns = ps;
-    bool n_more = p_more && next_slice(nub, ns);
-    uint32_t ninfo = n_more ? rowinfo[(int64_t)ns * 32 + lane] : 0u;
-    int64_t nbase = n_more ? rowptr[(int64_t)ns * 32] : 0;
-    uint32_t phases = 0;
-    int n_issued = 0, n_cons = 0;
-
-    auto issue = [&]() {
-        const int st = n_issued % NST;
-        n_issued++;
-        const int len = (int)(pinfo & kLenMaskB);
-        const int maxlen = __shfl_sync(0xffffffffu, len, 0);
-        const int hi = min(len, pk + KSEG), lo = min(len, pk);
-        const int cnt = (int)__reduce_add_sync(0xffffffffu, (unsigned)(hi - lo));
-        unsigned char *sb = wbase + (size_t)st * ST::BYTES;
-        __syncwarp();
-        ((uint32_t *)(sb + 32))[lane] = pinfo;
-        if (lane == 0) {
-            const int64_t beg = pbase + poff;
-            int *hdr = (int *)sb;
-            *(int64_t *)hdr = beg; hdr[2] = cnt; hdr[3] = pk; hdr[4] = ps; hdr[5] = (int)pub;
-            if (cnt > 0) {
-                fence_proxy_async_smem();
-                const int64_t c0 = beg & ~3LL, c1 = (beg + cnt + 3) & ~3LL;
-                const int64_t v0 = beg & ~(int64_t)(ST::VALIGN - 1), v1 = (beg + cnt + ST::VALIGN - 1) & ~(int64_t)(ST::VALIGN - 1);
-                const uint32_t cb = (uint32_t)(c1 - c0) * 4u, vb = (uint32_t)((v1 - v0) * (int64_t)sizeof(ValT));
-                const uint32_t bar = bar0 + 8 * st;
-                mbar_expect_tx(bar, cb + vb);
-                bulk_g2s(smem_u32(sb + ST::HDR_BYTES), col + c0, cb, bar, pol_s);
-                bulk_g2s(smem_u32(sb + ST::HDR_BYTES + ST::COL_BYTES), val + v0, vb, bar, pol_s);
-            }
-        }
-        __syncwarp();
-        poff += cnt;
-        pk += KSEG;
-        if (pk >= maxlen) {                                 // slice finished (an empty slice is one empty segment)
-            p_more = n_more;
-            pub = nub; ps = ns; pinfo = ninfo; pbase = nbase; pk = 0; poff = 0;
-            if (n_more) {
-                n_more = next_slice(nub, ns);
-                ninfo = n_more ? rowinfo[(int64_t)ns * 32 + lane] : 0u;
-                nbase = n_more ? rowptr[(int64_t)ns * 32] : 0;
-            }
-        }
-    };
-
-#pragma unroll 1
-    for (int st = 0; st < NST && p_more; st++) issue();
-
-    VecT acc0 = VT::zero(), acc1 = VT::zero(), zv = VT::zero();
-    uint32_t xphase = 0;
-#pragma unroll 1
-    for (int64_t ub = blockIdx.x; ub < u_cnt; ub += gridDim.x) {
-        const int64_t c0 = (u_lo + ub) * D;                 // first column (= first global row) of the block
-        const int64_t r0 = c0 - row_lo, r1 = r0 + D;        // local rows of the block
-        __syncthreads();                                    // every warp has finished reading the previous block from xs
-        if (threadIdx.x == 0) {
-            fence_proxy_async_smem();
-            mbar_expect_tx(xbar, xbytes);
-            bulk_g2s_plain(smem_u32(xs), x + c0, xbytes, xbar);
-            if (ub + gridDim.x < u_cnt)                     // the CTA's next block: into L2 now, so that the switch finds it there
-                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(x + c0 + (int64_t)gridDim.x * D), "r"(xbytes) : "memory");
-        }
-        mbar_wait(xbar, xphase);
-        xphase ^= 1u;
-#pragma unroll 1
-        while (n_cons < n_issued) {
-            const int st = n_cons % NST;
-            unsigned char *sb = wbase + (size_t)st * ST::BYTES;
-            if (((const int *)sb)[5] != (int)ub) break;     // the next segment belongs to a later block
-            const int4 h = *(const int4 *)sb;               // beg (lo, hi), cnt, k0
-            const int s = ((const int *)sb)[4];
-            const uint32_t info = ((const uint32_t *)(sb + 32))[lane];
-            const int len = (int)(info & kLenMaskB);
-            const int maxlen = __shfl_sync(0xffffffffu, len, 0);
-            const int minlen = __shfl_sync(0xffffffffu, len, 31);
-            const int cnt = h.z, k0 = h.w;
-            const int64_t row = (int64_t)s * 32 + (info >> 24);
-            const bool mine = row >= r0 && row < r1;        // a slice that straddles two blocks is streamed for both
-            if (k0 == 0) {
-                acc0 = VT::zero(); acc1 = VT::zero();
-                if (mine && use_beta) zv = z[row];          // requested with the first segment, used after the last
-            }
-            if (cnt > 0) {
-                mbar_wait(bar0 + 8 * st, (phases >> st) & 1u);
-                phases ^= 1u << st;
-                const int32_t *scol = (const int32_t *)(sb + ST::HDR_BYTES) + (h.x & 3) + lane;
-                const ValT *sval = (const ValT *)(sb + ST::HDR_BYTES + ST::COL_BYTES) + (h.x & (ST::VALIGN - 1)) + lane;
-                if (k0 + KSEG <= minlen) {                  // full segment: entry (u, lane) at u*32 + lane
-                    int idx[KSEG];
-#pragma unroll
-                    for (int u = 0; u < KSEG; u++) idx[u] = mine ? (int)((int64_t)scol[u * 32] - c0) : 0;
-#pragma unroll
-                    for (int u = 0; u < KSEG; u++) {
-                        const VecT xv = xs[idx[u]];
-                        ArithT w;
-                        if constexpr (kDict) w = sdict[sval[u * 32]]; else w = sval[u * 32];
-                        if (u & 1) mac(acc1, w, xv); else mac(acc0, w, xv);
-                    }
-                } else {
-                    // ragged segment, in batches like the full one (offsets, then all columns, then all gathers, then the
-                    // products): lanes without diagonal k0 + u read entry 0 of the stage and x[0] of the block and skip the fma.
-                    // (A first version branched per diagonal: 8 serialised LDS -> LDS -> DFMA chains per segment, and two
-                    // thirds of this part's segments are ragged: profiles/r02_ncu_block_bulk_first_version.txt)
-                    bool a[KSEG];
-                    int o[KSEG], idx[KSEG];
-                    int off = 0;
-#pragma unroll
-                    for (int u = 0; u < KSEG; u++) {
-                        a[u] = (k0 + u < len) && mine;
-                        o[u] = a[u] ? off : 0;
-                        off += __popc(__ballot_sync(0xffffffffu, k0 + u < len));
-                    }
-#pragma unroll
-                    for (int u = 0; u < KSEG; u++) { const int c = scol[o[u]]; idx[u] = a[u] ? (int)((int64_t)c - c0) : 0; }
-                    VecT xv[KSEG];
-                    ArithT w[KSEG];
-#pragma unroll
-                    for (int u = 0; u < KSEG; u++) xv[u] = xs[idx[u]];
-#pragma unroll
-                    for (int u = 0; u < KSEG; u++) { if constexpr (kDict) w[u] = sdict[sval[o[u]]]; else w[u] = sval[o[u]]; }
-#pragma unroll
-                    for (int u = 0; u < KSEG; u++) {
-                        if (a[u]) { if (u & 1) mac(acc1, w[u], xv[u]); else mac(acc0, w[u], xv[u]); }
-                    }
-                }
-            }
-            if (k0 + KSEG >= maxlen && mine) {              // last segment of the slice: the epilogue of sjds.cu
-                const VecT acc = VT::add(acc0, acc1);
-                VecT out = VT::scale(s_scal[0], acc);
-                if (use_gamma) out = VT::add(out, VT::scale(s_scal[1], xs[row - r0]));
-                if (use_beta) out = VT::add(out, VT::scale(s_scal[2], zv));
-                y[row] = out;
-            }
-            __syncwarp();                                   // every lane is done with the stage before it is refilled
-            n_cons++;
-            if (p_more) issue();
-        }
-    }
-}
-
-template <typename ValT, typename VecT, int NW, int NST, int KSEG>
-static int launch_block_bulk_cfg(const qbgpu_matrix *A, const FusedArgs &a, int64_t D, bool probe_only = false)
-{
-    Context &c = ctx();
-    using ST = BulkStage<ValT, KSEG>;
-    auto kern = sjds_block_bulk_kernel<ValT, VecT, NW, NST, KSEG>;
-    const size_t xs_off = ((size_t)64 * NW + 16 + 127) / 128 * 128;
-    const size_t ring_off = xs_off + ((size_t)D * sizeof(VecT) + 127) / 128 * 128;
-    const size_t smem = ring_off + (size_t)NW * NST * ST::BYTES;
-    if (smem > 227 * 1024 || (D * (int64_t)sizeof(VecT)) % 16 != 0 || D * (int64_t)sizeof(VecT) >= (1 << 20)) return probe_only ? 1 : fail(QBGPU_ERR_STATE, "block-local bulk product: block and rings do not fit in shared memory");
-    if (probe_only) return 0;
-    static size_t smem_set = 0;
-    if (smem_set < smem) { QB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); smem_set = smem; }
-    const int64_t u_lo = A->row_lo / D, u_cnt = A->nrows() / D;
-    if (u_cnt == 0) return QBGPU_OK;
-    const int64_t cap = (int64_t)c.num_sms;                 // one CTA per SM
-    const int grid = (int)(u_cnt < cap ? u_cnt : cap);
-    kern<<<grid, NW * 32, smem, c.stream>>>(A->nrows(), A->row_lo, D, u_lo, u_cnt, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val,
-                                            (const VecT *)a.x, (const VecT *)a.z, (VecT *)a.y, a.alpha, a.gamma, a.beta, a.scal_mode, a.sc,
-                                            A->vdict, (uint32_t)xs_off, (uint32_t)ring_off);
-    QB_LAUNCH_COUNT();
-    QB_CUDA(cudaGetLastError());
-    return QBGPU_OK;
-}
-
-static int g_block_smem_variant = -1;
-void set_block_smem_variant(int v) { g_block_smem_variant = v; }
 
 template <typename ValT, typename VecT, int NT, int U, int MINB>
 static int launch_block_smem_cfg(const qbgpu_matrix *A, const FusedArgs &a, int64_t D)
@@ -917,74 +591,33 @@ static int launch_block_smem_cfg(const qbgpu_matrix *A, const FusedArgs &a, int6
     const int64_t cap = (int64_t)c.num_sms * bps;
     const int grid = (int)(u_cnt < cap ? u_cnt : cap);
     const int use_bulk = ((D * (int64_t)sizeof(VecT)) % 16 == 0 && D * (int64_t)sizeof(VecT) < (1 << 20)) ? 1 : 0;
-    const bool fuse_in = a.x_ref != nullptr && sizeof(VecT) == 8;      // (the caller only sets x_ref for fp64 vectors)
     kern<<<grid, NT, smem, c.stream>>>(A->nrows(), A->row_lo, D, u_lo, u_cnt, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val,
                                        (const VecT *)a.x, (const VecT *)a.z, (VecT *)a.y, a.alpha, a.gamma, a.beta, a.scal_mode, a.sc,
-                                       A->vdict, use_bulk, fuse_in ? (const double2 *)a.x_ref : nullptr, a.perm_inv,
-                                       fuse_in ? (VecT *)const_cast<void *>(a.x) : nullptr, a.imag_flag, A->period_slices, A->period_entries);
+                                       A->vdict, use_bulk, A->period_slices, A->period_entries);
     QB_LAUNCH_COUNT();
     QB_CUDA(cudaGetLastError());
     return QBGPU_OK;
 }
 
-template <typename ValT, typename VecT>
-static int launch_block_smem_typed(const qbgpu_matrix *A, const FusedArgs &a, int64_t D)
-{
-    // default 1: the register-fed kernel (2).  20 = the ring-fed kernel (3) with 24 warps x 2 stages x 6 diagonals where block +
-    // rings fit in shared memory, else (2): measured on BASELINE config 3 it is 2 % faster alone (7.72 against 7.89 ms,
-    // profiles/r02_block_bulk_sweep_hubbard4x4.txt) and a wash inside the whole product (16.61 against 16.66 ms), so the
-    // simpler kernel stays the default.  10..18: other ring shapes (tuning builds).
-    if (g_block_smem_variant < 0) g_block_smem_variant = getenv("QBGPU_BLOCK_SMEM") ? atoi(getenv("QBGPU_BLOCK_SMEM")) : 1;
-    switch (g_block_smem_variant) {
-    case 20: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 24, 2, 6>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 24, 2, 6>(A, a, D); break;
-#ifdef QBGPU_TUNING_VARIANTS
-    case 2: return launch_block_smem_cfg<ValT, VecT, 1024, 4, 1>(A, a, D);
-    case 3: return launch_block_smem_cfg<ValT, VecT, 512, 16, 1>(A, a, D);
-    case 4: return launch_block_smem_cfg<ValT, VecT, 768, 8, 1>(A, a, D);
-    case 5: return launch_block_smem_cfg<ValT, VecT, 512, 8, 1>(A, a, D);
-    case 6: return launch_block_smem_cfg<ValT, VecT, 1024, 6, 1>(A, a, D);
-#endif
-    case 7: return launch_block_smem_cfg<ValT, VecT, 1024, 8, 1>(A, a, D);
-    // 10..: the stream through stage rings (kernel (3)); needs block + rings within 227 KB and no fused way in
-    case 10: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 8, 4, 8>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 8, 4, 8>(A, a, D); break;
-    case 11: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 12, 3, 8>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 12, 3, 8>(A, a, D); break;
-    case 12: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 16, 2, 8>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 16, 2, 8>(A, a, D); break;
-    case 13: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 8, 5, 6>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 8, 5, 6>(A, a, D); break;
-    case 14: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 16, 3, 4>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 16, 3, 4>(A, a, D); break;
-    case 15: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 8, 3, 10>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 8, 3, 10>(A, a, D); break;
-    case 16: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 32, 2, 4>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 32, 2, 4>(A, a, D); break;
-    case 17: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 24, 2, 6>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 24, 2, 6>(A, a, D); break;
-    case 18: if (!a.x_ref && launch_block_bulk_cfg<ValT, VecT, 20, 3, 4>(A, a, D, true) == 0) return launch_block_bulk_cfg<ValT, VecT, 20, 3, 4>(A, a, D); break;
-    default: break;
-    }
-    return launch_block_smem_cfg<ValT, VecT, 1024, 4, 1>(A, a, D);
-}
-
 // Can the block-local kernel serve this handle?  (sliced-jagged layout, rows = whole blocks of D, block fits in shared memory)
-// Default: blocks up to 112 KB (two CTAs per SM, or one with half of the SRAM left as L1: the matrix stream is register-fed
-// and its loads in flight are tracked in L1 lines).  A 206 KB block (BASELINE config 3 with complex vectors) leaves 28 KB of
-// L1 and the stream then stalls at 3.2 TB/s (profiles/r02_ncu_species_stored_first_bulk_kernels_hubbard4x4.csv): 13.6 ms
-// against 10.1 ms for the plain kernel, so such blocks take the plain kernel unless QBGPU_BLOCK_SMEM_MAX_KB says otherwise.
+// Blocks up to 112 KB (two CTAs per SM, or one with half of the SRAM left as L1: the matrix stream is register-fed and its
+// loads in flight are tracked in L1 lines).  A 206 KB block (BASELINE config 3 with complex vectors) leaves 28 KB of L1 and
+// the stream then stalls at 3.2 TB/s (profiles/r02_ncu_species_stored_first_bulk_kernels_hubbard4x4.csv): 13.6 ms against
+// 10.1 ms for the plain kernel, so such blocks take the plain kernel.
 bool block_smem_applicable(const qbgpu_matrix *A, int64_t D)
 {
-    if (g_block_smem_variant == 0) return false;
-    if (g_block_smem_variant < 0 && getenv("QBGPU_BLOCK_SMEM") && atoi(getenv("QBGPU_BLOCK_SMEM")) == 0) return false;
+    constexpr size_t kMaxBlockBytes = 112 * 1024;
     if (A->format != QBGPU_FORMAT_SELL || D <= 0 || A->row_lo % D != 0 || A->nrows() % D != 0) return false;
-    size_t max_kb = 112;
-    if (const char *e = getenv("QBGPU_BLOCK_SMEM_MAX_KB")) max_kb = (size_t)atoi(e);
-    if (max_kb > 220) max_kb = 220;
-    return (size_t)D * A->vec_bytes() <= max_kb * 1024;
+    return (size_t)D * A->vec_bytes() <= kMaxBlockBytes;
 }
-
-bool sjds_block_variant_ok() { return g_block_smem_variant != 0; }
 
 int launch_spmv_block_smem(const qbgpu_matrix *A, const FusedArgs &a, int64_t D)
 {
     if (a.dots) return fail(QBGPU_ERR_ARG, "block-local product: the running dots belong to the closing pass");
-    if (A->ndict) return A->api_complex ? launch_block_smem_typed<uint8_t, double2>(A, a, D) : launch_block_smem_typed<uint8_t, double>(A, a, D);
-    if (!A->api_complex) return launch_block_smem_typed<double, double>(A, a, D);
-    if (A->val_real) return launch_block_smem_typed<double, double2>(A, a, D);
-    return launch_block_smem_typed<double2, double2>(A, a, D);
+    if (A->ndict) return A->api_complex ? launch_block_smem_cfg<uint8_t, double2, 1024, 4, 1>(A, a, D) : launch_block_smem_cfg<uint8_t, double, 1024, 4, 1>(A, a, D);
+    if (!A->api_complex) return launch_block_smem_cfg<double, double, 1024, 4, 1>(A, a, D);
+    if (A->val_real) return launch_block_smem_cfg<double, double2, 1024, 4, 1>(A, a, D);
+    return launch_block_smem_cfg<double2, double2, 1024, 4, 1>(A, a, D);
 }
 
 }  // namespace qb

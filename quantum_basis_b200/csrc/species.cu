@@ -349,21 +349,6 @@ __global__ void __launch_bounds__(kPBlock) species_fill_kernel(SpeciesView V, in
 }
 
 
-// traversal order of the cross part's 32-row slices: by (tile of the slice's first down index, slice index)
-__global__ void __launch_bounds__(256) ord_desc_kernel(int64_t nsl, const int32_t *__restrict__ order, const uint32_t *__restrict__ rowinfo, uint2 *out)
-{
-    const int lane = threadIdx.x & 31;
-    const int64_t wpb = blockDim.x / 32;
-    for (int64_t it = (int64_t)blockIdx.x * wpb + (threadIdx.x >> 5); it < nsl; it += (int64_t)gridDim.x * wpb) {
-        const int s = order[it];
-        const uint32_t info = rowinfo[(int64_t)s * 32 + lane];
-        const uint32_t len0 = __shfl_sync(0xffffffffu, info, 0) & 0xFFFFFFu;
-        const bool same = (info >> 24) == (uint32_t)lane && (info & 0xFFFFFFu) == len0;
-        const bool uni = __all_sync(0xffffffffu, same);
-        if (lane == 0) out[it] = make_uint2((uint32_t)s, uni ? (0x80000000u | len0) : 0u);
-    }
-}
-
 static void make_slice_order(int64_t n, int64_t Dd, int W, std::vector<int32_t> &order)
 {
     const int64_t ns = (n + 31) / 32;
@@ -411,8 +396,7 @@ int species_build_stored(qbgpu_matrix_t *out, const HostTables &T, const ModelPa
         int64_t g = 32, r = Dd % 32;
         while (r) { const int64_t t = g % r; g = r; r = t; }               // gcd(32, Dd)
         const int64_t pb = 32 / g;                                          // blocks per period
-        static const bool off = getenv("QBGPU_PERIODIC_META") && atoi(getenv("QBGPU_PERIODIC_META")) == 0;
-        if (!off && (u_hi - u_lo) >= 2 * pb) { A->period_slices = pb * Dd / 32; A->period_entries = pb * (S->tot_d + Dd); }
+        if ((u_hi - u_lo) >= 2 * pb) { A->period_slices = pb * Dd / 32; A->period_entries = pb * (S->tot_d + Dd); }
     }
 #define QB_CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { qbgpu_destroy(A); return cuda_fail(e_, #call, __FILE__, __LINE__); } } while (0)
     QB_CU(cudaMalloc(&A->rowptr, sizeof(int64_t) * (nloc + 1)));
@@ -434,7 +418,7 @@ int species_build_stored(qbgpu_matrix_t *out, const HostTables &T, const ModelPa
     QB_CU(cudaStreamSynchronize(c.stream));
     QB_CU(cudaGetLastError());
     // layout: always the sliced-jagged kernels (the traversal order of the cross part exists only there)
-    if ((flags & QBGPU_VALUE_DICT) || getenv("QBGPU_VALUE_DICT")) {
+    if (flags & QBGPU_VALUE_DICT) {
         int rc = value_dict_encode(A);
         if (rc == QBGPU_OK) rc = value_dict_encode(C);
         if (rc) { qbgpu_destroy(A); return rc; }
@@ -443,18 +427,6 @@ int species_build_stored(qbgpu_matrix_t *out, const HostTables &T, const ModelPa
     std::vector<int32_t> order;
     make_slice_order(nloc, Dd, S->tile, order);
     QB_CU(upload(&C->slice_order, order.data(), order.size(), c.stream));
-    {   // traversal descriptors of the cross part (sjds_bulk.cu): most of its slices hold 32 rows of one up configuration, all
-        // with the same number of up hops.  Opt-in (QBGPU_ORD_DESC=1): measured on BASELINE config 3 it saves 0.5 GB of rowinfo
-        // traffic per product and is still 0.12 ms SLOWER through MultMv (16.75 against 16.63 ms on the same box; the Lanczos
-        // loop gains 1 %): the rowinfo loads were prefetched a slice ahead anyway, the synthesis adds producer instructions.
-        static const bool on = getenv("QBGPU_ORD_DESC") && atoi(getenv("QBGPU_ORD_DESC")) != 0;
-        const int64_t nsl = (int64_t)order.size();
-        if (on && nsl > 0 && C->rowinfo) {
-            QB_CU(cudaMalloc(&C->ord_desc, sizeof(uint2) * (size_t)nsl));
-            ord_desc_kernel<<<(int)std::min<int64_t>((nsl + 7) / 8, 148 * 16), 256, 0, c.stream>>>(nsl, C->slice_order, C->rowinfo, C->ord_desc);
-            QB_LAUNCH_COUNT();
-        }
-    }
     QB_CU(cudaStreamSynchronize(c.stream));
     QB_CU(cudaGetLastError());
 #undef QB_CU
@@ -578,7 +550,7 @@ __device__ __forceinline__ void local_scalars(int scal_mode, const double *sc, d
     }
 }
 
-// BLOCK = 256, grid-stride (default), or BLOCK = 1024 with one contiguous range of rows per CTA (QBGPU_KRON_LOCAL=1: one
+// BLOCK = 256, grid-stride (default), or BLOCK = 1024 with one contiguous range of rows per CTA (variant 1: one
 // CTA per SM then walks through the blocks x[iu, :] one after the other, so that L1 holds the block being gathered from).
 // Rows [row0, row0 + nloc) of the operator (a shard: whole up configurations); x is the full vector, y and z the local rows.
 template <typename VecT, int BLOCK, bool RANGES, bool UNI>
@@ -615,7 +587,7 @@ kron_local_kernel(SpeciesView V, int64_t row0, int64_t nloc, const double *__res
     }
 }
 
-// QBGPU_KRON_LOCAL=2: one CTA of 1024 threads per up configuration; the block x[iu, :] (D_dn entries: 206 KB of complex
+// variant 2: one CTA of 1024 threads per up configuration; the block x[iu, :] (D_dn entries: 206 KB of complex
 // numbers for the 4x4 lattice) is staged in shared memory once and every gather of the block's rows reads it from there.
 template <typename VecT, bool UNI>
 __global__ void __launch_bounds__(1024, 1)
@@ -768,7 +740,7 @@ kron_cross_kernel(SpeciesView V, CrossItems I, int64_t u_lo, int64_t c_lo, int64
     }
 }
 
-static int g_kron_local_variant = -1;      // -1: not chosen yet (environment QBGPU_KRON_LOCAL, else 0)
+static int g_kron_local_variant = 0;       // qbgpu_debug_set_variant(1000 + v)
 void set_kron_local_variant(int v) { g_kron_local_variant = v; }
 
 template <typename VecT, bool DOTS, bool FILTER, bool FIRST, bool UNI = false>
@@ -801,9 +773,8 @@ static int launch_kron(const qbgpu_matrix *A, const FusedArgs &a)
     const SpeciesView V = view_of(S);
     const bool filter = A->sp_col_lo >= 0;
     if (A->sp_has_local) {
-        // pass 1 variants (QBGPU_KRON_LOCAL): 0 grid-stride / 256 threads (default), 1 contiguous row ranges / 1024 threads,
+        // pass 1 variants: 0 grid-stride / 256 threads (default), 1 contiguous row ranges / 1024 threads,
         // 2 block staged in shared memory (falls back to 0 when D_dn entries do not fit)
-        if (g_kron_local_variant < 0) g_kron_local_variant = getenv("QBGPU_KRON_LOCAL") ? atoi(getenv("QBGPU_KRON_LOCAL")) : 0;
         const int variant = g_kron_local_variant;
         const size_t stage_bytes = sizeof(VecT) * (size_t)S->Dd;
         const bool uni = S->amp_uni != 0.0;              // every bond with the same multiplicity: amplitude as an argument
@@ -857,8 +828,8 @@ int launch_spmv_species(const qbgpu_matrix *A, const FusedArgs &a)
     qbgpu_matrix L = *A;                                    // plain views: the production kernels see two ordinary matrices
     L.sp = nullptr; L.second = nullptr; L.perm = nullptr; L.perm_inv = nullptr;
     FusedArgs a1 = a;
-    a1.dots = nullptr;                                      // (a1 keeps x_ref / perm_inv / imag_flag: the fused way in belongs to pass 1)
-    a1.y_ref = nullptr;                                     // (... and the fused way out to pass 2)
+    a1.dots = nullptr;
+    a1.y_ref = nullptr;                                     // (the fused way out belongs to pass 2)
     // pass 1: every gather stays inside the block of one up configuration -> the block of x lives in shared memory
     QB_TRY(launch_spmv(&L, a1));                            // (block_D set: launch_spmv_sjds takes the block-local kernel when it fits)
     qbgpu_matrix C = *A->second;
@@ -1017,8 +988,7 @@ static int launch_to_native_tiled(const qbgpu_matrix *A, const void *src, void *
 static bool to_native_tiled_ok(const qbgpu_matrix *A, size_t elem)
 {
     const Species *S = (const Species *)A->sp;
-    static const bool off = getenv("QBGPU_PERM_TILED") && atoi(getenv("QBGPU_PERM_TILED")) == 0;
-    return !off && S && S->blk_start && S->blk_desc && S->nblk > 0 && elem * (size_t)S->blk_max_rows <= 200 * 1024;
+    return S && S->blk_start && S->blk_desc && S->nblk > 0 && elem * (size_t)S->blk_max_rows <= 200 * 1024;
 }
 
 // the way in of the real-content product: dst[p] = Re src[perm_inv[p]]; *flag = 1 as soon as one imaginary part is not zero
@@ -1127,9 +1097,6 @@ int mv_species(qbgpu_matrix *A, double2 alpha, const void *x, double2 beta, void
     // way out widens the result.  Exact: the real parts go through the identical fma sequence, the imaginary parts are exact
     // zeros either way.  A vector with any non-zero imaginary part takes the complex passes (QBGPU_MV_REAL_MODE=0: always).
     static const bool real_mode_on = !(getenv("QBGPU_MV_REAL_MODE") && atoi(getenv("QBGPU_MV_REAL_MODE")) == 0);
-    // opt-in (QBGPU_FUSE_WAY_IN=1), measured on BASELINE config 3 and SLOWER: the gathers of the staging phase are exposed in every
-    // block (pass 1: 7.31 -> 8.96 ms) while the tiled way in of its own costs 1.24 ms
-    static const bool fuse_in_on = getenv("QBGPU_FUSE_WAY_IN") && atoi(getenv("QBGPU_FUSE_WAY_IN")) != 0;
     const Species *S = (const Species *)A->sp;
     int *flag = (int *)(c.scal_dev + 57);
     auto complex_route = [&]() -> int {
@@ -1148,55 +1115,38 @@ int mv_species(qbgpu_matrix *A, double2 alpha, const void *x, double2 beta, void
     if (cplx && A->val_real && real_mode_on) {
         qbgpu_matrix R = *A;                                // same arrays, fp64 vectors
         R.api_complex = false;
-        qbgpu_matrix Lp = R;                                // (what launch_spmv_species will hand to pass 1)
-        Lp.sp = nullptr; Lp.second = nullptr;
-        // The way in can ride in pass 1 when that pass is the block-local kernel (it stages every block of x in shared memory
-        // anyway: it then gathers the block from the reference-order vector itself and leaves the fp64 copy behind for pass 2)
-        // and y is not read (beta == 0: the whole product can be repeated on the complex route if an imaginary part turns up).
-        const bool fuse = fuse_in_on && !use_beta && !S->matfree && A->second && block_smem_applicable(&Lp, S->Dd) && sjds_block_variant_ok();
         QB_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), c.stream));
-        if (fuse) {
+        if (to_native_tiled_ok(A, 8)) QB_TRY((launch_to_native_tiled<double2, double, true>(A, xd, px, flag)));
+        else {
+            to_native_real_check_kernel<<<grid_rows(A->n), kPBlock, 0, c.stream>>>(A->n, A->perm_inv, (const double2 *)xd, (double *)px, flag);
+            QB_LAUNCH_COUNT();
+            QB_CUDA(cudaGetLastError());
+        }
+        // The closing pass can write the reference's order itself (sjds_bulk.cu, OUT) when y is not read: the separate way
+        // out -- 0.9 ms of 17 on BASELINE config 3 -- is gone for 2 GB more traffic in pass 2.
+        const bool fuse_out = !use_beta && !S->matfree && A->second && A->row_lo == 0 && A->row_hi == A->n && sjds_bulk_out_fusable(A->second);
+        auto real_route = [&]() -> int {
             FusedArgs fa;
             fa.x = px; fa.y = py;
-            fa.x_ref = xd; fa.perm_inv = A->perm_inv; fa.imag_flag = flag;
+            if (fuse_out) { fa.y_ref = yd; fa.out_alpha = alpha; }
             QB_TRY(launch_spmv(&R, fa));
-            QB_TRY(vec_from_native(A, false, true, py, yd, alpha, beta));
-            int h;
+            if (!fuse_out) QB_TRY(vec_from_native(A, false, true, py, yd, alpha, beta));
+            return QBGPU_OK;
+        };
+        int h;
+        if (!use_beta && !A->last_x_had_imag) {
+            // y is not read: run the fp64 passes at once and look at the flag afterwards (the read-back then costs no idle
+            // time on the device); a vector with imaginary parts simply repeats the product on the complex route -- and
+            // the handle remembers it: the next call looks at the flag first (a caller with complex vectors pays the wasted
+            // passes once, not per product)
+            QB_TRY(real_route());
             QB_TRY(read_flag(h));
-            if (h != 0) QB_TRY(complex_route());            // rare: a vector with imaginary parts; y was not read, so simply redo
+            A->last_x_had_imag = h != 0;
+            if (h != 0) QB_TRY(complex_route());
         } else {
-            if (to_native_tiled_ok(A, 8)) QB_TRY((launch_to_native_tiled<double2, double, true>(A, xd, px, flag)));
-            else {
-                to_native_real_check_kernel<<<grid_rows(A->n), kPBlock, 0, c.stream>>>(A->n, A->perm_inv, (const double2 *)xd, (double *)px, flag);
-                QB_LAUNCH_COUNT();
-                QB_CUDA(cudaGetLastError());
-            }
-            // The closing pass can write the reference's order itself (sjds_bulk.cu, OUT) when y is not read: the separate way
-            // out -- 0.9 ms of 17 on BASELINE config 3 -- is gone for 2 GB more traffic in pass 2.
-            const bool fuse_out = !use_beta && !S->matfree && A->second && A->row_lo == 0 && A->row_hi == A->n && sjds_bulk_out_fusable(A->second);
-            auto real_route = [&]() -> int {
-                FusedArgs fa;
-                fa.x = px; fa.y = py;
-                if (fuse_out) { fa.y_ref = yd; fa.out_alpha = alpha; }
-                QB_TRY(launch_spmv(&R, fa));
-                if (!fuse_out) QB_TRY(vec_from_native(A, false, true, py, yd, alpha, beta));
-                return QBGPU_OK;
-            };
-            int h;
-            if (!use_beta && !A->last_x_had_imag) {
-                // y is not read: run the fp64 passes at once and look at the flag afterwards (the read-back then costs no idle
-                // time on the device); a vector with imaginary parts simply repeats the product on the complex route -- and
-                // the handle remembers it: the next call looks at the flag first (a caller with complex vectors pays the wasted
-                // passes once, not per product)
-                QB_TRY(real_route());
-                QB_TRY(read_flag(h));
-                A->last_x_had_imag = h != 0;
-                if (h != 0) QB_TRY(complex_route());
-            } else {
-                QB_TRY(read_flag(h));
-                A->last_x_had_imag = h != 0;
-                if (h == 0) QB_TRY(real_route()); else QB_TRY(complex_route());
-            }
+            QB_TRY(read_flag(h));
+            A->last_x_had_imag = h != 0;
+            if (h == 0) QB_TRY(real_route()); else QB_TRY(complex_route());
         }
     } else {
         QB_TRY(complex_route());
@@ -1283,7 +1233,6 @@ int qbgpu_row_view(qbgpu_matrix_t A, int64_t r0, int64_t r1, int64_t tile_period
         std::vector<int32_t> order;
         make_slice_order(r1 - r0, tile_period, tile < 32 ? 64 : tile, order);
         V->slice_order = nullptr;
-        V->ord_desc = nullptr;                              // (the descriptors describe the whole part's traversal)
         cudaError_t e = upload(&V->slice_order, order.data(), order.size(), ctx().stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(ctx().stream);
         if (e != cudaSuccess) { cudaFree(V->slice_order); delete V; return cuda_fail(e, "row_view: slice order", __FILE__, __LINE__); }

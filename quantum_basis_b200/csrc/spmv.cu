@@ -155,13 +155,7 @@ int autotune(qbgpu_matrix *A, int flags)
     int lanes = 2;
     while (lanes < 32 && mean > 4.0 * lanes) lanes *= 2;
     A->lanes = lanes;
-    // profiling aid: QBGPU_FORCE_FORMAT=sell|csr pins the layout (under ncu every launch is replayed cold and
-    // serialised, which would mislead the timing pass below)
-    if (const char *ff = getenv("QBGPU_FORCE_FORMAT")) {
-        if (!strcmp(ff, "sell")) flags |= QBGPU_FORMAT_SELL;
-        else if (!strcmp(ff, "csr")) flags |= QBGPU_FORMAT_CSR | QBGPU_NO_AUTOTUNE;
-    }
-    if ((flags & QBGPU_VALUE_DICT) || getenv("QBGPU_VALUE_DICT")) {
+    if (flags & QBGPU_VALUE_DICT) {
         QB_TRY(value_dict_encode(A));                       // opt-in 1-byte value codes; only the sliced-jagged kernel decodes them
         if (A->ndict) return sjds_convert(A, true);
     }

@@ -34,6 +34,17 @@ def test_every_declared_symbol_is_exported_and_bound(L):
     assert sorted(_lib.EXPORTS) == decl, "python binding table and header disagree"
 
 
+def test_debug_set_variant_accepts_only_the_species_pass1_variants(L):
+    try:
+        for vid in (1000, 1001, 1002):
+            assert L.qbgpu_debug_set_variant(vid) == 0
+        for vid in (0, 45, 999, 1003, 2001, 3020):
+            assert L.qbgpu_debug_set_variant(vid) == 1, vid             # QBGPU_ERR_ARG
+            assert f"unknown id {vid} ".encode() in L.qbgpu_last_error()
+    finally:
+        assert L.qbgpu_debug_set_variant(1000) == 0
+
+
 def test_library_is_sm100a_only():
     import subprocess
     out = subprocess.run(["cuobjdump", "--list-elf", qb.LIB_PATH], capture_output=True, text=True).stdout
