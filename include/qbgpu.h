@@ -48,7 +48,8 @@ extern "C" {
                                   * (rank of the up configuration, rank of the down configuration) and multiply in two passes
                                   * (see "species order" below); results and calling convention are unchanged */
 #define QBGPU_VALUE_DICT    16   /* opt-in: store fp64 values as 1-byte codes into a table of the distinct values when there
-                                    are at most 256 of them (lossless; products are bit-identical); implies FORMAT_SELL */
+                                    are at most 256 of them (lossless; products are bit-identical); implies FORMAT_SELL.
+                                    Stored species-order handles pack their values without it (see "species order") */
 
 typedef struct qbgpu_matrix *qbgpu_matrix_t;     /* replaces `sparse_matrix_t handle` (src/qbasis.h:985) */
 
@@ -58,7 +59,8 @@ typedef struct {
     int64_t nnz_stored;     /* entries in the device layout (full expanded Hermitian rows)         */
     int64_t nnz_input;      /* entries of the host CSR it was created from (upper triangle if sym) */
     int     val_is_real;    /* 1: values stored as fp64 (input was real or all imaginary parts == 0) */
-    int     value_dict;     /* > 0: number of dictionary entries; values are stored as 1-byte codes (QBGPU_VALUE_DICT) */
+    int     value_dict;     /* > 0: number of dictionary entries; values are stored as 1-byte codes (QBGPU_VALUE_DICT)
+                               or, on a stored species-order handle, as codes packed beside the columns */
     int     api_is_complex; /* 1: created through a z entry point                                  */
     int     format;         /* QBGPU_FORMAT_CSR or QBGPU_FORMAT_SELL                               */
     int     lanes;          /* threads per row chosen for the CSR-vector kernel                    */
@@ -323,8 +325,14 @@ int qbgpu_species_parts(qbgpu_matrix_t A, qbgpu_matrix_t *local_part, qbgpu_matr
  * handle keeps its vectors INTERNALLY in the order  p = rank(up configuration) * D_dn + rank(down configuration)  and
  * multiplies in two passes: (diagonal + hops of the down electrons), whose gathers stay inside one contiguous block of
  * D_dn entries, then (hops of the up electrons) traversed by tiles of down indices whose gathered columns stay in L2.
- *   qbgpu_build_hubbard          + flag: the two parts are stored (sliced-jagged layout, same entries and bytes as the
- *                                  ordinary handle) and multiplied by the production kernel;
+ *   qbgpu_build_hubbard          + flag: the two parts are stored (sliced-jagged layout, same entries as the ordinary
+ *                                  handle) and multiplied by the production kernels.  A handle built without a row
+ *                                  range (row_hi < 0) with real values stores each entry as one 32-bit word,
+ *                                  column | code << (bit width of n - 1), with code an index into the part's table of
+ *                                  distinct values (info.value_dict: the local part's table): 4 bytes per entry instead
+ *                                  of 12, bit-identical products.  Row shards (also one row range covering all rows),
+ *                                  complex values (QBGPU_KEEP_COMPLEX) and tables that do not fit keep fp64 or complex
+ *                                  values;
  *   qbgpu_create_matfree_hubbard + flag: nothing is stored but per-species hop tables (a few MB).
  * The calling convention does not change: qbgpu_{d,z}mv, qbgpu_lanczos_*, qbgpu_eigenvec_cg_*, qbgpu_energy_scale_*,
  * qbgpu_kpm_moments_* and qbgpu_trlan take and return vectors in the REFERENCE's order (they permute on the way in and
@@ -353,6 +361,15 @@ int qbgpu_debug_species_host(int nsites, int nup, int ndn, int nbonds, const int
 int qbgpu_debug_species_parts_host(int nsites, int nup, int ndn, int nbonds, const int32_t *bonds, double t, double U, int tile,
                                    int64_t u_lo, int64_t u_hi, int nparts, const int64_t *part_bounds, const int32_t *order,
                                    const double *x, double *y_local);
+
+/* The packed entry words of the two stored parts, computed on the host with the build's rules (species order, a handle
+ * built without a row range, real values).  cbits <= 0: the build's column width (bit width of n - 1).  out[5] = {cbits, local table entries,
+ * cross table entries, local part packed (0/1), cross part packed (0/1)}; a part is packed when its table fits in the
+ * 32 - cbits bits above the column (and has at most 256 entries).  table_* (256 doubles each, in code order) and
+ * words_* (the parts' entries in CSR order, as qbgpu_debug_species_host lists them; written only for a packed part) may
+ * be NULL. */
+int qbgpu_debug_species_packed_host(int nsites, int nup, int ndn, int nbonds, const int32_t *bonds, double t, double U, int cbits,
+                                    int64_t *out, double *table_local, uint32_t *words_local, double *table_cross, uint32_t *words_cross);
 
 /* --------------------------------------------------------------------- translation-symmetric sectors
  * Device counterpart of model::fill_Weisse_table + enumerate_basis_repr + generate_Ham_sparse_repr

@@ -108,6 +108,7 @@ _SIGS = {
     "qbgpu_debug_rows_host": [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, dbl, dbl, dbl, i64, vp, vp, C.c_int, vp],
     "qbgpu_debug_species_parts_host": [C.c_int, C.c_int, C.c_int, C.c_int, vp, dbl, dbl, C.c_int, i64, i64, C.c_int, vp, vp, vp, vp],
     "qbgpu_debug_species_host": [C.c_int, C.c_int, C.c_int, C.c_int, vp, dbl, dbl, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],
+    "qbgpu_debug_species_packed_host": [C.c_int, C.c_int, C.c_int, C.c_int, vp, dbl, dbl, C.c_int, vp, vp, vp, vp, vp],
     "qbgpu_build_heisenberg_orbit": [C.POINTER(vp), C.c_int, C.c_int, C.c_int, vp, vp, C.c_int, vp, dbl, C.c_int, vp, i64],
 }
 _RESTYPES = {"qbgpu_last_error": C.c_char_p, "qbgpu_version": C.c_char_p, "qbgpu_kernel_launches": C.c_int64,

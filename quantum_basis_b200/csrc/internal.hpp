@@ -2,6 +2,7 @@
 #pragma once
 #include "common.cuh"
 #include "../../include/qbgpu.h"
+#include <cmath>
 
 // Device-resident matrix behind qbgpu_matrix_t.
 //
@@ -30,6 +31,10 @@ struct qbgpu_matrix {
     // of 1-byte codes into vdict[ndict]; products decode through shared memory and are bit-identical.
     double  *vdict = nullptr;
     int      ndict = 0;
+    // > 0: packed layout (the stored parts of a species handle built without a row range, real values; species.cu): col[]
+    // holds one 32-bit word per entry, column | code << cbits, where cbits is the bit width of n - 1 and code indexes
+    // vdict[ndict]; there is no val array.  4 bytes per entry instead of 12; products decode the identical doubles and are bit-identical.
+    int      cbits = 0;
     // QBGPU_FORMAT_MATFREE: no stored entries at all; `mf` owns the sector tables, the bond list and the per-row
     // basis states from which every row is regenerated inside the product (builders.cu).
     void    *mf = nullptr;
@@ -70,7 +75,7 @@ struct qbgpu_matrix {
     mutable bool last_x_had_imag = false;      // mv_species: the previous vector had non-zero imaginary parts -> look at the flag BEFORE the fp64 passes
     double  upload_s = 0, convert_s = 0, autotune_s = 0;
     int64_t nrows() const { return row_hi - row_lo; }
-    size_t  val_bytes() const { return ndict ? 1 : (val_real ? 8 : 16); }
+    size_t  val_bytes() const { return cbits ? 0 : ndict ? 1 : (val_real ? 8 : 16); }
     size_t  vec_bytes() const { return api_complex ? 16 : 8; }
 };
 
@@ -99,7 +104,17 @@ struct FusedArgs {
 int launch_spmv(const qbgpu_matrix *A, const FusedArgs &args, int lanes_override = 0);
 int autotune(qbgpu_matrix *A, int flags = 0);
 int sjds_convert(qbgpu_matrix *A, bool forward);
-int value_dict_encode(qbgpu_matrix *A);               // matrix.cu: try to replace fp64 values by 1-byte codes
+int value_dict_encode(qbgpu_matrix *A, int max_entries = 256);   // matrix.cu: try to replace fp64 values by 1-byte codes
+// order of a value table: by value, -0.0 before +0.0 (distinct bit patterns), so that a layout does not depend on thread timing
+inline bool value_table_less(double a, double b) { return a != b ? a < b : std::signbit(a) > std::signbit(b); }
+// Packed entry words (qbgpu_matrix::cbits): the column takes the bit width of n - 1, the value code the bits above it.  A
+// table fits when its codes do (and the 256 entries the product kernels stage in shared memory).
+constexpr uint32_t kPackedMaxTable = 256;
+__host__ __device__ inline int packed_col_bits(int64_t n)
+{ int b = 1; while (b < 31 && ((n - 1) >> b) != 0) b++; return b; }
+__host__ __device__ inline bool packed_table_fits(int64_t ntable, int cbits)
+{ return ntable > 0 && ntable <= (int64_t)kPackedMaxTable && ntable <= (int64_t)1 << (32 - cbits); }
+__host__ __device__ inline uint32_t packed_word(int32_t col, uint32_t code, int cbits) { return (uint32_t)col | code << cbits; }
 int launch_spmv_sjds(const qbgpu_matrix *A, const FusedArgs &args);
 // sjds_bulk.cu: the same product with the matrix stream moved by cp.async.bulk into per-warp shared-memory rings, and the
 // block-local product (rows of block u reference only columns of block u) with the block of x staged in shared memory

@@ -308,7 +308,7 @@ __global__ void __launch_bounds__(kCBlock) dict_encode_kernel(int64_t nnz, const
     }
 }
 
-int value_dict_encode(qbgpu_matrix *A)
+int value_dict_encode(qbgpu_matrix *A, int max_entries)
 {
     Context &c = ctx();
     if (!A->val_real || A->ndict || A->format != QBGPU_FORMAT_CSR || A->nnz == 0) return QBGPU_OK;
@@ -329,15 +329,12 @@ int value_dict_encode(qbgpu_matrix *A)
     QB_CU(cudaMemcpyAsync(slots.data(), d_slots, sizeof(unsigned long long) * kDictSlots, cudaMemcpyDeviceToHost, c.stream));
     QB_CU(cudaMemcpyAsync(&count, d_count, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
     QB_CU(cudaStreamSynchronize(c.stream));
-    if (count > 256) { cleanup(); return QBGPU_OK; }        // not compressible: keep the fp64 values
+    if (count > 256 || count > max_entries) { cleanup(); return QBGPU_OK; }      // not compressible: keep the fp64 values
     // order the dictionary by value so that the layout does not depend on thread timing
     std::vector<std::pair<double, int>> keys;
     for (int h = 0; h < kDictSlots; h++)
         if (slots[h] != kEmptyKey) { double v; memcpy(&v, &slots[h], 8); keys.push_back({v, h}); }
-    std::sort(keys.begin(), keys.end(), [](const std::pair<double, int> &a, const std::pair<double, int> &b) {
-        if (a.first != b.first) return a.first < b.first;
-        return std::signbit(a.first) > std::signbit(b.first);       // -0.0 before +0.0: distinct bit patterns
-    });
+    std::sort(keys.begin(), keys.end(), [](const std::pair<double, int> &a, const std::pair<double, int> &b) { return value_table_less(a.first, b.first); });
     std::vector<int> slot_code(kDictSlots, 0);
     std::vector<double> dict(256, 0.0);
     for (size_t j = 0; j < keys.size(); j++) { dict[j] = keys[j].first; slot_code[keys[j].second] = (int)j; }
@@ -499,6 +496,7 @@ int qbgpu_download_expanded(qbgpu_matrix_t A, int64_t *rowptr, int32_t *col, voi
     if (!A || !rowptr || !col || !val) return fail(QBGPU_ERR_ARG, "null argument");
     QB_TRY(no_species(A, "download_expanded"));
     if (A->mf || A->mf_sec) return fail(QBGPU_ERR_STATE, "matrix-free handle: there are no stored entries to download");
+    if (A->cbits) return fail(QBGPU_ERR_STATE, "download_expanded: not available for packed entry words (a part of a species-order handle)");
     const bool jag = (A->format == QBGPU_FORMAT_SELL);      // hand back plain CSR order whatever the resident layout
     if (jag) QB_TRY(sjds_convert(A, false));
     QB_CUDA(cudaStreamSynchronize(ctx().stream));

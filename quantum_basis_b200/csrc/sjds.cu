@@ -67,13 +67,15 @@ spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *
                  const uint32_t *__restrict__ rowinfo, const int32_t *__restrict__ col, const ValT *__restrict__ val,
                  const VecT *__restrict__ x, const VecT *z, VecT *y, double2 alpha, double2 gamma, double2 beta,
                  int scal_mode, const double *__restrict__ sc, double *dots_out, double *partials, unsigned *ticket,
-                 const double *__restrict__ vdict)
+                 const double *__restrict__ vdict, int cbits)
 {
     using VT = VecTraits<VecT>;
     constexpr bool kDict = sizeof(ValT) == 1;               // 1-byte codes into a <= 256-entry fp64 dictionary
-    using ArithT = typename std::conditional<kDict, double, ValT>::type;
-    __shared__ double sdict[kDict ? 256 : 1];
-    if (kDict) { sdict[threadIdx.x] = vdict[threadIdx.x]; __syncthreads(); }      // kSBlock == 256 threads
+    constexpr bool kPacked = std::is_same<ValT, uint32_t>::value;   // packed words col | code << cbits (no val array)
+    using ArithT = typename std::conditional<kDict || kPacked, double, ValT>::type;
+    __shared__ double sdict[kDict || kPacked ? 256 : 1];
+    if (kDict || kPacked) { sdict[threadIdx.x] = vdict[threadIdx.x]; __syncthreads(); }      // kSBlock == 256 threads
+    const uint32_t cmask = kPacked ? (1u << cbits) - 1u : ~0u;
     constexpr int WPB = kSBlock / 32;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint64_t pol_s = l2_policy_evict_first(), pol_x = XPOL >= 1 ? l2_policy_evict_last() : 0;
@@ -117,15 +119,17 @@ spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *
                 VecT xv[U];
 #pragma unroll
                 for (int u = 0; u < U; u++) c[u] = ld_i32(col + o[u], pol_s);
+                if constexpr (!kPacked) {
 #pragma unroll
-                for (int u = 0; u < U; u++) v[u] = ld_f64(val + o[u], pol_s);
+                    for (int u = 0; u < U; u++) v[u] = ld_f64(val + o[u], pol_s);
+                }
 #pragma unroll
-                for (int u = 0; u < U; u++) xv[u] = ld_x<XPOL>(x + c[u], pol_x);
+                for (int u = 0; u < U; u++) xv[u] = ld_x<XPOL>(x + ((uint32_t)c[u] & cmask), pol_x);
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     VecT t = (u & 1) ? acc1 : acc0;
                     ArithT w;
-                    if constexpr (kDict) w = sdict[v[u]]; else w = v[u];
+                    if constexpr (kPacked) w = sdict[(uint32_t)c[u] >> cbits]; else if constexpr (kDict) w = sdict[v[u]]; else w = v[u];
                     mac(t, w, xv[u]);
                     if (a[u]) { if (u & 1) acc1 = t; else acc0 = t; }
                 }
@@ -133,14 +137,15 @@ spmv_sjds_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     c[u] = 0; v[u] = ValT{};
-                    if (a[u]) { c[u] = ld_i32(col + o[u], pol_s); v[u] = ld_f64(val + o[u], pol_s); }
+                    if (a[u]) { c[u] = ld_i32(col + o[u], pol_s); if constexpr (!kPacked) v[u] = ld_f64(val + o[u], pol_s); }
                 }
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     if (a[u]) {
                         ArithT w;
-                        if constexpr (kDict) w = sdict[v[u]]; else w = v[u];
-                        if (u & 1) mac(acc1, w, ld_x<XPOL>(x + c[u], pol_x)); else mac(acc0, w, ld_x<XPOL>(x + c[u], pol_x));
+                        if constexpr (kPacked) w = sdict[(uint32_t)c[u] >> cbits]; else if constexpr (kDict) w = sdict[v[u]]; else w = v[u];
+                        const VecT xv = ld_x<XPOL>(x + ((uint32_t)c[u] & cmask), pol_x);
+                        if (u & 1) mac(acc1, w, xv); else mac(acc0, w, xv);
                     }
                 }
             }
@@ -185,7 +190,7 @@ static int launch_sjds_cfg(const qbgpu_matrix *A, const FusedArgs &a)
     const int grid = (int)(want < cap ? want : cap);
     kern<<<grid, kSBlock, 0, c.stream>>>(nslices, nrows, A->row_lo, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val,
                                          (const VecT *)a.x, (const VecT *)a.z, (VecT *)a.y, a.alpha, a.gamma, a.beta,
-                                         a.scal_mode, a.sc, a.dots, c.partials, c.ticket, A->vdict);
+                                         a.scal_mode, a.sc, a.dots, c.partials, c.ticket, A->vdict, A->cbits);
     QB_LAUNCH_COUNT();
     QB_CUDA(cudaGetLastError());
     return QBGPU_OK;
@@ -366,11 +371,13 @@ int launch_spmv_sjds(const qbgpu_matrix *A, const FusedArgs &a)
     if (A->ring_world <= 1 && A->slice_order) return launch_spmv_sjds_bulk(A, a);
     if (a.y_ref) return fail(QBGPU_ERR_STATE, "fused way out: only the bulk-streamed kernel writes the reference's order (internal)");
     if (A->ring_world > 1) {
+        if (A->cbits) return fail(QBGPU_ERR_STATE, "ring-fused product: not available for packed entry words");
         if (A->ndict) return A->api_complex ? launch_sjds_ring_typed<uint8_t, double2>(A, a) : launch_sjds_ring_typed<uint8_t, double>(A, a);
         if (!A->api_complex) return launch_sjds_ring_typed<double, double>(A, a);
         if (A->val_real) return launch_sjds_ring_typed<double, double2>(A, a);
         return launch_sjds_ring_typed<double2, double2>(A, a);
     }
+    if (A->cbits) return A->api_complex ? launch_sjds_typed<uint32_t, double2>(A, a) : launch_sjds_typed<uint32_t, double>(A, a);
     if (A->ndict) return A->api_complex ? launch_sjds_typed<uint8_t, double2>(A, a) : launch_sjds_typed<uint8_t, double>(A, a);
     if (!A->api_complex) return launch_sjds_typed<double, double>(A, a);
     if (A->val_real) return launch_sjds_typed<double, double2>(A, a);
@@ -470,6 +477,7 @@ static int sjds_convert_typed(qbgpu_matrix *A, bool forward)
 int sjds_convert(qbgpu_matrix *A, bool forward)
 {
     if (forward == (A->format == QBGPU_FORMAT_SELL)) return QBGPU_OK;
+    if (A->cbits) return fail(QBGPU_ERR_STATE, "packed entry words stay in the sliced-jagged layout");
     if (A->ndict) return sjds_convert_typed<uint8_t>(A, forward);
     return A->val_real ? sjds_convert_typed<double>(A, forward) : sjds_convert_typed<double2>(A, forward);
 }

@@ -8,9 +8,9 @@
 //
 //  (1) spmv_sjds_bulk_kernel -- every warp owns a ring of NST stages in shared memory.  A stage receives one SEGMENT of a
 //      32-row slice: KSEG consecutive jagged diagonals, which are one contiguous range of col[] and of val[] (sjds.cu), so a
-//      segment is two bulk copies (UBLKCP in the SASS) that complete on the stage's mbarrier.  NST-1 segments are in flight
-//      per warp while one is consumed: the stream is fetched exactly once, in whole lines, with no registers held, and the
-//      only long-latency instructions left in the loop are the gathers of x, issued KSEG at a time.
+//      segment is two bulk copies (UBLKCP in the SASS; one for packed words) that complete on the stage's mbarrier.  NST-1
+//      segments are in flight per warp while one is consumed: the stream is fetched exactly once, in whole lines, with no
+//      registers held, and the only long-latency instructions left in the loop are the gathers of x, issued KSEG at a time.
 //      The producer is the consumer warp itself (lane 0 issues): no CTA-wide synchronisation, ragged slices are natural.
 //
 //  (2) sjds_block_smem_kernel -- for a matrix whose rows [u*D, (u+1)*D) only reference columns of the same block (the
@@ -78,23 +78,25 @@ __device__ __forceinline__ double lds_val(const double *p, uint64_t pol)
 { double v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol)); return v; }
 __device__ __forceinline__ double2 lds_val(const double2 *p, uint64_t pol)
 { double2 v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.f64 {%0, %1}, [%2], %3;" : "=d"(v.x), "=d"(v.y) : "l"(p), "l"(pol)); return v; }
-__device__ __forceinline__ uint8_t lds_val(const uint8_t *p, uint64_t pol)
-{ unsigned v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol)); return (uint8_t)v; }
 
 // ------------------------------------------------------------------------------------------ (1) bulk-streamed product
 // Stage layout (per warp, per stage; every area 16-byte aligned):
 //   hdr[8]  int32 : [0..1] first entry of the segment (int64), [2] entries, [3] first diagonal k0, [4] slice index (< 2^31)
 //   info[32] uint32: rowinfo of the slice
 //   col  int32[CAP + 8], val ValT[CAP + VPAD]: the copies start at the entry rounded DOWN to a 16-byte boundary
+//   (packed words, ValT = uint32_t: the col area holds col | code << cbits and there is no val area)
 template <typename ValT, int KSEG> struct BulkStage {
+    static constexpr bool PACKED = std::is_same<ValT, uint32_t>::value;
     static constexpr int CAP = 32 * KSEG;
     static constexpr int VALIGN = 16 / (int)sizeof(ValT) > 0 ? 16 / (int)sizeof(ValT) : 1;   // entries per 16 bytes of val
     static constexpr int VPAD = 2 * VALIGN;
     static constexpr int HDR_BYTES = 32 + 128;
     static constexpr int COL_BYTES = (CAP + 8) * 4;
-    static constexpr int VAL_BYTES = ((CAP + VPAD) * (int)sizeof(ValT) + 15) / 16 * 16;
+    static constexpr int VAL_BYTES = PACKED ? 0 : ((CAP + VPAD) * (int)sizeof(ValT) + 15) / 16 * 16;
     static constexpr int BYTES = HDR_BYTES + COL_BYTES + VAL_BYTES;
 };
+// the mbarriers of one warp's ring (8 bytes per stage) come before all rings, in whole 64-byte blocks per warp
+constexpr int bulk_bar_bytes(int nst) { return (8 * nst + 63) / 64 * 64; }
 
 // What the consumer keeps of a segment between its two phases (gathers issued / products accumulated)
 template <typename VecT> struct SegState {
@@ -123,7 +125,7 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
                       const uint32_t *__restrict__ rowinfo, const int32_t *__restrict__ col, const ValT *__restrict__ val,
                       const VecT *__restrict__ x, const VecT *z, VecT *y, double2 alpha, double2 gamma, double2 beta,
                       int scal_mode, const double *__restrict__ sc, double *dots_out, double *partials, unsigned *ticket,
-                      const double *__restrict__ vdict, const int32_t *__restrict__ order,
+                      const double *__restrict__ vdict, const int32_t *__restrict__ order, int cbits,
                       const int32_t *__restrict__ perm_inv = nullptr, double2 *y_ref = nullptr, double2 out_alpha = {1.0, 0.0})
 {
     static_assert(!OUT || (sizeof(VecT) == 8 && !DOTS), "the fused way out serves the fp64 closing pass");
@@ -132,14 +134,17 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
     using Seg = SegState<VecT>;
     static_assert(KSEG % 2 == 0 && KSEG >= 2, "diagonal k accumulates into accumulator k & 1 (the order of sjds.cu)");
     static_assert(NST >= 3, "the pipelined consumer holds two stages");
-    constexpr bool kDict = sizeof(ValT) == 1;
-    using ArithT = typename std::conditional<kDict, double, ValT>::type;
+    constexpr bool kPacked = ST::PACKED;
+    static_assert(kPacked || sizeof(ValT) >= 8, "values are fp64, complex, or packed codes");
+    using ArithT = typename std::conditional<kPacked, double, ValT>::type;
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ double sdict[kDict ? 256 : 1];
-    if (kDict) { for (int i = threadIdx.x; i < 256; i += NW * 32) sdict[i] = vdict[i]; __syncthreads(); }
+    __shared__ double sdict[kPacked ? kPackedMaxTable : 1];
+    if (kPacked) { for (int i = threadIdx.x; i < (int)kPackedMaxTable; i += NW * 32) sdict[i] = vdict[i]; __syncthreads(); }
+    const uint32_t cmask = kPacked ? (1u << cbits) - 1u : ~0u;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned char *wbase = smem_raw + 64 * NW + (size_t)warp * NST * ST::BYTES;      // [NW][8] barriers (64 B per warp) first
-    const uint32_t bar0 = smem_u32(smem_raw + 64 * warp);
+    constexpr int BARB = bulk_bar_bytes(NST);
+    unsigned char *wbase = smem_raw + BARB * NW + (size_t)warp * NST * ST::BYTES;    // [NW][NST] barriers first
+    const uint32_t bar0 = smem_u32(smem_raw + BARB * warp);
     if (lane == 0) {
 #pragma unroll
         for (int s = 0; s < NST; s++) mbar_init(bar0 + 8 * s, 1);
@@ -208,11 +213,11 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
                 fence_proxy_async_smem();
                 const int64_t c0 = beg & ~3LL, c1 = (beg + cnt + 3) & ~3LL;                       // 16-byte aligned col range
                 const int64_t v0 = beg & ~(int64_t)(ST::VALIGN - 1), v1 = (beg + cnt + ST::VALIGN - 1) & ~(int64_t)(ST::VALIGN - 1);
-                const uint32_t cb = (uint32_t)(c1 - c0) * 4u, vb = (uint32_t)((v1 - v0) * (int64_t)sizeof(ValT));
+                const uint32_t cb = (uint32_t)(c1 - c0) * 4u, vb = kPacked ? 0u : (uint32_t)((v1 - v0) * (int64_t)sizeof(ValT));
                 const uint32_t bar = bar0 + 8 * st;
                 mbar_expect_tx(bar, cb + vb);
                 bulk_g2s(smem_u32(sb + ST::HDR_BYTES), col + c0, cb, bar, pol_s);
-                bulk_g2s(smem_u32(sb + ST::HDR_BYTES + ST::COL_BYTES), val + v0, vb, bar, pol_s);
+                if constexpr (!kPacked) bulk_g2s(smem_u32(sb + ST::HDR_BYTES + ST::COL_BYTES), val + v0, vb, bar, pol_s);
             }
         }
         __syncwarp();
@@ -253,16 +258,16 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
         if (g.cnt > 0) {
             mbar_wait(bar0 + 8 * st, (phases >> st) & 1u);
             phases ^= 1u << st;
-            const int32_t *scol = (const int32_t *)(sb + ST::HDR_BYTES) + (h.x & 3) + lane;
+            const uint32_t *scol = (const uint32_t *)(sb + ST::HDR_BYTES) + (h.x & 3) + lane;
             if (g.full) {
 #pragma unroll
-                for (int u = 0; u < KSEG; u++) xv[u] = ldx_hint(x + scol[u * 32], pol_x);
+                for (int u = 0; u < KSEG; u++) xv[u] = ldx_hint(x + (scol[u * 32] & cmask), pol_x);
             } else {
                 int off = 0;
 #pragma unroll
                 for (int u = 0; u < KSEG; u++) {
                     const bool a = g.k0 + u < len;
-                    if (a) xv[u] = ldx_hint(x + scol[off], pol_x);
+                    if (a) xv[u] = ldx_hint(x + (scol[off] & cmask), pol_x);
                     off += __popc(__ballot_sync(0xffffffffu, a));
                 }
             }
@@ -282,12 +287,13 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
         if (g.cnt > 0) {
             const int begl = *(const int *)sb;
             const ValT *sval = (const ValT *)(sb + ST::HDR_BYTES + ST::COL_BYTES) + (begl & (ST::VALIGN - 1)) + lane;
+            const uint32_t *sword = (const uint32_t *)(sb + ST::HDR_BYTES) + (begl & 3) + lane;
             // diagonal k0 + u goes to accumulator (k0 + u) & 1 == u & 1 (KSEG is even): the order of sjds.cu
             if (g.full) {
 #pragma unroll
                 for (int u = 0; u < KSEG; u++) {
                     ArithT w;
-                    if constexpr (kDict) w = sdict[sval[u * 32]]; else w = sval[u * 32];
+                    if constexpr (kPacked) w = sdict[sword[u * 32] >> cbits]; else w = sval[u * 32];
                     if (u & 1) mac(acc1, w, xv[u]); else mac(acc0, w, xv[u]);
                 }
             } else {
@@ -298,7 +304,7 @@ spmv_sjds_bulk_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int6
                     const bool a = g.k0 + u < len;
                     if (a) {
                         ArithT w;
-                        if constexpr (kDict) w = sdict[sval[off]]; else w = sval[off];
+                        if constexpr (kPacked) w = sdict[sword[off] >> cbits]; else w = sval[off];
                         if (u & 1) mac(acc1, w, xv[u]); else mac(acc0, w, xv[u]);
                     }
                     off += __popc(__ballot_sync(0xffffffffu, a));
@@ -362,7 +368,7 @@ static int launch_bulk_cfg(const qbgpu_matrix *A, const FusedArgs &a)
     Context &c = ctx();
     using ST = BulkStage<ValT, KSEG>;
     auto kern = spmv_sjds_bulk_kernel<ValT, VecT, DOTS, KEEP, NW, NST, KSEG, OUT>;
-    constexpr size_t smem = 64 * NW + (size_t)NW * NST * ST::BYTES;
+    constexpr size_t smem = (size_t)bulk_bar_bytes(NST) * NW + (size_t)NW * NST * ST::BYTES;
     static int blocks_per_sm = 0;
     if (blocks_per_sm == 0) {
         QB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -379,22 +385,32 @@ static int launch_bulk_cfg(const qbgpu_matrix *A, const FusedArgs &a)
     const int grid = (int)(want < cap ? want : cap);
     kern<<<grid, NW * 32, smem, c.stream>>>(nslices, nrows, A->row_lo, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val,
                                             (const VecT *)a.x, (const VecT *)a.z, (VecT *)a.y, a.alpha, a.gamma, a.beta,
-                                            a.scal_mode, a.sc, a.dots, c.partials, c.ticket, A->vdict, A->slice_order,
+                                            a.scal_mode, a.sc, a.dots, c.partials, c.ticket, A->vdict, A->slice_order, A->cbits,
                                             OUT ? a.perm_inv : nullptr, OUT ? (double2 *)a.y_ref : nullptr, a.out_alpha);
     QB_LAUNCH_COUNT();
     QB_CUDA(cudaGetLastError());
     return QBGPU_OK;
 }
 
+// (warps per CTA, stages per warp, diagonals per segment).  What the stage rings take from the SM's 256 KB of SRAM is lost
+// to L1, and L1 lines are what gathers in flight are tracked in: with fp64 vectors a fat ring (106 KB per CTA, two CTAs)
+// is best; with complex vectors (twice the lines per gather) a leaner one (profiles/r02_bulk_sweep_*.txt: 8,4,8 is 2x
+// slower than 8,3,6 there).  Packed words (4 bytes per entry, one bulk copy per segment) keep the segment length and with it
+// the gathers in flight, and take more, smaller stages (78 KB of ring per CTA with fp64 vectors instead of 106).  On BASELINE
+// config 3 the closing pass no longer follows the stream's bytes in flight: 8 x 8, 10 x 8 and 6 x 16 measured 6.77, 6.83
+// and 6.75 ms (y += H_cross x, fp64 vectors, one B200 at 1000 W).
+template <typename ValT, typename VecT> struct BulkRing {
+    static constexpr bool kPacked = std::is_same<ValT, uint32_t>::value, kCplx = sizeof(VecT) == 16;
+    static constexpr int NW = 8;
+    static constexpr int NST = kPacked ? (kCplx ? 6 : 8) : (kCplx ? 3 : 4);
+    static constexpr int KSEG = kPacked ? (kCplx ? 6 : 8) : (kCplx ? 6 : 8);
+};
+
 template <typename ValT, typename VecT, bool DOTS, bool KEEP>
 static int launch_bulk_ring(const qbgpu_matrix *A, const FusedArgs &a)
 {
-    // (warps per CTA, stages per warp, diagonals per segment).  What the stage rings take from the SM's 256 KB of SRAM is lost
-    // to L1, and L1 lines are what gathers in flight are tracked in: with fp64 vectors a fat ring (106 KB per CTA, two CTAs)
-    // is best; with complex vectors (twice the lines per gather) a leaner one (profiles/r02_bulk_sweep_*.txt: 8,4,8 is 2x
-    // slower than 8,3,6 there).
-    if constexpr (sizeof(VecT) == 16) return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, 8, 3, 6>(A, a);
-    else return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, 8, 4, 8>(A, a);
+    using R = BulkRing<ValT, VecT>;
+    return launch_bulk_cfg<ValT, VecT, DOTS, KEEP, R::NW, R::NST, R::KSEG>(A, a);
 }
 
 template <typename ValT, typename VecT>
@@ -404,7 +420,8 @@ static int launch_bulk_typed(const qbgpu_matrix *A, const FusedArgs &a)
     const bool keep = !dots && a.scal_mode == 0 && a.z == a.y && a.beta.x == 1.0 && a.beta.y == 0.0 && a.gamma.x == 0.0 && a.gamma.y == 0.0;
     if (a.y_ref) {                                          // the closing pass of a species product writes the reference's order
         if constexpr (sizeof(VecT) == 8) {
-            if (keep && a.perm_inv) return launch_bulk_cfg<ValT, VecT, false, true, 8, 4, 8, true>(A, a);
+            using R = BulkRing<ValT, VecT>;
+            if (keep && a.perm_inv) return launch_bulk_cfg<ValT, VecT, false, true, R::NW, R::NST, R::KSEG, true>(A, a);
         }
         return fail(QBGPU_ERR_STATE, "fused way out: not the closing pass of a species handle (internal)");
     }
@@ -417,7 +434,8 @@ static int launch_bulk_typed(const qbgpu_matrix *A, const FusedArgs &a)
 // allocations keep 64 bytes of slack.
 int launch_spmv_sjds_bulk(const qbgpu_matrix *A, const FusedArgs &a)
 {
-    if (A->ndict) return A->api_complex ? launch_bulk_typed<uint8_t, double2>(A, a) : launch_bulk_typed<uint8_t, double>(A, a);
+    if (A->cbits) return A->api_complex ? launch_bulk_typed<uint32_t, double2>(A, a) : launch_bulk_typed<uint32_t, double>(A, a);
+    if (A->ndict) return fail(QBGPU_ERR_STATE, "bulk-streamed product: 1-byte dictionary codes are not supported (internal)");
     if (!A->api_complex) return launch_bulk_typed<double, double>(A, a);
     if (A->val_real) return launch_bulk_typed<double, double2>(A, a);
     return launch_bulk_typed<double2, double2>(A, a);
@@ -431,19 +449,21 @@ __global__ void __launch_bounds__(NT, MINB)
 sjds_block_smem_kernel(int64_t nrows, int64_t row_lo, int64_t D, int64_t u_lo, int64_t u_cnt, const int64_t *__restrict__ rowptr,
                        const uint32_t *__restrict__ rowinfo, const int32_t *__restrict__ col, const ValT *__restrict__ val,
                        const VecT *__restrict__ x, const VecT *z, VecT *y, double2 alpha, double2 gamma, double2 beta,
-                       int scal_mode, const double *__restrict__ sc, const double *__restrict__ vdict, int use_bulk,
+                       int scal_mode, const double *__restrict__ sc, const double *__restrict__ vdict, int cbits, int use_bulk,
                        int64_t P, int64_t EP)
 {
     using VT = VecTraits<VecT>;
-    constexpr bool kDict = sizeof(ValT) == 1;
-    using ArithT = typename std::conditional<kDict, double, ValT>::type;
+    constexpr bool kPacked = std::is_same<ValT, uint32_t>::value;     // packed words col | code << cbits, no val array
+    static_assert(kPacked || sizeof(ValT) >= 8, "values are fp64, complex, or packed codes");
+    using ArithT = typename std::conditional<kPacked, double, ValT>::type;
     constexpr int NWARP = NT / 32;
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ double sdict[kDict ? 256 : 1];
+    __shared__ double sdict[kPacked ? kPackedMaxTable : 1];
     __shared__ __align__(8) unsigned long long xbar_storage;
     VecT *xs = (VecT *)smem_raw;
     const uint32_t xbar = smem_u32(&xbar_storage);
-    if (kDict) { for (int i = threadIdx.x; i < 256; i += NT) sdict[i] = vdict[i]; }
+    const uint32_t cmask = kPacked ? (1u << cbits) - 1u : ~0u;
+    if (kPacked) { for (int i = threadIdx.x; i < (int)kPackedMaxTable; i += NT) sdict[i] = vdict[i]; }
     if (threadIdx.x == 0) { mbar_init(xbar, 1); mbar_fence_init(); }
     __syncthreads();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -519,15 +539,17 @@ sjds_block_smem_kernel(int64_t nrows, int64_t row_lo, int64_t D, int64_t u_lo, i
                 ValT v[U];
 #pragma unroll
                 for (int u = 0; u < U; u++) c[u] = lds_i32(cb + (k + u) * 32, pol_s);
+                if constexpr (!kPacked) {
 #pragma unroll
-                for (int u = 0; u < U; u++) v[u] = lds_val(vb + (k + u) * 32, pol_s);
+                    for (int u = 0; u < U; u++) v[u] = lds_val(vb + (k + u) * 32, pol_s);
+                }
                 if (!x_ready) { mbar_wait(xbar, xphase); xphase ^= 1u; x_ready = true; }
                 if (mine) {
 #pragma unroll
                     for (int u = 0; u < U; u++) {
-                        const VecT xv = xs[(int)((int64_t)c[u] - c0)];
+                        const VecT xv = xs[(int)((int64_t)(int32_t)((uint32_t)c[u] & cmask) - c0)];
                         ArithT w;
-                        if constexpr (kDict) w = sdict[v[u]]; else w = v[u];
+                        if constexpr (kPacked) w = sdict[(uint32_t)c[u] >> cbits]; else w = v[u];
                         if (u & 1) mac(acc1, w, xv); else mac(acc0, w, xv);      // U is even: diagonal k + u -> accumulator u & 1
                     }
                 }
@@ -546,14 +568,14 @@ sjds_block_smem_kernel(int64_t nrows, int64_t row_lo, int64_t D, int64_t u_lo, i
                     off += __popc(__ballot_sync(0xffffffffu, a));
                 }
 #pragma unroll
-                for (int u = 0; u < U; u++) if ((am >> u) & 1u) { c[u] = lds_i32(cb + o[u], pol_s); v[u] = lds_val(vb + o[u], pol_s); }
+                for (int u = 0; u < U; u++) if ((am >> u) & 1u) { c[u] = lds_i32(cb + o[u], pol_s); if constexpr (!kPacked) v[u] = lds_val(vb + o[u], pol_s); }
                 if (!x_ready) { mbar_wait(xbar, xphase); xphase ^= 1u; x_ready = true; }
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     if (((am >> u) & 1u) && mine) {
-                        const VecT xv = xs[(int)((int64_t)c[u] - c0)];
+                        const VecT xv = xs[(int)((int64_t)(int32_t)((uint32_t)c[u] & cmask) - c0)];
                         ArithT w;
-                        if constexpr (kDict) w = sdict[v[u]]; else w = v[u];
+                        if constexpr (kPacked) w = sdict[(uint32_t)c[u] >> cbits]; else w = v[u];
                         if (u & 1) mac(acc1, w, xv); else mac(acc0, w, xv);
                     }
                 }
@@ -593,7 +615,7 @@ static int launch_block_smem_cfg(const qbgpu_matrix *A, const FusedArgs &a, int6
     const int use_bulk = ((D * (int64_t)sizeof(VecT)) % 16 == 0 && D * (int64_t)sizeof(VecT) < (1 << 20)) ? 1 : 0;
     kern<<<grid, NT, smem, c.stream>>>(A->nrows(), A->row_lo, D, u_lo, u_cnt, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val,
                                        (const VecT *)a.x, (const VecT *)a.z, (VecT *)a.y, a.alpha, a.gamma, a.beta, a.scal_mode, a.sc,
-                                       A->vdict, use_bulk, A->period_slices, A->period_entries);
+                                       A->vdict, A->cbits, use_bulk, A->period_slices, A->period_entries);
     QB_LAUNCH_COUNT();
     QB_CUDA(cudaGetLastError());
     return QBGPU_OK;
@@ -614,7 +636,12 @@ bool block_smem_applicable(const qbgpu_matrix *A, int64_t D)
 int launch_spmv_block_smem(const qbgpu_matrix *A, const FusedArgs &a, int64_t D)
 {
     if (a.dots) return fail(QBGPU_ERR_ARG, "block-local product: the running dots belong to the closing pass");
-    if (A->ndict) return A->api_complex ? launch_block_smem_cfg<uint8_t, double2, 1024, 4, 1>(A, a, D) : launch_block_smem_cfg<uint8_t, double, 1024, 4, 1>(A, a, D);
+    // packed words: a third of the bytes per entry, and a trip takes 8 diagonals instead of 4.  Diagonal k still accumulates
+    // into k & 1, so the products stay bit-identical.  On BASELINE config 3 (fp64 vectors, one B200 at 1000 W) the pass no
+    // longer follows the bytes in flight: 8 and 10 diagonals per trip measured 5.57 and 5.67 ms (12 spill at 64 registers a
+    // thread).  Complex vectors take 6 (10 spill).
+    if (A->cbits) return A->api_complex ? launch_block_smem_cfg<uint32_t, double2, 1024, 6, 1>(A, a, D) : launch_block_smem_cfg<uint32_t, double, 1024, 8, 1>(A, a, D);
+    if (A->ndict) return fail(QBGPU_ERR_STATE, "block-local product: 1-byte dictionary codes are not supported (internal)");
     if (!A->api_complex) return launch_block_smem_cfg<double, double, 1024, 4, 1>(A, a, D);
     if (A->val_real) return launch_block_smem_cfg<double, double2, 1024, 4, 1>(A, a, D);
     return launch_block_smem_cfg<double2, double2, 1024, 4, 1>(A, a, D);

@@ -349,6 +349,13 @@ __global__ void __launch_bounds__(kPBlock) species_fill_kernel(SpeciesView V, in
 }
 
 
+// the packed layout of a stored part: col[i] = col[i] | code[i] << cbits (qbgpu_matrix::cbits)
+__global__ void __launch_bounds__(kPBlock) pack_codes_kernel(int64_t nnz, uint32_t *col, const uint8_t *__restrict__ code, int cbits)
+{
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nnz; i += (int64_t)gridDim.x * blockDim.x)
+        col[i] = packed_word((int32_t)col[i], code[i], cbits);
+}
+
 static void make_slice_order(int64_t n, int64_t Dd, int W, std::vector<int32_t> &order)
 {
     const int64_t ns = (n + 31) / 32;
@@ -370,6 +377,7 @@ int species_build_stored(qbgpu_matrix_t *out, const HostTables &T, const ModelPa
     const double t0 = wall_s();
     SpeciesHost H;
     qbgpu_matrix *A = nullptr;
+    const bool rows_given = row_hi >= 0;                    // built as a row shard of a multi-GPU run (also one covering all rows)
     if (row_hi < 0) row_hi = T.dim;
     const bool shard = !(row_lo == 0 && row_hi == T.dim);
     QB_TRY(species_common(&A, T, M, api_complex, H, !shard));
@@ -417,13 +425,27 @@ int species_build_stored(qbgpu_matrix_t *out, const HostTables &T, const ModelPa
     }
     QB_CU(cudaStreamSynchronize(c.stream));
     QB_CU(cudaGetLastError());
-    // layout: always the sliced-jagged kernels (the traversal order of the cross part exists only there)
-    if (flags & QBGPU_VALUE_DICT) {
-        int rc = value_dict_encode(A);
-        if (rc == QBGPU_OK) rc = value_dict_encode(C);
+    // layout: always the sliced-jagged kernels (the traversal order of the cross part exists only there).  A part of a handle
+    // built without a row range, with real values, stores packed words (qbgpu_matrix::cbits) when its table of distinct values
+    // fits beside the columns: 4 bytes per entry instead of 12, and the products are bound by the matrix stream.  Handles built
+    // as row shards -- a one-rank shard covering all rows too -- keep separate fp64 values: the multi-GPU drivers split their
+    // cross parts by columns and rows (qbgpu_species_split_cross, qbgpu_row_view).  So do complex values.
+    const int cbits = packed_col_bits(n);
+    if (!rows_given && A->val_real) {
+        const int max_table = (int)std::min<int64_t>(kPackedMaxTable, (int64_t)1 << (32 - cbits));
+        int rc = value_dict_encode(A, max_table);           // (leaves a part whose table would not fit as it is)
+        if (rc == QBGPU_OK) rc = value_dict_encode(C, max_table);
         if (rc) { qbgpu_destroy(A); return rc; }
     }
     { int rc = sjds_convert(A, true); if (rc == QBGPU_OK) rc = sjds_convert(C, true); if (rc) { qbgpu_destroy(A); return rc; } }
+    for (qbgpu_matrix *P : {A, C}) {
+        if (!P->ndict) continue;
+        pack_codes_kernel<<<grid_rows(P->nnz), kPBlock, 0, c.stream>>>(P->nnz, (uint32_t *)P->col, (const uint8_t *)P->val, cbits);
+        QB_LAUNCH_COUNT();
+        QB_CU(cudaStreamSynchronize(c.stream));
+        QB_CU(cudaGetLastError());
+        cudaFree(P->val); P->val = nullptr; P->cbits = cbits;
+    }
     std::vector<int32_t> order;
     make_slice_order(nloc, Dd, S->tile, order);
     QB_CU(upload(&C->slice_order, order.data(), order.size(), c.stream));
@@ -1193,6 +1215,7 @@ int qbgpu_species_split_cross(qbgpu_matrix_t A, int nparts, const int64_t *bound
     const Species *S = (const Species *)A->sp;
     if (!S || S->matfree || !A->second || A->borrowed) return fail(QBGPU_ERR_STATE, "species_split_cross: needs the owning stored species-order handle");
     qbgpu_matrix *Cx = A->second;
+    if (Cx->cbits) return fail(QBGPU_ERR_STATE, "species_split_cross: the cross part stores packed entry words (a handle built without a row range); build it as a row shard to split it");
     if (Cx->ndict) return fail(QBGPU_ERR_STATE, "species_split_cross: not available with dictionary-coded values");
     QB_TRY(split_columns(Cx, nparts, bounds, parts, QBGPU_FORMAT_SELL | QBGPU_NO_AUTOTUNE));
     const int64_t ns = (Cx->nrows() + 31) / 32;
@@ -1219,6 +1242,7 @@ int qbgpu_row_view(qbgpu_matrix_t A, int64_t r0, int64_t r1, int64_t tile_period
     if (!A || !view) return fail(QBGPU_ERR_ARG, "null argument");
     *view = nullptr;
     if (A->sp || A->mf || A->mf_sec || A->format != QBGPU_FORMAT_SELL) return fail(QBGPU_ERR_STATE, "row_view: needs a stored sliced-jagged handle (a part of a species handle, a shard)");
+    if (A->cbits) return fail(QBGPU_ERR_STATE, "row_view: the part stores packed entry words (a species handle built without a row range); only the parts of row shards can be cut");
     const int64_t nl = A->nrows();
     if (r0 < 0 || r1 < r0 || r1 > nl || r0 % 32 != 0 || (r1 % 32 != 0 && r1 != nl)) return fail(QBGPU_ERR_ARG, "row_view: the row range must consist of whole 32-row slices");
     if (A->slice_order && (tile_period <= 0 || r0 % tile_period != 0)) return fail(QBGPU_ERR_ARG, "row_view: a tile-ordered part must be cut at multiples of its tile period (D_dn)");
@@ -1337,6 +1361,59 @@ int qbgpu_debug_species_host(int nsites, int nup, int ndn, int nbonds, const int
                 const double acc = H.uniform_w > 0 ? kron_cross_acc<double, false, true>(V, H.ampw, iu, live ? id : V.Dd - 1, x, 0, 0, H.ampw[H.uniform_w])
                                                    : kron_cross_acc<double, false, false>(V, H.ampw, iu, live ? id : V.Dd - 1, x);
                 if (live) { y[iu * V.Dd + id] += acc; if (touched) touched[iu * V.Dd + id]++; }
+            }
+    }
+    return QBGPU_OK;
+}
+
+/* The packed layout of the two stored parts (qbgpu_matrix::cbits), computed on the host with the build's rules: the entries of
+ * species_fill_row in CSR order, each part's table of distinct values ordered by value_table_less, words packed_word(col,
+ * code, cbits).  cbits <= 0: the build's own width, packed_col_bits(n).  out[0] = cbits; out[1], out[2] = table entries of the
+ * local / cross part; out[3], out[4] = 1 when that part is packed (its table fits beside the columns), 0 when it keeps separate
+ * fp64 values.  table_* (256 entries each) and words_* (nnz_local / nnz_cross of qbgpu_debug_species_host) may be NULL. */
+int qbgpu_debug_species_packed_host(int nsites, int nup, int ndn, int nbonds, const int32_t *bonds, double t, double U, int cbits,
+                                    int64_t *out, double *table_local, uint32_t *words_local, double *table_cross, uint32_t *words_cross)
+{
+    if (nsites < 2 || nup < 0 || ndn < 0 || nup > nsites || ndn > nsites || nbonds < 1 || !bonds || !out || cbits > 31)
+        return fail(QBGPU_ERR_ARG, "debug_species_packed_host: bad argument");
+    HostTables T;
+    QB_TRY(make_tables(nsites, 2, nup, ndn, T));
+    static thread_local ModelParams M;
+    M.kind = 1; M.J = 0; M.t = t; M.U = U;
+    QB_TRY(merge_bonds(nsites, nbonds, bonds, M));
+    SpeciesHost H;
+    QB_TRY(build_host_tables(nsites, nup, ndn, M, H));
+    SpeciesView V;
+    V.Du = (int64_t)H.list[0].size(); V.Dd = (int64_t)H.list[1].size(); V.tot_u = (int64_t)H.hop[0].size(); V.tot_d = (int64_t)H.hop[1].size();
+    V.ulist = H.list[0].data(); V.dlist = H.list[1].data(); V.uptr = H.ptr[0].data(); V.dptr = H.ptr[1].data();
+    V.uhop = H.hop[0].data(); V.dhop = H.hop[1].data();
+    const int64_t n = V.Du * V.Dd;
+    if (n != T.dim) return fail(QBGPU_ERR_STATE, "debug_species_packed_host: dimension mismatch with the Lin tables");
+    if (cbits <= 0) cbits = packed_col_bits(n);
+    std::vector<int32_t> col[2] = {std::vector<int32_t>((size_t)(V.Du * (V.tot_d + V.Dd))), std::vector<int32_t>((size_t)(V.Dd * V.tot_u))};
+    std::vector<double> val[2] = {std::vector<double>(col[0].size()), std::vector<double>(col[1].size())};
+    for (int64_t p = 0; p < n; p++) species_fill_row<double>(V, H.ampw, H.diagk, p, col[0].data(), val[0].data(), col[1].data(), val[1].data());
+    out[0] = cbits;
+    double *tables[2] = {table_local, table_cross};
+    uint32_t *words[2] = {words_local, words_cross};
+    for (int part = 0; part < 2; part++) {
+        std::vector<double> tab;
+        {   // distinct bit patterns, in the order of the build's table
+            std::vector<uint64_t> bits(val[part].size());
+            memcpy(bits.data(), val[part].data(), 8 * bits.size());
+            std::sort(bits.begin(), bits.end());
+            bits.erase(std::unique(bits.begin(), bits.end()), bits.end());
+            for (uint64_t b : bits) { double v; memcpy(&v, &b, 8); tab.push_back(v); }
+            std::sort(tab.begin(), tab.end(), value_table_less);
+        }
+        const bool packed = packed_table_fits((int64_t)tab.size(), cbits);
+        out[1 + part] = (int64_t)tab.size();
+        out[3 + part] = packed ? 1 : 0;
+        if (tables[part]) for (size_t j = 0; j < kPackedMaxTable; j++) tables[part][j] = j < tab.size() ? tab[j] : 0.0;
+        if (words[part] && packed)
+            for (size_t i = 0; i < val[part].size(); i++) {
+                const uint32_t code = (uint32_t)(std::lower_bound(tab.begin(), tab.end(), val[part][i], value_table_less) - tab.begin());
+                words[part][i] = packed_word(col[part][i], code, cbits);
             }
     }
     return QBGPU_OK;
