@@ -16,6 +16,9 @@
  *   - `where` says where vector pointers live: QBGPU_HOST (the reference's calling convention: std::vector /
  *     ARPACK workd) or QBGPU_DEVICE (already resident, e.g. a torch tensor's data_ptr).
  *   - all work is issued on one CUDA stream per thread context (qbgpu_set_stream to adopt the caller's).
+ *   - device vectors: complex vectors 16-byte aligned (read as double2), fp64 vectors 8-byte aligned.  Any such pointer
+ *     works, e.g. a window of a larger vector; an fp64 x that is also 16-byte aligned lets pass 1 of a species-order
+ *     product copy each block of x with one bulk copy instead of thread by thread.
  */
 #ifndef QBGPU_H
 #define QBGPU_H
@@ -39,7 +42,8 @@ extern "C" {
 #define QBGPU_KEEP_COMPLEX   1   /* do not demote an all-real complex matrix to fp64 values */
 #define QBGPU_NO_AUTOTUNE    2   /* skip the kernel-variant timing pass at create */
 #define QBGPU_FORMAT_CSR     4   /* force the expanded-CSR kernels  */
-#define QBGPU_FORMAT_SELL    8   /* force the sliced-jagged kernels (32-row slices, jagged diagonals, no padding) */
+#define QBGPU_FORMAT_SELL    8   /* force the sliced-jagged kernels (32-row slices, jagged diagonals, no padding); refused
+                                    for a row of 2^24 or more entries */
 #define QBGPU_FORMAT_MATFREE 32  /* (info only) matrix-free handle: rows are regenerated inside the product */
 #define QBGPU_MATFREE_TERMS 64  /* qbgpu_create_matfree_*: also store one byte per entry naming the Hamiltonian term that
                                   * produces it (directed bond x spin), so the product replays each row -- column from the
@@ -48,8 +52,9 @@ extern "C" {
                                   * (rank of the up configuration, rank of the down configuration) and multiply in two passes
                                   * (see "species order" below); results and calling convention are unchanged */
 #define QBGPU_VALUE_DICT    16   /* opt-in: store fp64 values as 1-byte codes into a table of the distinct values when there
-                                    are at most 256 of them (lossless; products are bit-identical); implies FORMAT_SELL.
-                                    Stored species-order handles pack their values without it (see "species order") */
+                                    are at most 256 of them (lossless; products are bit-identical); implies FORMAT_SELL, and
+                                    like it refuses a row of 2^24 or more entries (default create keeps such a matrix in the
+                                    CSR layout).  Stored species-order handles pack their values without it (see "species order") */
 
 typedef struct qbgpu_matrix *qbgpu_matrix_t;     /* replaces `sparse_matrix_t handle` (src/qbasis.h:985) */
 

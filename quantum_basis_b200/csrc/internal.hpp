@@ -104,6 +104,7 @@ struct FusedArgs {
 int launch_spmv(const qbgpu_matrix *A, const FusedArgs &args, int lanes_override = 0);
 int autotune(qbgpu_matrix *A, int flags = 0);
 int sjds_convert(qbgpu_matrix *A, bool forward);
+int sjds_rows_fit(const qbgpu_matrix *A, bool *fits);   // every row shorter than 2^24 entries (the sliced-jagged length field)
 int value_dict_encode(qbgpu_matrix *A, int max_entries = 256);   // matrix.cu: try to replace fp64 values by 1-byte codes
 // order of a value table: by value, -0.0 before +0.0 (distinct bit patterns), so that a layout does not depend on thread timing
 inline bool value_table_less(double a, double b) { return a != b ? a < b : std::signbit(a) > std::signbit(b); }

@@ -390,8 +390,7 @@ int launch_spmv_sjds(const qbgpu_matrix *A, const FusedArgs &a)
 template <typename ValT, bool FORWARD>
 __global__ void __launch_bounds__(kSBlock)
 sjds_permute_kernel(int64_t s0, int64_t s1, int64_t nrows, const int64_t *__restrict__ rowptr, uint32_t *rowinfo,
-                    const int32_t *__restrict__ col, const ValT *__restrict__ val, int64_t base0, int32_t *tcol, ValT *tval,
-                    int *too_long)
+                    const int32_t *__restrict__ col, const ValT *__restrict__ val, int64_t base0, int32_t *tcol, ValT *tval)
 {
     constexpr int WPB = kSBlock / 32;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -399,8 +398,7 @@ sjds_permute_kernel(int64_t s0, int64_t s1, int64_t nrows, const int64_t *__rest
         const int64_t r = s * 32 + lane;
         const int64_t rs = r < nrows ? rowptr[r] : 0;
         const int64_t len64 = r < nrows ? rowptr[r + 1] - rs : 0;
-        if (__any_sync(0xffffffffu, len64 > (int64_t)kLenMask)) { if (lane == 0) atomicExch(too_long, 1); continue; }   // warp-uniform
-        const int len = (int)len64;
+        const int len = (int)len64;                         // (< 2^24: checked by sjds_rows_fit before any entry moves)
         int rank = 0, maxlen = 0;
         for (int j = 0; j < 32; j++) {                      // rank by (length desc, lane asc): a stable sort of 32 keys
             const int lj = __shfl_sync(0xffffffffu, len, j);
@@ -422,6 +420,37 @@ sjds_permute_kernel(int64_t s0, int64_t s1, int64_t nrows, const int64_t *__rest
     }
 }
 
+__global__ void __launch_bounds__(kSBlock) sjds_row_too_long_kernel(int64_t nrows, const int64_t *__restrict__ rowptr, int *too_long)
+{
+    for (int64_t r = (int64_t)blockIdx.x * kSBlock + threadIdx.x; r < nrows; r += (int64_t)gridDim.x * kSBlock)
+        if (rowptr[r + 1] - rowptr[r] > (int64_t)kLenMask) *too_long = 1;
+}
+
+// Does every row fit the 24-bit length field of the sliced-jagged row metadata?  (Asked before the conversion moves any entry:
+// a refused conversion leaves the CSR arrays as they were.)
+int sjds_rows_fit(const qbgpu_matrix *A, bool *fits)
+{
+    Context &c = ctx();
+    *fits = true;
+    const int64_t nrows = A->nrows();
+    if (nrows == 0) return QBGPU_OK;
+    int *d_flag = nullptr;
+    int flag = 0;
+    QB_CUDA(cudaMalloc(&d_flag, sizeof(int)));
+    cudaError_t e = cudaMemsetAsync(d_flag, 0, sizeof(int), c.stream);
+    if (e == cudaSuccess) {
+        sjds_row_too_long_kernel<<<(int)std::min<int64_t>((nrows + kSBlock - 1) / kSBlock, 148 * 16), kSBlock, 0, c.stream>>>(nrows, A->rowptr, d_flag);
+        QB_LAUNCH_COUNT();
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost, c.stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c.stream);
+    cudaFree(d_flag);
+    QB_CUDA(e);
+    *fits = flag == 0;
+    return QBGPU_OK;
+}
+
 template <typename ValT>
 static int sjds_convert_typed(qbgpu_matrix *A, bool forward)
 {
@@ -429,17 +458,20 @@ static int sjds_convert_typed(qbgpu_matrix *A, bool forward)
     const int64_t nrows = A->nrows();
     const int64_t nslices = (nrows + 31) / 32;
     if (nslices == 0) return QBGPU_OK;
+    if (forward) {
+        bool fits = true;
+        QB_TRY(sjds_rows_fit(A, &fits));
+        if (!fits) return fail(QBGPU_ERR_STATE, "sliced-jagged layout: a row is longer than 2^24-1 entries");
+    }
     if (forward && !A->rowinfo) QB_CUDA(cudaMalloc(&A->rowinfo, sizeof(uint32_t) * nslices * 32));
     // batches of slices re-ordered through a bounded temporary, then copied back over the same range
     const int64_t batch = 1 << 16;                          // 65,536 slices = 2,097,152 rows per batch
     const int64_t nb = (nslices + batch - 1) / batch;
     std::vector<int64_t> bidx(nb + 1), bofs(nb + 1);
     for (int64_t b = 0; b <= nb; b++) bidx[b] = std::min(nrows, b * batch * 32);
-    int64_t *d_idx = nullptr, *d_ofs = nullptr;
-    int *d_flag = nullptr;
     int32_t *tcol = nullptr;
     ValT *tval = nullptr;
-    auto cleanup = [&]() { cudaFree(d_idx); cudaFree(d_ofs); cudaFree(d_flag); cudaFree(tcol); cudaFree(tval); };
+    auto cleanup = [&]() { cudaFree(tcol); cudaFree(tval); };
 #define QB_CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { cleanup(); return cuda_fail(e_, #call, __FILE__, __LINE__); } } while (0)
     // boundary offsets rowptr[bidx[b]]
     for (int64_t b = 0; b <= nb; b++) QB_CU(cudaMemcpyAsync(&bofs[b], A->rowptr + bidx[b], sizeof(int64_t), cudaMemcpyDeviceToHost, c.stream));
@@ -448,28 +480,23 @@ static int sjds_convert_typed(qbgpu_matrix *A, bool forward)
     for (int64_t b = 0; b < nb; b++) maxspan = std::max(maxspan, bofs[b + 1] - bofs[b]);
     QB_CU(cudaMalloc(&tcol, sizeof(int32_t) * maxspan));
     QB_CU(cudaMalloc(&tval, sizeof(ValT) * maxspan));
-    QB_CU(cudaMalloc(&d_flag, sizeof(int)));
-    QB_CU(cudaMemsetAsync(d_flag, 0, sizeof(int), c.stream));
     for (int64_t b = 0; b < nb; b++) {
         const int64_t s0 = b * batch, s1 = std::min(nslices, (b + 1) * batch);
         const int64_t span = bofs[b + 1] - bofs[b];
         if (span == 0 && !forward) continue;               // (forward still has to write rowinfo for all-empty slices)
         const int grid = (int)std::min<int64_t>((s1 - s0 + 7) / 8, 148 * 16);
-        if (forward) sjds_permute_kernel<ValT, true><<<grid, kSBlock, 0, c.stream>>>(s0, s1, nrows, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val, bofs[b], tcol, tval, d_flag);
-        else         sjds_permute_kernel<ValT, false><<<grid, kSBlock, 0, c.stream>>>(s0, s1, nrows, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val, bofs[b], tcol, tval, d_flag);
+        if (forward) sjds_permute_kernel<ValT, true><<<grid, kSBlock, 0, c.stream>>>(s0, s1, nrows, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val, bofs[b], tcol, tval);
+        else         sjds_permute_kernel<ValT, false><<<grid, kSBlock, 0, c.stream>>>(s0, s1, nrows, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val, bofs[b], tcol, tval);
         QB_LAUNCH_COUNT();
         if (span) {
             QB_CU(cudaMemcpyAsync(A->col + bofs[b], tcol, sizeof(int32_t) * span, cudaMemcpyDeviceToDevice, c.stream));
             QB_CU(cudaMemcpyAsync((ValT *)A->val + bofs[b], tval, sizeof(ValT) * span, cudaMemcpyDeviceToDevice, c.stream));
         }
     }
-    int flag = 0;
-    QB_CU(cudaMemcpyAsync(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
     QB_CU(cudaStreamSynchronize(c.stream));
     QB_CU(cudaGetLastError());
     cleanup();
 #undef QB_CU
-    if (flag) return fail(QBGPU_ERR_STATE, "sliced-jagged layout: a row is longer than 2^24-1 entries");
     A->format = forward ? QBGPU_FORMAT_SELL : QBGPU_FORMAT_CSR;
     return QBGPU_OK;
 }

@@ -612,7 +612,10 @@ static int launch_block_smem_cfg(const qbgpu_matrix *A, const FusedArgs &a, int6
     if (u_cnt == 0) return QBGPU_OK;
     const int64_t cap = (int64_t)c.num_sms * bps;
     const int grid = (int)(u_cnt < cap ? u_cnt : cap);
-    const int use_bulk = ((D * (int64_t)sizeof(VecT)) % 16 == 0 && D * (int64_t)sizeof(VecT) < (1 << 20)) ? 1 : 0;
+    // cp.async.bulk needs a 16-byte-aligned source: every block of x starts at x + u*D, so D*sizeof(VecT) and x itself must be
+    // multiples of 16 (an fp64 x passed to the internal-order entry points may be only 8-byte aligned, e.g. a window of a
+    // larger vector); otherwise the threads copy the block
+    const int use_bulk = ((D * (int64_t)sizeof(VecT)) % 16 == 0 && D * (int64_t)sizeof(VecT) < (1 << 20) && ((uintptr_t)a.x & 15) == 0) ? 1 : 0;
     kern<<<grid, NT, smem, c.stream>>>(A->nrows(), A->row_lo, D, u_lo, u_cnt, A->rowptr, A->rowinfo, A->col, (const ValT *)A->val,
                                        (const VecT *)a.x, (const VecT *)a.z, (VecT *)a.y, a.alpha, a.gamma, a.beta, a.scal_mode, a.sc,
                                        A->vdict, A->cbits, use_bulk, A->period_slices, A->period_entries);

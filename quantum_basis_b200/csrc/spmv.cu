@@ -195,7 +195,9 @@ int autotune(qbgpu_matrix *A, int flags)
         if (ms < best) { best = ms; best_lanes = l; }
     }
     A->lanes = best_lanes;
-    if (!(flags & QBGPU_FORMAT_CSR)) {                       // try the sliced-jagged layout; keep it only if faster
+    bool sell_fits = !(flags & QBGPU_FORMAT_CSR);
+    if (sell_fits) QB_TRY(sjds_rows_fit(A, &sell_fits));   // a row of 2^24 entries or more: CSR-vector serves it alone
+    if (sell_fits) {                                        // try the sliced-jagged layout; keep it only if faster
         QB_TRY(sjds_convert(A, true));
         float ms = 0;
         QB_TRY(time3(0, ms));
