@@ -430,6 +430,29 @@ int qbgpu_sector_apply_sz(qbgpu_sector_t S_old, qbgpu_sector_t S_new, const doub
  * several threads in no fixed order either -- so results agree with it to rounding, not to the bit. */
 int qbgpu_sector_apply_ladder(qbgpu_sector_t S_old, qbgpu_sector_t S_new, int lower, const double *coef_reim,
                               const void *x_old_dev, void *y_new_dev);
+/* The same routine for one-site ELECTRON operators A = sum_r c_r O_r between electron sectors of one lattice (coefficients
+ * *_reim[2*nsites] in site order; device vectors x_old_dev (S_old) -> y_new_dev (S_new), which is overwritten).  The target
+ * momentum is the caller's choice, as for the spin entries:
+ *   - coefficients e^{+i q.r} move a vector from momentum K to K + q (S^z_q, n_q, S^-_q of the reference's examples);
+ *   - c_k = N^{-1/2} sum_r e^{-i k.r} c_r moves it from K to K - k, c+_k = N^{-1/2} sum_r e^{+i k.r} c+_r from K to K + k.
+ * Source rows with |x| < 2e-12 and rows of zero norm in either sector contribute nothing (src/model.cc:1752,1760,1810).
+ * Single-electron operators carry oprXphi's sign (src/basis.cc:2717-2731) and the translation sign of the representative
+ * in the sector they land in.  Every output row is computed once, in a fixed term order (the adjoint of A applied to the
+ * target representative), so repeated calls are bit-identical; for coefficients e^{+i q.r} between K and K + q this is the
+ * reference's scatter to rounding.  QBGPU_ERR_STATE on a spin sector, QBGPU_ERR_ARG on another lattice or particle numbers
+ * that do not match the operator. */
+/* A = sum_r cu[r] n_up,r + cd[r] n_dn,r.  S_old, S_new: same lattice, same N_up and N_dn.
+ * S^z_q: cd = -cu.  Charge n_q: cd = cu. */
+int qbgpu_sector_apply_density(qbgpu_sector_t S_old, qbgpu_sector_t S_new, const double *cu_reim,
+                               const double *cd_reim, const void *x_old_dev, void *y_new_dev);
+/* lower = 1: A = sum_r c[r] c+_{r,dn} c_{r,up}  (S^-; S_new has N_up-1, N_dn+1)
+ * lower = 0: the S^+ counterpart                 (S_new has N_up+1, N_dn-1) */
+int qbgpu_sector_apply_spin_flip(qbgpu_sector_t S_old, qbgpu_sector_t S_new, int lower,
+                                 const double *c_reim, const void *x_old_dev, void *y_new_dev);
+/* create = 0: A = sum_r c[r] c_{r,spin}   (S_new has one electron fewer of that spin; spin 0 up, 1 down)
+ * create = 1: A = sum_r c[r] c+_{r,spin}  (S_new has one more) */
+int qbgpu_sector_apply_fermion(qbgpu_sector_t S_old, qbgpu_sector_t S_new, int create, int spin,
+                               const double *c_reim, const void *x_old_dev, void *y_new_dev);
 /* Momentum sector for an ARBITRARY abelian symmetry group given as site permutations (BASELINE config 4: the tilted
  * 31-site triangular cluster, which the reference itself cannot build -- SURVEY F5 -- so there is no reference convention
  * to reproduce; representative = smallest bit pattern of the orbit, orbits on whose stabiliser the character is not

@@ -211,6 +211,38 @@ public:
         check(qbgpu_sector_build_hubbard(handle, &h, static_cast<int>(hops.size() / 3), hops.data(), t, U, fake_pos, flags), "qbgpu_sector_build_hubbard");
         return csr_mat<std::complex<double>>::adopt(h);
     }
+    // model::moprXvec_repr (src/model.cc:1716-1846) for one-site electron operators on device vectors: x_dev (this sector) ->
+    // y_dev (target, overwritten), one coefficient per site.  Coefficients e^{+i q.r} move a vector from K to K + q.
+    // A = sum_r cu[r] n_up,r + cd[r] n_dn,r (target: same particle numbers)
+    void apply_density(const electron_sector &target, const std::vector<std::complex<double>> &cu, const std::vector<std::complex<double>> &cd,
+                       const std::complex<double> *x_dev, std::complex<double> *y_dev) const
+    {
+        coef_size(cu); coef_size(cd);
+        check(qbgpu_sector_apply_density(handle, target.handle, reinterpret_cast<const double *>(cu.data()), reinterpret_cast<const double *>(cd.data()),
+                                         x_dev, y_dev), "qbgpu_sector_apply_density");
+    }
+    // A = sum_r c[r] c+_{r,dn} c_{r,up} (lower, S^-) or c+_{r,up} c_{r,dn} (S^+)
+    void apply_spin_flip(const electron_sector &target, bool lower, const std::vector<std::complex<double>> &c,
+                         const std::complex<double> *x_dev, std::complex<double> *y_dev) const
+    {
+        coef_size(c);
+        check(qbgpu_sector_apply_spin_flip(handle, target.handle, lower ? 1 : 0, reinterpret_cast<const double *>(c.data()), x_dev, y_dev),
+              "qbgpu_sector_apply_spin_flip");
+    }
+    // A = sum_r c[r] c_{r,spin} (create false) or c+_{r,spin}; spin 0 up, 1 down
+    void apply_fermion(const electron_sector &target, bool create, int spin, const std::vector<std::complex<double>> &c,
+                       const std::complex<double> *x_dev, std::complex<double> *y_dev) const
+    {
+        coef_size(c);
+        check(qbgpu_sector_apply_fermion(handle, target.handle, create ? 1 : 0, spin, reinterpret_cast<const double *>(c.data()), x_dev, y_dev),
+              "qbgpu_sector_apply_fermion");
+    }
+
+private:
+    void coef_size(const std::vector<std::complex<double>> &c) const
+    {
+        if (static_cast<int>(c.size()) != info.nsites) throw std::runtime_error("qbgpu::electron_sector: one coefficient per site");
+    }
 };
 
 }  // namespace qbgpu

@@ -7,5 +7,5 @@ is the thin host-side mirror of the reference's interface for that path (``csr_m
 """
 from ._lib import lib, QbgpuError, build_library, LIB_PATH  # noqa: F401
 from .csr import (csr_mat, lanczos, eigenvec_CG, eigenvec_CG_stepwise, energy_scale, kpm_moments, kpm_moments_stepwise, hess_eigen, vec_randomize,  # noqa: F401
-                  locate_E0_lanczos, locate_E0_iram, locate_Emax_iram, iram, trlan, herm_eigen, heisenberg, hubbard, heisenberg_orbit, Sector, ElectronSector, measure_repr_dynamic, measure_full_dynamic, measure_vrnl_dynamic, full_apply_diag, vec_disk_write, vec_disk_read, DeviceVector, lanczos_precision)
+                  locate_E0_lanczos, locate_E0_iram, locate_Emax_iram, iram, trlan, herm_eigen, heisenberg, hubbard, heisenberg_orbit, Sector, ElectronSector, measure_repr_dynamic, measure_repr_dynamic_electron, continued_fraction, measure_full_dynamic, measure_vrnl_dynamic, full_apply_diag, vec_disk_write, vec_disk_read, DeviceVector, lanczos_precision)
 from . import ckpt  # noqa: F401,E402  (reference-format Lanczos checkpoints, src/ckpt.cc)

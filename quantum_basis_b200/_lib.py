@@ -89,6 +89,8 @@ _SIGS = {
     "qbgpu_sector_create_electron": [C.POINTER(vp), C.c_int, vp, C.c_int, C.c_int, vp],
     "qbgpu_sector_build_hubbard": [vp, C.POINTER(vp), C.c_int, vp, dbl, dbl, dbl, C.c_int],
     "qbgpu_sector_apply_sz": [vp, vp, vp, vp, vp], "qbgpu_sector_apply_ladder": [vp, vp, C.c_int, vp, vp, vp],
+    "qbgpu_sector_apply_density": [vp, vp, vp, vp, vp, vp], "qbgpu_sector_apply_spin_flip": [vp, vp, C.c_int, vp, vp, vp],
+    "qbgpu_sector_apply_fermion": [vp, vp, C.c_int, C.c_int, vp, vp, vp],
     "qbgpu_full_apply_diag": [C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp],
     "qbgpu_debug_full_apply_diag_host": [C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp],
     "qbgpu_native_order": [vp, C.POINTER(C.c_int)], "qbgpu_vec_to_native": [vp, vp, vp], "qbgpu_vec_from_native": [vp, vp, vp],

@@ -434,6 +434,50 @@ class ElectronSector(Sector):
         check(lib().qbgpu_sector_build_hubbard(self._h, C.byref(h), int(h3.shape[0]), C.c_void_p(h3.ctypes.data), float(t), float(U), float(fake_pos), flags))
         return csr_mat._adopt(h, True)
 
+    # model::moprXvec_repr (src/model.cc:1716-1846) for one-site electron operators, x in this sector -> DeviceVector in
+    # `new_sector` (written into `out` when given).  Coefficients e^{+i q.r} move a vector from momentum K to K + q;
+    # c_k = N^{-1/2} sum_r e^{-i k.r} c_r moves it from K to K - k.  See include/qbgpu.h for the sign and norm rules.
+    def _coef(self, c):
+        cf = np.ascontiguousarray(c, dtype=np.complex128)
+        if cf.size != self.nsites:
+            raise QbgpuError("one coefficient per site")
+        return cf
+
+    def _xy(self, new_sector, x, out):
+        xd = x if isinstance(x, DeviceVector) else DeviceVector.from_numpy(np.ascontiguousarray(x, dtype=np.complex128))
+        if xd.n < self.dim:
+            raise QbgpuError("x must hold the dimension of this sector")
+        y = out if out is not None else DeviceVector(new_sector.dim)
+        if y.n < new_sector.dim:
+            raise QbgpuError("out must hold the dimension of the new sector")
+        return xd, y
+
+    def apply_density(self, new_sector, cu, cd, x, out=None):
+        """A = sum_r cu[r] n_up,r + cd[r] n_dn,r (S^z_q: cd = -cu; charge density n_q: cd = cu); `new_sector` has the same
+        particle numbers."""
+        a, b = self._coef(cu), self._coef(cd)
+        xd, y = self._xy(new_sector, x, out)
+        check(lib().qbgpu_sector_apply_density(self._h, new_sector._h, C.c_void_p(a.ctypes.data), C.c_void_p(b.ctypes.data),
+                                               C.c_void_p(xd.ptr), C.c_void_p(y.ptr)))
+        return y
+
+    def apply_spin_flip(self, new_sector, c, x, lower=True, out=None):
+        """A = sum_r c[r] c+_{r,dn} c_{r,up} (lower=True, S^-: `new_sector` has N_up - 1, N_dn + 1) or its S^+ counterpart."""
+        cf = self._coef(c)
+        xd, y = self._xy(new_sector, x, out)
+        check(lib().qbgpu_sector_apply_spin_flip(self._h, new_sector._h, int(bool(lower)), C.c_void_p(cf.ctypes.data),
+                                                 C.c_void_p(xd.ptr), C.c_void_p(y.ptr)))
+        return y
+
+    def apply_fermion(self, new_sector, c, x, create=False, spin=0, out=None):
+        """A = sum_r c[r] c_{r,spin} (create=False: `new_sector` has one electron fewer of that spin) or sum_r c[r] c+_{r,spin};
+        spin 0 is up, 1 is down."""
+        cf = self._coef(c)
+        xd, y = self._xy(new_sector, x, out)
+        check(lib().qbgpu_sector_apply_fermion(self._h, new_sector._h, int(bool(create)), int(spin), C.c_void_p(cf.ctypes.data),
+                                               C.c_void_p(xd.ptr), C.c_void_p(y.ptr)))
+        return y
+
 
 def measure_repr_dynamic(coef, sec_old, sec_new, mat_new, phi0, maxit, hessenberg, op="sz"):
     """model<T>::measure_repr_dynamic (src/model.cc:1897-1912) for A = sum_r coef[r] S^z_r (op="sz"), S^-_r ("s-") or
@@ -458,6 +502,53 @@ def measure_repr_dynamic(coef, sec_old, sec_new, mat_new, phi0, maxit, hessenber
     m = lanczos(0, maxit - 1, maxit, n, mat_new, v, hessenberg, "dnmcs")
     v.free()
     return m, nr.value
+
+
+def measure_repr_dynamic_electron(op, coefs, sec_old, sec_new, mat_new, phi0, maxit, hessenberg):
+    """model<T>::measure_repr_dynamic (src/model.cc:1897-1912) for one-site electron operators between ElectronSectors:
+    vec = A phi0 mapped into sec_new, norm = |vec|, then lanczos(0, maxit-1, maxit, ..., "dnmcs") from vec/norm on `mat_new`.
+      op = "density":             coefs = (cu, cd)     A = sum_r cu[r] n_up,r + cd[r] n_dn,r
+      op = "s-" / "s+":           coefs = c            A = sum_r c[r] c+_{r,dn} c_{r,up} / c+_{r,up} c_{r,dn}
+      op = "c_up" / "c_dn":       coefs = c            A = sum_r c[r] c_{r,s}
+      op = "cdag_up" / "cdag_dn": coefs = c            A = sum_r c[r] c+_{r,s}
+    Returns (m, norm) like measure_repr_dynamic; hessenberg[2*maxit] receives b in [0, m) and a in [maxit, maxit+m).  With
+    norm below lanczos_precision nothing is run and m = 0."""
+    n = sec_new.dim
+    v = DeviceVector(2 * n)
+    v.zero()
+    y = v.view(0, n)
+    if op == "density":
+        cu, cd = coefs
+        sec_old.apply_density(sec_new, cu, cd, phi0, out=y)
+    elif op in ("s-", "s+"):
+        sec_old.apply_spin_flip(sec_new, coefs, phi0, lower=(op == "s-"), out=y)
+    elif op in ("c_up", "c_dn", "cdag_up", "cdag_dn"):
+        sec_old.apply_fermion(sec_new, coefs, phi0, create=op.startswith("cdag"), spin=int(op.endswith("dn")), out=y)
+    else:
+        v.free()
+        raise QbgpuError("op must be 'density', 's-', 's+', 'c_up', 'c_dn', 'cdag_up' or 'cdag_dn'")
+    nr = C.c_double()
+    check(lib().qbgpu_dznrm2(n, C.c_void_p(v.ptr), C.byref(nr)))
+    if abs(nr.value) < lanczos_precision:
+        v.free()
+        return 0, nr.value
+    check(lib().qbgpu_zscal(n, (C.c_double * 2)(1.0 / nr.value, 0.0), C.c_void_p(v.ptr)))
+    m = lanczos(0, maxit - 1, maxit, n, mat_new, v, hessenberg, "dnmcs")
+    v.free()
+    return m, nr.value
+
+
+def continued_fraction(a, b, z):
+    """G(z) = 1 / (z - a_0 - b_1^2 / (z - a_1 - b_2^2 / ...)) from Lanczos coefficients a[0..m), b[0..m) (b[0] unused): the
+    evaluation of the reference's examples/trans_absent/latt_chain/plot_sqw.py:77-89.  With the dnmcs coefficients of
+    A phi0 / |A phi0| and z = E0 + omega + i eta, -|A phi0|^2 Im G / pi is the broadened spectral weight of A at omega."""
+    a = np.asarray(a, dtype=np.float64)
+    b = np.asarray(b, dtype=np.float64)
+    z = np.asarray(z)
+    g = np.zeros(z.shape, dtype=np.complex128)
+    for j in range(len(a) - 1, -1, -1):
+        g = 1.0 / (z - a[j] - (b[j + 1] ** 2 * g if j + 1 < len(a) else 0.0))
+    return g
 
 
 def full_apply_diag(kind, nsites, n0, n1, coef0, coef1, x, out=None):

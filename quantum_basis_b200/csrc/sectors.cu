@@ -614,6 +614,99 @@ __global__ void __launch_bounds__(kSBlock) sec_apply_ladder_kernel(SecDev So, Se
     }
 }
 
+// ------------------------------------------------------------------------------------------ one-site electron operators
+// model::moprXvec_repr (src/model.cc:1716-1846) for A = sum_r c_r O_r between electron sectors of one lattice (restated and pinned
+// in tests/repr_ops_fermion.py).  Coefficients travel by value: at most 16 sites.
+struct ElCoef { double2 c[2][16]; };
+
+// Diagonal branch (:1758-1761), O_r = cu_r n_up,r + cd_r n_dn,r: the representative keeps its row and
+//   y[j] = sqrt(nu_old[j] / nu_new[j]) * x[j] * sum_r (cu_r n_up,r + cd_r n_dn,r)(state_j),
+// rows with |x[j]|, nu_old[j] or nu_new[j] below lanczos_precision give 0 (:1752, :1760).
+__global__ void __launch_bounds__(kSBlock) el_apply_density_kernel(SecDev S, const double *__restrict__ nu_new, ElCoef C,
+                                                                   const double2 *__restrict__ x, double2 *y)
+{
+    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < S.n; r += (int64_t)gridDim.x * blockDim.x) {
+        const double2 xj = x[r];
+        const double nj = S.nu[r], ni = nu_new[r];
+        double2 out = make_double2(0.0, 0.0);
+        if (hypot(xj.x, xj.y) >= 2e-12 && nj >= 2e-12 && ni >= 2e-12) {
+            uint32_t a, b;
+            sec_halves(S, S.keys[r], a, b);
+            const uint32_t st = sec_zip(S, a, b);
+            double2 d = make_double2(0.0, 0.0);
+            for (int site = 0; site < S.nsites; site++) {
+                if ((st >> (2 * site)) & 1u) { d.x = __dadd_rn(d.x, C.c[0][site].x); d.y = __dadd_rn(d.y, C.c[0][site].y); }
+                if ((st >> (2 * site + 1)) & 1u) { d.x = __dadd_rn(d.x, C.c[1][site].x); d.y = __dadd_rn(d.y, C.c[1][site].y); }
+            }
+            const double w = __dsqrt_rn(__ddiv_rn(nj, ni));
+            const double2 t = make_double2(__dmul_rn(w, xj.x), __dmul_rn(w, xj.y));
+            out = make_double2(__dsub_rn(__dmul_rn(t.x, d.x), __dmul_rn(t.y, d.y)), __dadd_rn(__dmul_rn(t.x, d.y), __dmul_rn(t.y, d.x)));
+        }
+        y[r] = out;
+    }
+}
+
+// c_{r,sp} (create = 0) or c+_{r,sp} on st with oprXphi's sign (src/basis.cc:2717-2731, the halves of el_hop): parity of the
+// electrons below site r, and for spin down the up electron of site r, counted on the state the operator acts on.
+__device__ __forceinline__ bool el_one(uint32_t st, int r, int sp, int create, uint32_t &s2, int &sg)
+{
+    const uint32_t bit = 1u << (2 * r + sp);
+    if (create ? (st & bit) != 0u : (st & bit) == 0u) return false;
+    sg = __popc(st & ((1u << (2 * r)) - 1u)) & 1;
+    if (sp) sg ^= (st >> (2 * r)) & 1u;
+    s2 = st ^ bit;
+    return true;
+}
+
+// Off-diagonal branch (:1762-1834) for one- and two-operator terms on one site (c, c+, S^- = c+_dn c_up, S^+ = c+_up c_dn).  The
+// reference scatters every term of the OLD representative j into the new sector,
+//     y[i] += sqrt(nu_old[j] / nu_new[i]) * x[j] * c_r * conj(phase_new[t]) * (-1)^(operator sign + el_trans_sign(rep_i, t)),
+// which needs fp64 atomics and lands in no fixed order.  Here every output row is written once instead: the ADJOINT term
+// (nops operators ops[0] then ops[1], each (spin, create)) acts on the NEW representative i, the state it produces is brought to
+// its representative j in the OLD sector with the same rule, and y[i] takes the conjugate of that element:
+//     y[i] = sum_r sqrt(nu_new[i] / nu_old[j]) * c_r * phase_old[t] * (-1)^(operator sign + el_trans_sign(rep_j, t)) * x[j],
+// terms in site order -- the same matrix for coefficients e^{+i q.r} between K and K + q, bit-identical from run to run.
+__global__ void __launch_bounds__(kSBlock) el_apply_gather_kernel(SecDev So, SecDev Sn, const double2 *__restrict__ phase_old, ElCoef C,
+                                                                  int nops, int sp0, int cr0, int sp1, int cr1,
+                                                                  const double2 *__restrict__ x, double2 *y)
+{
+    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < Sn.n; r += (int64_t)gridDim.x * blockDim.x) {
+        const double ni = Sn.nu[r];
+        double2 acc = make_double2(0.0, 0.0);
+        if (ni >= 2e-12) {
+            uint32_t a, b;
+            sec_halves(Sn, Sn.keys[r], a, b);
+            const uint32_t st = sec_zip(Sn, a, b);
+            for (int site = 0; site < Sn.nsites; site++) {
+                uint32_t s1, s2;
+                int g1, g2 = 0;
+                if (!el_one(st, site, sp0, cr0, s1, g1)) continue;
+                s2 = s1;
+                if (nops == 2 && !el_one(s1, site, sp1, cr1, s2, g2)) continue;
+                uint32_t a2, b2, ca = 0, cb = 0;
+                sec_unzip(So, s2, a2, b2);
+                const int t = sec_canon(So, a2, b2, ca, cb);
+                if (t < 0) continue;
+                const int64_t j = sec_lookup(So, sec_key(So, ca, cb));
+                if (j < 0) continue;
+                const double nj = So.nu[j];
+                if (!(nj >= 2e-12)) continue;                                          // :1810
+                const double2 xj = x[j];
+                if (!(hypot(xj.x, xj.y) >= 2e-12)) continue;                           // :1752
+                const double w = __dsqrt_rn(__ddiv_rn(ni, nj));
+                const double2 cf = C.c[0][site], ph = phase_old[t];
+                const double2 cp = make_double2(__dsub_rn(__dmul_rn(cf.x, ph.x), __dmul_rn(cf.y, ph.y)),
+                                                __dadd_rn(__dmul_rn(cf.x, ph.y), __dmul_rn(cf.y, ph.x)));
+                double re = __dmul_rn(w, __dsub_rn(__dmul_rn(cp.x, xj.x), __dmul_rn(cp.y, xj.y)));
+                double im = __dmul_rn(w, __dadd_rn(__dmul_rn(cp.x, xj.y), __dmul_rn(cp.y, xj.x)));
+                if ((g1 ^ g2 ^ el_trans_sign(So, sec_zip(So, ca, cb), t)) & 1) { re = -re; im = -im; }
+                acc.x = __dadd_rn(acc.x, re); acc.y = __dadd_rn(acc.y, im);
+            }
+        }
+        y[r] = acc;
+    }
+}
+
 static double wall_clock() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 struct FlagToInt { __host__ __device__ int operator()(uint8_t f) const { return (int)f; } };
 static int sgrid(int64_t n) { int64_t g = (n + kSBlock - 1) / kSBlock; if (g < 1) g = 1; if (g > 148 * 64) g = 148 * 64; return (int)g; }
@@ -1034,6 +1127,80 @@ int qbgpu_sector_apply_ladder(qbgpu_sector_t S_old, qbgpu_sector_t S_new, int lo
     QB_CUDA(e);
     QB_CUDA(cudaGetLastError());
     return QBGPU_OK;
+}
+
+}  // extern "C"
+
+// checks shared by the electron operator entries: both sectors electron sectors (else QBGPU_ERR_STATE) on one lattice, and
+// S_new's particle numbers (nup, ndn) = S_old's + (dup, ddn)
+static int el_op_check(const char *who, qbgpu_sector_t So, qbgpu_sector_t Sn, const void *coef, const void *x, const void *y, int dup, int ddn)
+{
+    char msg[160];
+    if (!So || !Sn || !coef || !x || !y) { snprintf(msg, sizeof(msg), "%s: null argument", who); return fail(QBGPU_ERR_ARG, msg); }
+    if (!So->electron || !Sn->electron) { snprintf(msg, sizeof(msg), "%s: electron sectors only", who); return fail(QBGPU_ERR_STATE, msg); }
+    if (So->nsites != Sn->nsites || So->dim != Sn->dim || memcmp(So->L, Sn->L, sizeof(So->L)) != 0) {
+        snprintf(msg, sizeof(msg), "%s: the two sectors must share the lattice", who); return fail(QBGPU_ERR_ARG, msg);
+    }
+    if (Sn->ndown != So->ndown + dup || Sn->ndn != So->ndn + ddn) {
+        snprintf(msg, sizeof(msg), "%s: the target sector must have (N_up, N_dn) = (%d, %d), it has (%d, %d)", who, So->ndown + dup, So->ndn + ddn,
+                 Sn->ndown, Sn->ndn);
+        return fail(QBGPU_ERR_ARG, msg);
+    }
+    return QBGPU_OK;
+}
+
+static int el_gather(qbgpu_sector_t So, qbgpu_sector_t Sn, const double *c_reim, int nops, int sp0, int cr0, int sp1, int cr1, const void *x, void *y)
+{
+    Context &c = ctx();
+    ElCoef C;
+    memset(&C, 0, sizeof(C));
+    memcpy(C.c[0], c_reim, sizeof(double2) * So->nsites);
+    el_apply_gather_kernel<<<sgrid(Sn->n), kSBlock, 0, c.stream>>>(So->dev, Sn->dev, So->d_phase, C, nops, sp0, cr0, sp1, cr1,
+                                                                   (const double2 *)x, (double2 *)y);
+    QB_LAUNCH_COUNT();
+    QB_CUDA(cudaGetLastError());
+    QB_CUDA(cudaStreamSynchronize(c.stream));
+    return QBGPU_OK;
+}
+
+extern "C" {
+
+int qbgpu_sector_apply_density(qbgpu_sector_t S_old, qbgpu_sector_t S_new, const double *cu_reim, const double *cd_reim, const void *x_old_dev,
+                               void *y_new_dev)
+{
+    const int rc = el_op_check("sector_apply_density", S_old, S_new, cu_reim, x_old_dev, y_new_dev, 0, 0);
+    if (rc != QBGPU_OK) return rc;
+    if (!cd_reim) return fail(QBGPU_ERR_ARG, "sector_apply_density: null argument");
+    if (S_old->n != S_new->n || S_old->dev.lin_order != S_new->dev.lin_order) return fail(QBGPU_ERR_ARG, "sector_apply_density: different representatives");
+    Context &c = ctx();
+    ElCoef C;
+    memset(&C, 0, sizeof(C));
+    memcpy(C.c[0], cu_reim, sizeof(double2) * S_old->nsites);
+    memcpy(C.c[1], cd_reim, sizeof(double2) * S_old->nsites);
+    el_apply_density_kernel<<<sgrid(S_old->n), kSBlock, 0, c.stream>>>(S_old->dev, S_new->d_nu, C, (const double2 *)x_old_dev, (double2 *)y_new_dev);
+    QB_LAUNCH_COUNT();
+    QB_CUDA(cudaGetLastError());
+    QB_CUDA(cudaStreamSynchronize(c.stream));
+    return QBGPU_OK;
+}
+
+int qbgpu_sector_apply_spin_flip(qbgpu_sector_t S_old, qbgpu_sector_t S_new, int lower, const double *c_reim, const void *x_old_dev, void *y_new_dev)
+{
+    const int rc = el_op_check("sector_apply_spin_flip", S_old, S_new, c_reim, x_old_dev, y_new_dev, lower ? -1 : 1, lower ? 1 : -1);
+    if (rc != QBGPU_OK) return rc;
+    // the adjoint term acting on the new representative: S^+ = c+_up c_dn for lower, S^- = c+_dn c_up otherwise
+    return lower ? el_gather(S_old, S_new, c_reim, 2, 1, 0, 0, 1, x_old_dev, y_new_dev)
+                 : el_gather(S_old, S_new, c_reim, 2, 0, 0, 1, 1, x_old_dev, y_new_dev);
+}
+
+int qbgpu_sector_apply_fermion(qbgpu_sector_t S_old, qbgpu_sector_t S_new, int create, int spin, const double *c_reim, const void *x_old_dev,
+                               void *y_new_dev)
+{
+    if (spin != 0 && spin != 1) return fail(QBGPU_ERR_ARG, "sector_apply_fermion: spin is 0 (up) or 1 (down)");
+    const int d = create ? 1 : -1;
+    const int rc = el_op_check("sector_apply_fermion", S_old, S_new, c_reim, x_old_dev, y_new_dev, spin == 0 ? d : 0, spin == 1 ? d : 0);
+    if (rc != QBGPU_OK) return rc;
+    return el_gather(S_old, S_new, c_reim, 1, spin, create ? 0 : 1, 0, 0, x_old_dev, y_new_dev);    // adjoint: c+ for c, c for c+
 }
 
 int qbgpu_sector_build_heisenberg(qbgpu_sector_t S, qbgpu_matrix_t *A, int nbonds, const int32_t *bonds, double J, double fake_pos, int flags)
