@@ -505,9 +505,27 @@ int qbgpu_species_ref_rows(int nsites, int nup, int ndn, int64_t row_lo, int64_t
  * wrote are final everywhere); bit 1 (2): barrier AFTER the product (every rank's pulls are done: the own slice of X[b] may be
  * rewritten).  Without bit 1 write the next x into the other buffer (the loops below ping-pong) or call qbgpu_dist_barrier. */
 int qbgpu_dist_mv(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, int b, void *y_local_dev, int barrier);
-/* lanczos(0, np, maxit, ...) of src/lanczos.cc:134-266 on the shards: "sr_val0" with the stop rule of :228-248, or "dnmcs" */
+/* lanczos(0, np, maxit, ...) of src/lanczos.cc:134-266 on the shards: "sr_val0" with the stop rule of :228-248, or "dnmcs"
+ * ("sr_val1" needs phi0: qbgpu_dist_lanczos_val1) */
 int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, int64_t np, int64_t maxit, int64_t *m,
                        double *hess, const char *purpose, int stop_on_breakdown);
+/* lanczos(0, np, maxit, ..., "sr_val1") of src/lanczos.cc:134-266 on the shards: the loop of qbgpu_dist_lanczos (stop rule of
+ * sr_val0) with the re-orthogonalisation against phi0 of :218-226 in every step after the first.  Start: the normalised start
+ * vector, orthogonal to phi0, in the own slice of X[0] and visible to the peers.  phi0_local: this rank's rows of phi0 (device,
+ * element type of D, in the shard's order), not NULL.  The projection is decided on the device from the all-reduced
+ * <phi0, v_m> (|<phi0, v_m>| > 2e-12, as the reference) and is in the stream before the next step's transfers: no host round
+ * trip.  On return the normalised v_m is the own slice of X[m % 2], v_{m-1} of X[(m-1) % 2], as for qbgpu_dist_lanczos.  On a
+ * breakdown (|b_m| < 2e-12 with stop_on_breakdown) the reference stops before it projects; here v_m handed back is the one
+ * after the projection of step m (when the projection ran), normalised.  hess is the same either way. */
+int qbgpu_dist_lanczos_val1(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, const void *phi0_local, int64_t np, int64_t maxit,
+                            int64_t *m, double *hess, int stop_on_breakdown);
+/* model<T>::locate_E0_lanczos(nev, ncv, maxit) of src/model.cc:1124-1316 on the shards; collective.  0 < nev <= 2,
+ * nev-1 <= ncv <= nev (else QBGPU_ERR_ARG).  eigenvals[nev] on every rank (E0, E1); phi_local: ncv vectors of this rank's rows
+ * one after the other (device, element type of D, in the shard's order: the internal order for species-order shards; may be
+ * NULL if ncv == 0); steps[4] / accuracies[4]: Lanczos E0, CG phi0, Lanczos E1, CG phi1 (0 for stages not run).  ref_row_dev
+ * as for qbgpu_dist_randomize (NULL for ordinary shards).  Overwrites X[0] and X[1]. */
+int qbgpu_dist_locate_e0_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, const int32_t *ref_row_dev,
+                                 int nev, int ncv, int64_t maxit, double *eigenvals, void *phi_local, int64_t *steps, double *accuracies);
 /* energy_scale of src/kpm.cc:45-88; Chebyshev moments of the own slices of X[0]; eigenvec_CG of src/lanczos.cc:281-341 */
 int qbgpu_dist_energy_scale(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, const int32_t *ref_row_dev, double *lo, double *hi,
                             double extend, int64_t iters);

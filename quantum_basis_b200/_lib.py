@@ -107,6 +107,8 @@ _SIGS = {
     "qbgpu_dist_energy_scale": [vp, vp, vp, vp, C.POINTER(dbl), C.POINTER(dbl), dbl, i64],
     "qbgpu_dist_kpm_moments": [vp, vp, vp, dbl, dbl, i64, vp],
     "qbgpu_dist_eigenvec_cg": [vp, vp, vp, i64, C.POINTER(i64), vp, C.POINTER(dbl), vp, vp, vp, vp],
+    "qbgpu_dist_lanczos_val1": [vp, vp, vp, vp, i64, i64, C.POINTER(i64), vp, C.c_int],
+    "qbgpu_dist_locate_e0_lanczos": [vp, vp, vp, vp, C.c_int, C.c_int, i64, vp, vp, vp, vp],
     "qbgpu_debug_rows_host": [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, dbl, dbl, dbl, i64, vp, vp, C.c_int, vp],
     "qbgpu_debug_species_parts_host": [C.c_int, C.c_int, C.c_int, C.c_int, vp, dbl, dbl, C.c_int, i64, i64, C.c_int, vp, vp, vp, vp],
     "qbgpu_debug_species_host": [C.c_int, C.c_int, C.c_int, C.c_int, vp, dbl, dbl, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],

@@ -16,15 +16,18 @@
 //     same stop-rule decision) that is also the barrier which makes the freshly written slices visible.  One 32-thread
 //     kernel, a few microseconds; no host involvement, no collective library.
 //
-// Loops: lanczos (reference src/lanczos.cc:134-266, purposes sr_val0 / dnmcs, with the stop rule of :228-248 evaluated on
-// every rank from the identical reduced (a, b)), eigenvec_CG (:281-341), energy_scale (src/kpm.cc:45-88), Chebyshev
-// moments, and the plain product.  The local arithmetic is the single-GPU kernels'; only the reductions differ (a sum of
-// per-rank sums), so E0 agrees with the single-GPU run to round-off of the reductions (~1e-15 relative).
+// Loops: lanczos (reference src/lanczos.cc:134-266, purposes sr_val0 / dnmcs / sr_val1, with the stop rule of :228-248
+// evaluated on every rank from the identical reduced (a, b); sr_val1 re-orthogonalises against phi0 on the device, see
+// dist_lanczos_loop), eigenvec_CG (:281-341), energy_scale (src/kpm.cc:45-88), Chebyshev moments, the plain product, and the
+// four stages of model<T>::locate_E0_lanczos (src/model.cc:1124-1316: E0, phi0, E1, phi1) in one call.  The local arithmetic
+// is the single-GPU kernels'; only the reductions differ (a sum of per-rank sums), so E0 agrees with the single-GPU run to
+// round-off of the reductions (~1e-15 relative).
 #include "internal.hpp"
 #include <cfloat>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <string>
 #include <vector>
 
 namespace qb {
@@ -326,6 +329,26 @@ __global__ void __launch_bounds__(256) dist_randomize_kernel(int64_t nloc, int64
     }
 }
 
+// x <- (x - <phi0, x> phi0) / |x - <phi0, x> phi0| over the shards (x, phi0: this rank's rows): the cblas dot, axpy, nrm2 and
+// scal of src/model.cc:1240-1252 and :1302-1311, each sum reduced across the ranks.  The caller passes a barrier before x is pulled.
+static int dist_orthonormalize(qbgpu_dist *D, const void *phi0, void *x)
+{
+    Context &c = ctx();
+    const int64_t nloc = D->nloc();
+    double *t = D->scal + 32;                               // [0], [1] = <phi0, x>, [2] = |x|^2
+    if (nloc) QB_TRY(vec_dotc(nloc, D->cplx, phi0, x, t)); else QB_CUDA(cudaMemsetAsync(t, 0, sizeof(double) * 2, c.stream));
+    QB_TRY(dist_allreduce(D, t, 2));
+    double h[2];
+    QB_TRY(read_scalars(t, h, 2));
+    if (nloc) QB_TRY(vec_axpy(nloc, D->cplx, make_double2(-h[0], D->cplx ? -h[1] : 0.0), phi0, x));
+    if (nloc) QB_TRY(vec_nrm2sq(nloc, D->cplx, x, t + 2)); else QB_CUDA(cudaMemsetAsync(t + 2, 0, sizeof(double), c.stream));
+    QB_TRY(dist_allreduce(D, t + 2, 1));
+    double nn;
+    QB_TRY(read_scalars(t + 2, &nn, 1));
+    if (nloc) QB_TRY(vec_scal(nloc, D->cplx, make_double2(1.0 / sqrt(nn), 0.0), x));
+    return QBGPU_OK;
+}
+
 }  // namespace qb
 
 using namespace qb;
@@ -525,20 +548,11 @@ int qbgpu_dist_mv(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest
     return QBGPU_OK;
 }
 
-/* lanczos(0, np, maxit, m, dim, H, v, hessenberg, purpose) of src/lanczos.cc:134-266 on the shards.  Start: the normalised
- * start vector's slice in the own part of X[0], visible to the peers (qbgpu_dist_randomize, or write it and call
- * qbgpu_dist_barrier).  purpose: "sr_val0" (stop rule of :228-248; every rank takes the same decision from the identical
- * reduced coefficients) or "dnmcs" (np steps unless b_m < 2e-12).  hess[2*maxit]: b in [0,maxit), a in [maxit, 2 maxit), on
- * every rank.  On return the normalised v_m is the own slice of X[m % 2], v_{m-1} of X[(m-1) % 2]. */
-int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, int64_t np, int64_t maxit, int64_t *m_out,
-                       double *hess, const char *purpose, int stop_on_breakdown)
+// the loop of qbgpu_dist_lanczos / qbgpu_dist_lanczos_val1; phi (this rank's rows of phi0, or null): sr_val1.  Without phi no
+// kernel of the re-orthogonalisation is launched.
+static int dist_lanczos_loop(qbgpu_dist *D, const qbgpu_matrix *local_part, const qbgpu_matrix *rest, int64_t np, int64_t maxit, int64_t *m_out,
+                             double *hess, bool is_val, const void *phi, int stop_on_breakdown)
 {
-    QB_TRY(ensure_init());
-    QB_TRY(dist_check(D, local_part, rest));
-    if (!m_out || !hess || !purpose) return fail(QBGPU_ERR_ARG, "dist_lanczos: null argument");
-    const bool is_val = strcmp(purpose, "sr_val0") == 0, is_dn = strcmp(purpose, "dnmcs") == 0;
-    if (!is_val && !is_dn) return fail(QBGPU_ERR_ARG, "dist_lanczos: purpose must be sr_val0 or dnmcs");
-    if (!(np >= 0 && np < maxit)) return fail(QBGPU_ERR_ARG, "dist_lanczos: need 0 <= np < maxit");
     *m_out = 0;
     for (int64_t j = 0; j < 2 * maxit; j++) hess[j] = 0.0;
     if (np == 0) return QBGPU_OK;
@@ -546,6 +560,7 @@ int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t
     const bool cplx = D->cplx;
     const int64_t nloc = D->nloc();
     double *state = D->scal;                                // 8 doubles (lanczos_step_*), then scratch
+    double *p1 = D->scal + 24;                              // sr_val1: the projection's 8 doubles (vecops.cu: lanczos_step_b_phi)
     double *ab_dev = nullptr;
     QB_CUDA(cudaMalloc(&ab_dev, sizeof(double) * 2 * maxit));
     double *b_dev = ab_dev, *a_dev = ab_dev + maxit;
@@ -574,8 +589,8 @@ int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t
     bool early_issued = false;                              // the early parts of the coming step are already in the stream
     // QBGPU_VERBOSE: device time of the phases of a step (events on the compute stream) and host time between the steps
     const bool prof = getenv("QBGPU_VERBOSE") != nullptr;
-    cudaEvent_t pe[6] = {};
-    double tph[5] = {0, 0, 0, 0, 0};
+    cudaEvent_t pe[7] = {};
+    double tph[6] = {0, 0, 0, 0, 0, 0};
     if (prof) for (auto &e : pe) cudaEventCreate(&e);
     auto rec = [&](int i) { if (prof) cudaEventRecord(pe[i], c.stream); };
     while (m < np) {
@@ -589,15 +604,33 @@ int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t
         rec(1);
         if (int rc = dist_allreduce(D, state + 3, 1)) return done2(rc);
         rec(2);
-        if (int rc = lanczos_step_b(nloc, cplx, D->own(bx), uz, state, w)) return done2(rc);
-        rec(3);
-        if (int rc = dist_allreduce(D, state + 6, 1)) return done2(rc);      // also the barrier that makes X[bz] final everywhere
-        rec(4);
-        if (int rc = lanczos_step_c(state, a_dev, b_dev, m)) return done2(rc);
+        if (!phi) {
+            if (int rc = lanczos_step_b(nloc, cplx, D->own(bx), uz, state, w)) return done2(rc);
+            rec(3);
+            if (int rc = dist_allreduce(D, state + 6, 1)) return done2(rc);      // also the barrier that makes X[bz] final everywhere
+            rec(4);
+            if (int rc = lanczos_step_c(state, a_dev, b_dev, m)) return done2(rc);
+        } else {                                            // step b with the partials |U|^2, <phi0, U>: one all-reduce of 3
+            if (int rc = lanczos_step_b_phi(nloc, cplx, D->own(bx), uz, phi, state, p1, w)) return done2(rc);
+            rec(3);
+            if (int rc = dist_allreduce(D, p1, 3)) return done2(rc);
+            rec(4);
+            if (int rc = lanczos_step_c_phi(state, p1, a_dev, b_dev, m)) return done2(rc);
+        }
         cudaMemcpyAsync(c.scal_host, a_dev + (m - 1), sizeof(double), cudaMemcpyDeviceToHost, c.stream);
         cudaMemcpyAsync(c.scal_host + 1, b_dev + m, sizeof(double), cudaMemcpyDeviceToHost, c.stream);
         if (ev_ab) cudaEventRecord(ev_ab, c.stream);
         rec(5);
+        if (phi) {
+            // re-orthogonalisation (src/lanczos.cc:218-226), decided by step c from the reduced sums -- bit-identical on every
+            // rank, so every rank takes the same branch: U -= h phi0 and the partial |U|^2 (a pass that does nothing when the
+            // flag is off), the all-reduce (unconditional: also the barrier that makes the projected X[bz] final everywhere),
+            // sx = 1/|U|.  All of it is in the stream before the next step's pulls and early parts below.
+            if (int rc = lanczos_project(nloc, cplx, phi, uz, p1)) return done2(rc);
+            if (int rc = dist_allreduce(D, p1 + 6, 1)) return done2(rc);
+            if (int rc = lanczos_project_finalize(state, p1)) return done2(rc);
+        }
+        rec(6);
         // the slices of the NEXT step's vector (unnormalised: its scale travels as a scalar) are final now: start fetching
         // them -- and, with the scratch vector, multiplying by the early parts -- before the host reads the coefficients back
         // and decides whether there is a next step (if not: harmless)
@@ -610,8 +643,8 @@ int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t
         hess[maxit + m - 1] = c.scal_host[0];
         hess[m] = c.scal_host[1];
         if (prof) {
-            cudaEventSynchronize(pe[5]);
-            for (int i = 0; i < 5; i++) { float f = 0; cudaEventElapsedTime(&f, pe[i], pe[i + 1]); tph[i] += f; }
+            cudaEventSynchronize(pe[6]);
+            for (int i = 0; i < 6; i++) { float f = 0; cudaEventElapsedTime(&f, pe[i], pe[i + 1]); tph[i] += f; }
         }
         if (m == 1) continue;
         if (stop_on_breakdown && fabs(hess[m]) < kLanczosPrecisionD) break;                        // src/lanczos.cc:216
@@ -631,8 +664,9 @@ int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t
     }
     *m_out = m;
     if (prof) {
-        if (D->rank == 0) fprintf(stderr, "[qbgpu dist_lanczos] %lld steps on %d ranks, device ms per step: product %.3f | all-reduce %.3f | update pass %.3f | all-reduce %.3f | scalars+readback %.3f\n",
-                                  (long long)m, D->world, tph[0] / m, tph[1] / m, tph[2] / m, tph[3] / m, tph[4] / m);
+        if (D->rank == 0) fprintf(stderr, "[qbgpu dist_lanczos%s] %lld steps on %d ranks, device ms per step: product %.3f | all-reduce %.3f | update pass %.3f | all-reduce %.3f | scalars+readback %.3f%s\n",
+                                  phi ? " sr_val1" : "", (long long)m, D->world, tph[0] / m, tph[1] / m, tph[2] / m, tph[3] / m, tph[4] / m,
+                                  phi ? (" | projection+all-reduce " + std::to_string(tph[5] / m)).c_str() : "");
         for (auto &e : pe) cudaEventDestroy(e);
     }
     if (int rc = dist_wait(D)) return done2(rc);             // (a fetch started for a step that did not happen)
@@ -644,6 +678,36 @@ int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t
     if (int rc = dist_allreduce(D, D->scal + 8, 0)) return done2(rc);
     return done2(dist_timed_out(D, "dist_lanczos"));
 }
+
+/* lanczos(0, np, maxit, m, dim, H, v, hessenberg, purpose) of src/lanczos.cc:134-266 on the shards.  Start: the normalised
+ * start vector's slice in the own part of X[0], visible to the peers (qbgpu_dist_randomize, or write it and call
+ * qbgpu_dist_barrier).  purpose: "sr_val0" (stop rule of :228-248; every rank takes the same decision from the identical
+ * reduced coefficients) or "dnmcs" (np steps unless b_m < 2e-12).  hess[2*maxit]: b in [0,maxit), a in [maxit, 2 maxit), on
+ * every rank.  On return the normalised v_m is the own slice of X[m % 2], v_{m-1} of X[(m-1) % 2]. */
+int qbgpu_dist_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, int64_t np, int64_t maxit, int64_t *m_out,
+                       double *hess, const char *purpose, int stop_on_breakdown)
+{
+    QB_TRY(ensure_init());
+    QB_TRY(dist_check(D, local_part, rest));
+    if (!m_out || !hess || !purpose) return fail(QBGPU_ERR_ARG, "dist_lanczos: null argument");
+    const bool is_val = strcmp(purpose, "sr_val0") == 0, is_dn = strcmp(purpose, "dnmcs") == 0;
+    if (!is_val && !is_dn) return fail(QBGPU_ERR_ARG, "dist_lanczos: purpose must be sr_val0 or dnmcs");
+    if (!(np >= 0 && np < maxit)) return fail(QBGPU_ERR_ARG, "dist_lanczos: need 0 <= np < maxit");
+    return dist_lanczos_loop(D, local_part, rest, np, maxit, m_out, hess, is_val, nullptr, stop_on_breakdown);
+}
+
+/* lanczos(0, np, maxit, ..., "sr_val1") of src/lanczos.cc:134-266 on the shards: the loop above (stop rule of sr_val0) with the
+ * re-orthogonalisation against phi0 of :218-226 in every step after the first, decided and applied on the device. */
+int qbgpu_dist_lanczos_val1(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, const void *phi0_local, int64_t np, int64_t maxit,
+                            int64_t *m_out, double *hess, int stop_on_breakdown)
+{
+    QB_TRY(ensure_init());
+    QB_TRY(dist_check(D, local_part, rest));
+    if (!m_out || !hess || !phi0_local) return fail(QBGPU_ERR_ARG, "dist_lanczos_val1: null argument (phi0_local, m or hess)");
+    if (!(np >= 0 && np < maxit)) return fail(QBGPU_ERR_ARG, "dist_lanczos_val1: need 0 <= np < maxit");
+    return dist_lanczos_loop(D, local_part, rest, np, maxit, m_out, hess, true, phi0_local, stop_on_breakdown);
+}
+
 
 /* energy_scale of src/kpm.cc:45-88 on the shards: iters-1 Lanczos steps from vec_randomize(seed 1), bounds widened by extend. */
 int qbgpu_dist_energy_scale(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, const int32_t *ref_row, double *lo, double *hi,
@@ -771,6 +835,77 @@ int qbgpu_dist_eigenvec_cg(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matr
     *m_io = m;
     *accu_out = accu;
     return dist_timed_out(D, "dist_eigenvec_cg");
+}
+
+
+/* model<T>::locate_E0_lanczos(nev, ncv, maxit) of src/model.cc:1124-1316 on the shards, stage by stage as csr.locate_E0_lanczos
+ * runs it on one GPU (same seeds, same order): E0 by sr_val0 Lanczos from vec_randomize(1); phi0 by eigenvec_CG from
+ * vec_randomize(1); E1 by sr_val1 Lanczos from vec_randomize(1) projected off phi0; phi1 by eigenvec_CG at E1 from
+ * vec_randomize(8), orthonormalised against phi0 when the gap is below 2e-12 (:1302-1311).  Uses X[0] and X[1]. */
+int qbgpu_dist_locate_e0_lanczos(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matrix_t rest, const int32_t *ref_row, int nev, int ncv,
+                                 int64_t maxit, double *eigenvals, void *phi_local, int64_t *steps, double *accuracies)
+{
+    QB_TRY(ensure_init());
+    QB_TRY(dist_check(D, local_part, rest));
+    if (!(nev > 0 && nev <= 2 && nev - 1 <= ncv && ncv <= nev))
+        return fail(QBGPU_ERR_ARG, "dist_locate_e0_lanczos: need 0 < nev <= 2 and nev-1 <= ncv <= nev (src/model.cc:1141)");
+    if (!eigenvals || !steps || !accuracies || (ncv > 0 && !phi_local)) return fail(QBGPU_ERR_ARG, "dist_locate_e0_lanczos: null argument (eigenvals, steps, accuracies, or phi_local with ncv > 0)");
+    if (maxit < 2) return fail(QBGPU_ERR_ARG, "dist_locate_e0_lanczos: need maxit >= 2");
+    for (int i = 0; i < 4; i++) { steps[i] = 0; accuracies[i] = 0.0; }
+    Context &c = ctx();
+    const int64_t nloc = D->nloc();
+    const size_t vb = D->esize * (size_t)nloc;
+    std::vector<double> hess(2 * maxit), ritz(maxit);
+    // the lowest Ritz value of a finished run and its residual estimate |b_m s_{m-1}|
+    auto lowest = [&](int64_t m, double *E, double *accu) -> int {
+        double s_last = 0.0;
+        if (hess_eigen_host(hess.data(), maxit, m, ritz.data(), nullptr, &s_last)) return fail(QBGPU_ERR_NUMERIC, "hess_eigen: QL did not converge");
+        *E = ritz[0];
+        *accu = fabs(hess[m] * s_last);
+        return QBGPU_OK;
+    };
+    // stage 1 (:1165-1196): E0
+    QB_TRY(qbgpu_dist_randomize(D, 0, 1, ref_row));
+    int64_t m = 0;
+    QB_TRY(dist_lanczos_loop(D, local_part, rest, maxit - 1, maxit, &m, hess.data(), true, nullptr, 1));
+    double E0 = 0.0;
+    QB_TRY(lowest(m, &E0, &accuracies[0]));
+    eigenvals[0] = E0;
+    steps[0] = m;
+    if (ncv == 0) return QBGPU_OK;
+    // stage 2 (:1205-1231): phi0 = eigenvec_CG(E0) from vec_randomize(1)
+    char *phi0 = (char *)phi_local, *phi1 = ncv == 2 ? phi0 + vb : nullptr;
+    DevBufGuard r, p, pp;                                   // CG work vectors, freed on every way out
+    QB_CUDA(r.alloc(vb)); QB_CUDA(p.alloc(vb)); QB_CUDA(pp.alloc(vb));
+    auto seeded = [&](void *dst, uint32_t seed) -> int {    // dst <- this rank's rows of vec_randomize(seed), via X[0]
+        QB_TRY(qbgpu_dist_randomize(D, 0, seed, ref_row));
+        if (nloc) QB_CUDA(cudaMemcpyAsync(dst, D->own(0), vb, cudaMemcpyDeviceToDevice, c.stream));
+        return QBGPU_OK;
+    };
+    QB_TRY(seeded(phi0, 1));
+    const double e0[2] = {E0, 0.0};
+    QB_TRY(qbgpu_dist_eigenvec_cg(D, local_part, rest, maxit, &steps[1], e0, &accuracies[1], phi0, r.p, p.p, pp.p));
+    double gap = 0.0;
+    if (nev == 2) {
+        // stage 3 (:1233-1265): E1 by Lanczos from vec_randomize(1) projected off phi0, re-orthogonalised in every step
+        QB_TRY(qbgpu_dist_randomize(D, 0, 1, ref_row));
+        QB_TRY(dist_orthonormalize(D, phi0, D->own(0)));
+        QB_TRY(dist_allreduce(D, D->scal + 8, 0));          // barrier: the start vector is final everywhere before the pulls
+        int64_t m1 = 0;
+        QB_TRY(dist_lanczos_loop(D, local_part, rest, maxit - 1, maxit, &m1, hess.data(), true, phi0, 1));
+        QB_TRY(lowest(m1, &eigenvals[1], &accuracies[2]));
+        steps[2] = m1;
+        gap = eigenvals[1] - E0;
+    }
+    if (ncv == 2) {
+        // stage 4 (:1275-1315): phi1 = eigenvec_CG(E1) from vec_randomize(8); a degenerate pair is orthonormalised
+        QB_TRY(seeded(phi1, 8));
+        const double e1[2] = {eigenvals[1], 0.0};
+        QB_TRY(qbgpu_dist_eigenvec_cg(D, local_part, rest, maxit, &steps[3], e1, &accuracies[3], phi1, r.p, p.p, pp.p));
+        if (gap < kLanczosPrecisionD) QB_TRY(dist_orthonormalize(D, phi0, phi1));
+    }
+    QB_TRY(dist_allreduce(D, D->scal + 8, 0));
+    return dist_timed_out(D, "dist_locate_e0_lanczos");
 }
 
 }  // extern "C"

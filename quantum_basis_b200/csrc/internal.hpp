@@ -168,6 +168,13 @@ int vec_take_real(int64_t n, const void *cplx_in, double *real_out);
 int vec_put_real(int64_t n, const double *real_in, void *cplx_out);
 int lanczos_step_b(int64_t nloc, bool cplx, const void *ux_local, void *uz_local, double *state, const void *w_in = nullptr);                    // w_in: uz = w_in - a*sx*ux (out of place)
 int lanczos_step_c(double *state, double *a_dev, double *b_dev, int64_t m);
+// sr_val1 step on device scalars (p1: 8 doubles, layout in vecops.cu): step b with the partial <phi0, U>, step c with the
+// projection decision, the projection pass with its partial |U|^2, and the new scale once that partial is reduced
+int lanczos_step_b_phi(int64_t nloc, bool cplx, const void *ux_local, void *uz_local, const void *phi_local, const double *state, double *p1,
+                       const void *w_in = nullptr);
+int lanczos_step_c_phi(double *state, double *p1, double *a_dev, double *b_dev, int64_t m);
+int lanczos_project(int64_t nloc, bool cplx, const void *phi_local, void *uz_local, double *p1);
+int lanczos_project_finalize(double *state, const double *p1);
 int cg_update_vr(int64_t n, bool cplx, const double *sc, void *v, void *r, const void *p, const void *pp);
 int cg_update_p(int64_t n, bool cplx, double *sc, const void *r, void *p);
 int scale_copy(int64_t n, bool cplx, const double *scale_dev, double scale_imm, const void *src, void *dst);

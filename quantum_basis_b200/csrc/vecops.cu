@@ -250,6 +250,111 @@ int lanczos_step_c(double *state, double *a_dev, double *b_dev, int64_t m)
     return QBGPU_OK;
 }
 
+// ------------------------------------------------------------------ Lanczos step re-orthogonalised against phi0 (sr_val1)
+// The reference's re-orthogonalisation (src/lanczos.cc:218-226: tmp = <phi0, v_m>; if |tmp| > 2e-12 { v_m -= tmp phi0;
+// v_m /= |v_m| }) on the unnormalised vector v_m = sx*U: U -= h phi0 with h = <phi0, U>, then sx = 1/|U|.  The decision is
+// taken on the device from the reduced sums, so a multi-GPU loop can order the projection before the next step's pulls
+// without a host round trip.  p1 (device, 8 doubles): [0] = |U|^2, [1], [2] = Re, Im <phi0, U> (partials, then reduced),
+// [3] = projection flag, [4], [5] = -h, [6] = |U - h phi0|^2, [7] spare.
+// step b with the phi0 dot: as lanczos_b_kernel, plus the partial <phi0, U> of the freshly written U, in the same pass
+template <typename VecT>
+__global__ void __launch_bounds__(kVBlock, 4) lanczos_b_phi_kernel(int64_t n, const VecT *__restrict__ ux, const VecT *win, VecT *uz,
+                                                                   const VecT *__restrict__ phi, const double *state, double *p1,
+                                                                   double *partials, unsigned *ticket)
+{
+    using VT = VecTraits<VecT>;
+    const double f = -state[3] * state[0];
+    double d[3] = {0.0, 0.0, 0.0};
+    // loads batched as in lanczos_b_kernel: 96 bytes per thread in flight (4 real or 2 complex elements of three operands;
+    // 4 complex ones spill at the 64 registers of 4 blocks per SM)
+    constexpr int B = sizeof(VecT) == 16 ? 2 : 4;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += B * stride) {
+        VecT w[B], v[B], q[B];
+#pragma unroll
+        for (int k = 0; k < B; k++) { const int64_t j = i + k * stride; if (j < n) { w[k] = win[j]; v[k] = ux[j]; q[k] = phi[j]; } }
+#pragma unroll
+        for (int k = 0; k < B; k++) {
+            const int64_t j = i + k * stride;
+            if (j < n) {
+                const VecT r = VT::add(w[k], VT::rscale(f, v[k]));
+                uz[j] = r;
+                d[0] += VT::abs2(r);
+                const double2 h = VT::conj_mul(q[k], r);
+                d[1] += h.x; d[2] += h.y;
+            }
+        }
+    }
+    block_reduce_finalize<3, kVBlock>(d, partials, ticket, p1);
+}
+// step c for sr_val1: lanczos_c_kernel on the reduced |U|^2 (b_m is recorded before the projection, as the reference records
+// it), then the decision |h sx| > 2e-12 with the new sx = 1/b_m.  No projection in the start-up step (m == 1): the reference's
+// first step has no checks (:167-191).
+__global__ void lanczos_c_phi_kernel(double *state, double *p1, double *a_dev, double *b_dev, int64_t m)
+{
+    const double b = sqrt(p1[0]);
+    a_dev[m - 1] = state[3];
+    b_dev[m] = b;
+    const double sx_old = state[0];
+    const double sx = 1.0 / b;
+    state[0] = sx;
+    state[1] = sx_old;
+    state[2] = b;
+    const double tr = p1[1] * sx, ti = p1[2] * sx;
+    p1[3] = (m > 1 && sqrt(tr * tr + ti * ti) > 2e-12) ? 1.0 : 0.0;
+    p1[4] = -p1[1];
+    p1[5] = -p1[2];
+}
+// projection pass: when the flag is set U += (-h) phi0 and p1[6] = partial |U|^2 (else 0; the vector is not touched)
+template <typename VecT>
+__global__ void __launch_bounds__(kVBlock, 4) lanczos_project_kernel(int64_t n, const VecT *__restrict__ phi, VecT *uz, double *p1,
+                                                                     double *partials, unsigned *ticket)
+{
+    using VT = VecTraits<VecT>;
+    double d[1] = {0.0};
+    if (p1[3] != 0.0) {
+        const double2 c = make_double2(p1[4], p1[5]);
+        GRID_STRIDE(i, n) { const VecT r = VT::add(uz[i], VT::scale(c, phi[i])); uz[i] = r; d[0] += VT::abs2(r); }
+    }
+    block_reduce_finalize<1, kVBlock>(d, partials, ticket, p1 + 6);
+}
+// after the all-reduce of p1[6]: the projected vector's scale
+__global__ void lanczos_project_finalize_kernel(double *state, const double *p1)
+{
+    if (p1[3] != 0.0) state[0] = 1.0 / sqrt(p1[6]);
+}
+
+int lanczos_step_b_phi(int64_t nloc, bool cplx, const void *ux_local, void *uz_local, const void *phi_local, const double *state, double *p1,
+                       const void *w_in)
+{
+    Context &c = ctx();
+    if (!w_in) w_in = uz_local;
+    if (cplx) LAUNCH_V(lanczos_b_phi_kernel<double2>, nloc, nloc, (const double2 *)ux_local, (const double2 *)w_in, (double2 *)uz_local, (const double2 *)phi_local, state, p1, c.partials, c.ticket);
+    else      LAUNCH_V(lanczos_b_phi_kernel<double>, nloc, nloc, (const double *)ux_local, (const double *)w_in, (double *)uz_local, (const double *)phi_local, state, p1, c.partials, c.ticket);
+    return QBGPU_OK;
+}
+int lanczos_step_c_phi(double *state, double *p1, double *a_dev, double *b_dev, int64_t m)
+{
+    lanczos_c_phi_kernel<<<1, 1, 0, ctx().stream>>>(state, p1, a_dev, b_dev, m);
+    QB_LAUNCH_COUNT();
+    QB_CUDA(cudaGetLastError());
+    return QBGPU_OK;
+}
+int lanczos_project(int64_t nloc, bool cplx, const void *phi_local, void *uz_local, double *p1)
+{
+    Context &c = ctx();
+    if (cplx) LAUNCH_V(lanczos_project_kernel<double2>, nloc, nloc, (const double2 *)phi_local, (double2 *)uz_local, p1, c.partials, c.ticket);
+    else      LAUNCH_V(lanczos_project_kernel<double>, nloc, nloc, (const double *)phi_local, (double *)uz_local, p1, c.partials, c.ticket);
+    return QBGPU_OK;
+}
+int lanczos_project_finalize(double *state, const double *p1)
+{
+    lanczos_project_finalize_kernel<<<1, 1, 0, ctx().stream>>>(state, p1);
+    QB_LAUNCH_COUNT();
+    QB_CUDA(cudaGetLastError());
+    return QBGPU_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ CG passes
 // sc (device): [0]=gamma (residual norm, `accu`) [1],[2]=delta=<p,pp> (re,im) [3]=|pp|^2 scratch [4]=|r|^2
 // pass 1 (src/lanczos.cc:324-327): alpha = gamma^2/delta ; v += alpha p ; r -= alpha pp ; sc[4] = |r|^2

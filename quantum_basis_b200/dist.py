@@ -638,6 +638,45 @@ class NativeDist:
                                                 C.c_void_p(v_ptr), C.c_void_p(r_ptr), C.c_void_p(p_ptr), C.c_void_p(pp_ptr)))
         return int(m.value), accu.value
 
+    def lanczos_val1(self, local, rest, phi0_ptr, np_, maxit, stop_on_breakdown=True):
+        """sr_val1 Lanczos (re-orthogonalised against phi0 in every step) from the normalised start vector in the own slice of
+        X[0], orthogonal to phi0; phi0_ptr: this rank's rows of phi0 (device).  Returns (m, hess) like lanczos()."""
+        hess = np.zeros(2 * maxit)
+        m = C.c_int64(0)
+        self._chk(self.L.qbgpu_dist_lanczos_val1(self.h, self._hp(local), rest.handle, C.c_void_p(phi0_ptr), np_, maxit, C.byref(m),
+                                                 C.c_void_p(hess.ctypes.data), int(stop_on_breakdown)))
+        return int(m.value), hess
+
+    def locate_E0_lanczos(self, local, rest, nev=1, ncv=1, maxit=1000, ref_rows_ptr=None):
+        """model<T>::locate_E0_lanczos (src/model.cc:1124-1316) on the shards: the keys of csr.locate_E0_lanczos, with the
+        eigenvectors as this rank's rows in the shard's order (the internal order for species-order shards)."""
+        import torch
+        if not (0 < nev <= 2 and nev - 1 <= ncv <= nev):
+            raise ValueError("need 0 < nev <= 2 and nev-1 <= ncv <= nev")          # the reference's assert, :1141
+        w = np.zeros(2)
+        steps = np.zeros(4, dtype=np.int64)
+        accu = np.zeros(4)
+        comps = 2 if self.complex else 1
+        phi = torch.zeros(max(ncv * self.nloc * comps, 1), dtype=torch.float64, device="cuda") if ncv > 0 else None
+        self._chk(self.L.qbgpu_dist_locate_e0_lanczos(self.h, self._hp(local), rest.handle, C.c_void_p(ref_rows_ptr) if ref_rows_ptr else None,
+                                                      nev, ncv, maxit, C.c_void_p(w.ctypes.data), C.c_void_p(phi.data_ptr()) if phi is not None else None,
+                                                      C.c_void_p(steps.ctypes.data), C.c_void_p(accu.ctypes.data)))
+        out = {"eigenvals": [float(w[0])], "eigenvecs": [], "lanczos_steps": int(steps[0]), "lanczos_accuracy": float(accu[0])}
+        if ncv == 0:
+            return out
+        out["cg_steps"], out["cg_accuracy"] = int(steps[1]), float(accu[1])
+        vecs = phi.cpu().numpy()[:ncv * self.nloc * comps]
+        vecs = (vecs.view(np.complex128) if self.complex else vecs).reshape(ncv, self.nloc)
+        if nev == 2:
+            out["eigenvals"].append(float(w[1]))
+            out["gap"] = float(w[1] - w[0])
+            out["lanczos_steps_E1"] = int(steps[2])
+        out["eigenvecs"].append(vecs[0].copy())
+        if ncv == 2:
+            out["cg_steps_E1"], out["cg_accuracy_E1"] = int(steps[3]), float(accu[3])
+            out["eigenvecs"].append(vecs[1].copy())
+        return out
+
     def destroy(self):
         if self.h:
             self.L.qbgpu_dist_destroy(self.h)
