@@ -379,13 +379,18 @@ int qbgpu_debug_species_packed_host(int nsites, int nup, int ndn, int nbonds, co
 /* --------------------------------------------------------------------- translation-symmetric sectors
  * Device counterpart of model::fill_Weisse_table + enumerate_basis_repr + generate_Ham_sparse_repr
  * (src/model.cc:205-249, 275-487, 688-836) for spin-1/2 models on untilted lattices with one site per unit cell and
- * periodic boundaries in every direction (chain, square, triangular; at most 32 sites, at least one even direction):
+ * periodic boundaries in every direction (chain, square, triangular; at most 36 sites, at least one even direction):
  * the representatives, their order (Lin order when the reference's Lin tables exist, bisection order otherwise),
  * the norms and every matrix element are those of the reference bit for bit (tests/repr_builders.py restates the
  * convention and is pinned against 39 sectors assembled by the compiled reference).  BASELINE configs 2 and 5.
  *   L[dim]: lattice extents; k[dim]: momentum integers as passed to enumerate_basis_repr; ndown: number of down spins
  *   (digit 1), Sz_total = nsites/2 - ndown.  Sites are numbered like the reference's lattice class: first even
- *   direction fastest (src/lattice.cc:591-615). */
+ *   direction fastest (src/lattice.cc:591-615).
+ * Up to 32 sites a state is a 32-bit word; 34- and 36-site sectors keep 64-bit states and keys (qbgpu_sector_states64).
+ * Device memory of a sector with n representatives: 8 n (norms) + 4 n (keys; 8 n at 34 and 36 sites) + the segment table
+ * (256 KB up to 32 sites, at most 4 bytes per representative beyond) + the sublattice tables (2 MB at 32 sites, 19 MB at 36).
+ * The (Sz = 0, k) sectors of 36 sites hold about 2.5e8 representatives: 2 GB of keys, 2 GB of norms and 4 GB per complex
+ * vector, so they run through qbgpu_sector_matfree_heisenberg. */
 typedef struct qbgpu_sector *qbgpu_sector_t;
 typedef struct {
     int64_t dim;                 /* number of representatives, including those of zero norm */
@@ -393,11 +398,14 @@ typedef struct {
     int     nsites;
     int     lin_order;           /* 1: Lin-table order (odd-site label, even-site label); 0: integer order */
     double  enumerate_seconds, norms_seconds;
+    double  lin_check_seconds;   /* host part of enumerate_seconds: the Lin-table existence check over the keys */
+    int     state_bits;          /* 32, or 64 for sectors whose states need qbgpu_sector_states64 */
 } qbgpu_sector_info;
 int qbgpu_sector_create(qbgpu_sector_t *S, int dim, const int32_t *L, int ndown, const int32_t *k);
 int qbgpu_sector_destroy(qbgpu_sector_t S);
 int qbgpu_sector_get_info(qbgpu_sector_t S, qbgpu_sector_info *info);
-int qbgpu_sector_states(qbgpu_sector_t S, uint32_t *states_host);      /* bit s set = site s down, row order */
+int qbgpu_sector_states(qbgpu_sector_t S, uint32_t *states_host);      /* bit s set = site s down, row order; QBGPU_ERR_STATE when state_bits = 64 */
+int qbgpu_sector_states64(qbgpu_sector_t S, uint64_t *states_host);    /* the same as 64-bit words, for every sector */
 int qbgpu_sector_norms(qbgpu_sector_t S, double *nu_host);
 /* H = J sum_bonds S_i.S_j in that sector (bonds[2*nbonds] site pairs, duplicates are separate terms like repeated
  * add_Ham calls); fake_pos is model's constructor argument (default 100, src/qbasis.h:1337). */
@@ -536,6 +544,9 @@ int qbgpu_dist_eigenvec_cg(qbgpu_dist_t D, qbgpu_matrix_t local_part, qbgpu_matr
 /* pass 1 of the matrix-free species-order product: id = 1000 + v, v = 0 grid-stride rows (default), 1 contiguous row ranges
  * with one 1024-thread CTA per SM, 2 block x[iu, :] staged in shared memory.  Any other id: QBGPU_ERR_ARG. */
 int qbgpu_debug_set_variant(int id);
+/* word width of the spin sectors created afterwards: 0 by size (32-bit states up to 32 sites, the default), 64 the 64-bit
+ * path for every spin sector (to compare both widths on one sector).  Any other value: QBGPU_ERR_ARG. */
+int qbgpu_debug_sector_words(int bits);
 /* Rows of a full-basis Heisenberg (kind 0, n0 = down spins) or Hubbard (kind 1, n0/n1 = N_up/N_dn) operator recomputed on the
  * HOST in long double from the Lin tables (reference src/basis.cc:1144-1190) and the generators' own row function: the
  * size-independent parity check of bench.py on the BASELINE-size matrices.  rows: indices in the reference's order; x_host: the

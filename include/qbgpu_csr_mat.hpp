@@ -165,7 +165,9 @@ public:
     sector &operator=(const sector &) = delete;
     ~sector() { if (handle) qbgpu_sector_destroy(handle); }
     int64_t dim() const { return info.dim; }
+    // 32-bit bit patterns (QBGPU_ERR_STATE for the 34- and 36-site sectors, info.state_bits == 64: use states64())
     std::vector<uint32_t> states() const { std::vector<uint32_t> s(info.dim); check(qbgpu_sector_states(handle, s.data()), "qbgpu_sector_states"); return s; }
+    std::vector<uint64_t> states64() const { std::vector<uint64_t> s(info.dim); check(qbgpu_sector_states64(handle, s.data()), "qbgpu_sector_states64"); return s; }
     std::vector<double> norms() const { std::vector<double> s(info.dim); check(qbgpu_sector_norms(handle, s.data()), "qbgpu_sector_norms"); return s; }
     // H = J sum_bonds S_i.S_j (bonds = {i0, j0, i1, j1, ...}); fake_pos as in model's constructor (qbasis.h:1337)
     csr_mat<std::complex<double>> heisenberg(const std::vector<int32_t> &bonds, double J = 1.0, double fake_pos = 100.0, int flags = 0) const

@@ -18,7 +18,7 @@ class QbgpuError(RuntimeError):
 
 class SectorInfo(C.Structure):
     _fields_ = [("dim", C.c_int64), ("zero_norm", C.c_int64), ("nsites", C.c_int), ("lin_order", C.c_int),
-                ("enumerate_seconds", C.c_double), ("norms_seconds", C.c_double)]
+                ("enumerate_seconds", C.c_double), ("norms_seconds", C.c_double), ("lin_check_seconds", C.c_double), ("state_bits", C.c_int)]
 
 
 class MatrixInfo(C.Structure):
@@ -83,7 +83,8 @@ _SIGS = {
     "qbgpu_create_matfree_heisenberg": [C.POINTER(vp), C.c_int, C.c_int, C.c_int, vp, dbl, C.c_int, C.c_int, i64, i64],
     "qbgpu_create_matfree_hubbard": [C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_int, vp, dbl, dbl, C.c_int, C.c_int, i64, i64],
     "qbgpu_sector_create": [C.POINTER(vp), C.c_int, vp, C.c_int, vp], "qbgpu_sector_destroy": [vp],
-    "qbgpu_sector_get_info": [vp, C.POINTER(SectorInfo)], "qbgpu_sector_states": [vp, vp], "qbgpu_sector_norms": [vp, vp],
+    "qbgpu_sector_get_info": [vp, C.POINTER(SectorInfo)], "qbgpu_sector_states": [vp, vp], "qbgpu_sector_states64": [vp, vp],
+    "qbgpu_sector_norms": [vp, vp], "qbgpu_debug_sector_words": [C.c_int],
     "qbgpu_sector_build_heisenberg": [vp, C.POINTER(vp), C.c_int, vp, dbl, dbl, C.c_int],
     "qbgpu_sector_matfree_heisenberg": [vp, C.POINTER(vp), C.c_int, vp, dbl, dbl],
     "qbgpu_sector_create_electron": [C.POINTER(vp), C.c_int, vp, C.c_int, C.c_int, vp],

@@ -344,11 +344,21 @@ class Sector:
         check(lib().qbgpu_sector_get_info(self._h, C.byref(info)))
         self.dim, self.zero_norm, self.nsites, self.lin_order = info.dim, info.zero_norm, info.nsites, bool(info.lin_order)
         self.enumerate_seconds, self.norms_seconds = info.enumerate_seconds, info.norms_seconds
+        self.lin_check_seconds, self.state_bits = info.lin_check_seconds, info.state_bits
 
     def states(self):
-        """Bit patterns of the representatives in row order (bit s set = site s down)."""
+        """Bit patterns of the representatives in row order (bit s set = site s down): uint32, or uint64 for the
+        34- and 36-site sectors whose states take 64 bits (`state_bits`)."""
+        if self.state_bits == 64:
+            return self.states64()
         out = np.empty(self.dim, dtype=np.uint32)
         check(lib().qbgpu_sector_states(self._h, C.c_void_p(out.ctypes.data)))
+        return out
+
+    def states64(self):
+        """The same bit patterns as uint64, for every sector."""
+        out = np.empty(self.dim, dtype=np.uint64)
+        check(lib().qbgpu_sector_states64(self._h, C.c_void_p(out.ctypes.data)))
         return out
 
     def norms(self):
@@ -426,6 +436,7 @@ class ElectronSector(Sector):
         check(lib().qbgpu_sector_get_info(self._h, C.byref(info)))
         self.dim, self.zero_norm, self.nsites, self.lin_order = info.dim, info.zero_norm, info.nsites, bool(info.lin_order)
         self.enumerate_seconds, self.norms_seconds = info.enumerate_seconds, info.norms_seconds
+        self.lin_check_seconds, self.state_bits = info.lin_check_seconds, info.state_bits
 
     def hubbard(self, hops, t=1.0, U=1.1, fake_pos=100.0, flags=0):
         """hops: directed (to, from, spin) triples in the order of the caller's add_Ham calls."""

@@ -43,16 +43,24 @@
 namespace qb {
 
 constexpr int kSBlock = 128;
-constexpr int kMaxTrans = 32;          // one site per cell, at most 32 sites
+constexpr int kMaxTrans = 36;          // one site per cell, at most 36 sites
 constexpr int kMaxTerms = 128;         // bond terms per Hamiltonian
 
-struct SecDev {                        // passed to kernels by value
+// Word widths of a sector.  Spin sectors of at most 32 sites keep half states in 16 bits and parent states / keys in 32;
+// the 34- and 36-site spin sectors take 32-bit halves (at most 18 bits used) and 64-bit parent states and keys.  Both
+// instantiations run the same code: what a product computes does not depend on the width.  Electron sectors are narrow.
+struct Narrow { using H = uint16_t; using P = uint32_t; };
+struct Wide   { using H = uint32_t; using P = uint64_t; };
+
+template <class W> struct SecDevT {    // passed to kernels by value
+    using H = typename W::H;
+    using P = typename W::P;
     int nsites, nsub, ntrans, shift, lin_order;
     int64_t n;
-    const uint16_t *subT;              // [nsubtrans << nsub]  subT[(j << nsub) + x] = S_j x
-    const uint16_t *rep;               // [1 << nsub]
+    const H *subT;                     // [nsubtrans << nsub]  subT[(j << nsub) + x] = S_j x
+    const H *rep;                      // [1 << nsub]
     const uint8_t  *dist;              // [1 << nsub]
-    const uint32_t *keys;              // [n] ascending; Lin key (b << nsub | a) or the zipped bit pattern
+    const P *keys;                     // [n] ascending; Lin key (b << nsub | a) or the zipped bit pattern
     const uint32_t *seg;               // [(1 << (2 nsub - shift)) + 1] first index with key >> shift >= h
     const double   *nu;                // [n]
     uint8_t fwd_swap[kMaxTrans], fwd_ja[kMaxTrans], fwd_jb[kMaxTrans];   // T_i (a,b)
@@ -63,6 +71,8 @@ struct SecDev {                        // passed to kernels by value
     int16_t kt[kMaxTrans];             // k.t in units of 1/N
     const uint16_t *invmask;           // [ntrans][16]  invmask[i*16 + s1] = sites s2 > s1 that translation i moves in front of s1
 };
+using SecDev = SecDevT<Narrow>;
+using SecDev64 = SecDevT<Wide>;
 
 __host__ __device__ __forceinline__ uint32_t spread_bits(uint32_t x)
 {
@@ -80,6 +90,26 @@ __host__ __device__ __forceinline__ uint32_t squeeze_bits(uint32_t x)
     x = (x | (x >> 2)) & 0x0F0F0F0Fu;
     x = (x | (x >> 4)) & 0x00FF00FFu;
     x = (x | (x >> 8)) & 0x0000FFFFu;
+    return x;
+}
+__host__ __device__ __forceinline__ uint64_t spread_bits(uint64_t x)
+{
+    x &= 0xFFFFFFFFull;
+    x = (x | (x << 16)) & 0x0000FFFF0000FFFFull;
+    x = (x | (x << 8)) & 0x00FF00FF00FF00FFull;
+    x = (x | (x << 4)) & 0x0F0F0F0F0F0F0F0Full;
+    x = (x | (x << 2)) & 0x3333333333333333ull;
+    x = (x | (x << 1)) & 0x5555555555555555ull;
+    return x;
+}
+__host__ __device__ __forceinline__ uint64_t squeeze_bits(uint64_t x)
+{
+    x &= 0x5555555555555555ull;
+    x = (x | (x >> 1)) & 0x3333333333333333ull;
+    x = (x | (x >> 2)) & 0x0F0F0F0F0F0F0F0Full;
+    x = (x | (x >> 4)) & 0x00FF00FF00FF00FFull;
+    x = (x | (x >> 8)) & 0x0000FFFF0000FFFFull;
+    x = (x | (x >> 16)) & 0x00000000FFFFFFFFull;
     return x;
 }
 
@@ -100,22 +130,27 @@ __host__ __device__ __forceinline__ uint32_t squeeze_digits(uint32_t x)
     x = (x | (x >> 8)) & 0x0000FFFFu;
     return x;
 }
-template <class SD> __device__ __forceinline__ uint32_t sec_zip(const SD &S, uint32_t a, uint32_t b)
-{ return S.electron ? (spread_digits(a) | (spread_digits(b) << 2)) : (spread_bits(a) | (spread_bits(b) << 1)); }
-template <class SD> __device__ __forceinline__ void sec_unzip(const SD &S, uint32_t st, uint32_t &a, uint32_t &b)
+// spin parent state of the halves (a even sites, b odd sites)
+template <class P> __device__ __forceinline__ P spin_zip(uint32_t a, uint32_t b) { return spread_bits((P)a) | (spread_bits((P)b) << 1); }
+template <class W> __device__ __forceinline__ typename W::P sec_zip(const SecDevT<W> &S, uint32_t a, uint32_t b)
 {
-    if (S.electron) { a = squeeze_digits(st); b = squeeze_digits(st >> 2); }
-    else { a = squeeze_bits(st); b = squeeze_bits(st >> 1); }
+    using P = typename W::P;
+    return S.electron ? (P)(spread_digits(a) | (spread_digits(b) << 2)) : spin_zip<P>(a, b);
+}
+template <class W> __device__ __forceinline__ void sec_unzip(const SecDevT<W> &S, typename W::P st, uint32_t &a, uint32_t &b)
+{
+    if (S.electron) { a = squeeze_digits((uint32_t)st); b = squeeze_digits((uint32_t)st >> 2); }
+    else { a = (uint32_t)squeeze_bits(st); b = (uint32_t)squeeze_bits(st >> 1); }
 }
 
-__device__ __forceinline__ void sec_move(const SecDev &S, int swap, int ja, int jb, uint32_t a, uint32_t b, uint32_t &ao, uint32_t &bo)
+template <class W> __device__ __forceinline__ void sec_move(const SecDevT<W> &S, int swap, int ja, int jb, uint32_t a, uint32_t b, uint32_t &ao, uint32_t &bo)
 {
-    const uint16_t *Ta = S.subT + ((size_t)ja << S.nsub), *Tb = S.subT + ((size_t)jb << S.nsub);
+    const typename W::H *Ta = S.subT + ((size_t)ja << S.nsub), *Tb = S.subT + ((size_t)jb << S.nsub);
     if (swap) { ao = Ta[b]; bo = Tb[a]; } else { ao = Ta[a]; bo = Tb[b]; }
 }
 
 // (a, b) -> representative halves (ca, cb) and the smallest displacement i with state = T_i (ca zip cb)
-__device__ __forceinline__ int sec_canon(const SecDev &S, uint32_t a, uint32_t b, uint32_t &ca, uint32_t &cb)
+template <class W> __device__ __forceinline__ int sec_canon(const SecDevT<W> &S, uint32_t a, uint32_t b, uint32_t &ca, uint32_t &cb)
 {
     const uint32_t rs = min((uint32_t)S.rep[a], (uint32_t)S.rep[b]);
     int best = 0x7fffffff, bi = -1;
@@ -123,36 +158,42 @@ __device__ __forceinline__ int sec_canon(const SecDev &S, uint32_t a, uint32_t b
         uint32_t ai, bb;
         sec_move(S, S.inv_swap[i], S.inv_ja[i], S.inv_jb[i], a, b, ai, bb);
         if (ai != rs) continue;
-        const int key = (int)S.dist[bb] * kMaxTrans + i;
+        const int key = (int)S.dist[bb] * (int)(8 * sizeof(typename W::P)) + i;     // (dist, i) in lexicographic order: i < 32 or 64
         if (key < best) { best = key; bi = i; ca = ai; cb = bb; }
     }
     return bi;
 }
 
-__device__ __forceinline__ uint32_t sec_key(const SecDev &S, uint32_t a, uint32_t b)
+template <class W> __device__ __forceinline__ typename W::P sec_key(const SecDevT<W> &S, uint32_t a, uint32_t b)
 {
-    return S.lin_order ? ((b << S.nsub) | a) : sec_zip(S, a, b);
+    using P = typename W::P;
+    return S.lin_order ? (((P)b << S.nsub) | a) : sec_zip(S, a, b);
 }
-__device__ __forceinline__ void sec_halves(const SecDev &S, uint32_t key, uint32_t &a, uint32_t &b)
+template <class W> __device__ __forceinline__ void sec_halves(const SecDevT<W> &S, typename W::P key, uint32_t &a, uint32_t &b)
 {
-    if (S.lin_order) { a = key & ((1u << S.nsub) - 1u); b = key >> S.nsub; }
+    using P = typename W::P;
+    if (S.lin_order) { a = (uint32_t)(key & (((P)1 << S.nsub) - 1u)); b = (uint32_t)(key >> S.nsub); }
     else sec_unzip(S, key, a, b);
 }
-__device__ __forceinline__ int64_t sec_lookup(const SecDev &S, uint32_t key)
+template <class W> __device__ __forceinline__ int64_t sec_lookup(const SecDevT<W> &S, typename W::P key)
 {
-    const uint32_t h = key >> S.shift;
+    using P = typename W::P;
+    const uint32_t h = (uint32_t)(key >> S.shift);
     uint32_t lo = S.seg[h], hi = S.seg[h + 1];
-    while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; const uint32_t v = S.keys[mid]; if (v < key) lo = mid + 1; else hi = mid; }
+    while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; const P v = S.keys[mid]; if (v < key) lo = mid + 1; else hi = mid; }
     return (lo < S.seg[h + 1] && S.keys[lo] == key) ? (int64_t)lo : -1;
 }
 
 // ------------------------------------------------------------------------------------------ enumeration
-// candidate c = bIdx * nreps + r  <->  (a = reps[r], b = bIdx); ascending c is Lin order
-__global__ void __launch_bounds__(kSBlock) sec_flag_kernel(SecDev S, const uint16_t *__restrict__ reps, int nreps, int ndown, int64_t ncand,
-                                                           uint8_t *flag)
+// candidate c = bIdx * nreps + r  <->  (a = reps[r], b = bIdx); ascending c is Lin order.  A launch flags the candidates
+// [c0, c0 + ncand) into flag[0, ncand).
+template <class W>
+__global__ void __launch_bounds__(kSBlock) sec_flag_kernel(SecDevT<W> S, const typename W::H *__restrict__ reps, int nreps, int ndown, int64_t c0,
+                                                           int64_t ncand, uint8_t *flag)
 {
     for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < ncand; c += (int64_t)gridDim.x * blockDim.x) {
-        const uint32_t b = (uint32_t)(c / nreps), a = reps[c % nreps];
+        const int64_t cg = c0 + c;
+        const uint32_t b = (uint32_t)(cg / nreps), a = reps[cg % nreps];
         uint8_t ok = 0;
         if (__popc(a) + __popc(b) == ndown && a <= S.rep[b]) {
             ok = 1;
@@ -167,23 +208,29 @@ __global__ void __launch_bounds__(kSBlock) sec_flag_kernel(SecDev S, const uint1
     }
 }
 
-__global__ void __launch_bounds__(kSBlock) sec_cand_to_key_kernel(int64_t n, const uint16_t *__restrict__ reps, int nreps, int nsub, uint32_t *keys)
+// keys[i] holds a selected candidate index relative to the first candidate of the odd half b0
+template <class W>
+__global__ void __launch_bounds__(kSBlock) sec_cand_to_key_kernel(int64_t n, const typename W::H *__restrict__ reps, int nreps, int nsub, int64_t b0,
+                                                                  typename W::P *keys)
 {
+    using P = typename W::P;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        const uint32_t c = keys[i];
-        keys[i] = ((c / nreps) << nsub) | reps[c % nreps];
+        const uint32_t c = (uint32_t)keys[i];
+        keys[i] = ((P)(b0 + c / nreps) << nsub) | reps[c % nreps];
     }
 }
 
-__global__ void __launch_bounds__(kSBlock) sec_lin_to_zip_kernel(int64_t n, int nsub, uint32_t *keys)
+template <class P>
+__global__ void __launch_bounds__(kSBlock) sec_lin_to_zip_kernel(int64_t n, int nsub, P *keys)
 {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        const uint32_t k = keys[i];
-        keys[i] = spread_bits(k & ((1u << nsub) - 1u)) | (spread_bits(k >> nsub) << 1);
+        const P k = keys[i];
+        keys[i] = spin_zip<P>((uint32_t)(k & (((P)1 << nsub) - 1u)), (uint32_t)(k >> nsub));
     }
 }
 
-__global__ void __launch_bounds__(kSBlock) sec_seg_kernel(int64_t n, const uint32_t *__restrict__ keys, int shift, uint32_t nseg, uint32_t *seg)
+template <class P>
+__global__ void __launch_bounds__(kSBlock) sec_seg_kernel(int64_t n, const P *__restrict__ keys, int shift, uint32_t nseg, uint32_t *seg)
 {
     for (uint32_t h = blockIdx.x * blockDim.x + threadIdx.x; h <= nseg; h += gridDim.x * blockDim.x) {
         const uint64_t target = (uint64_t)h << shift;
@@ -193,7 +240,8 @@ __global__ void __launch_bounds__(kSBlock) sec_seg_kernel(int64_t n, const uint3
     }
 }
 
-__global__ void __launch_bounds__(kSBlock) sec_norm_kernel(SecDev S, double *nu, unsigned long long *zero_count)
+template <class W>
+__global__ void __launch_bounds__(kSBlock) sec_norm_kernel(SecDevT<W> S, double *nu, unsigned long long *zero_count)
 {
     for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < S.n; r += (int64_t)gridDim.x * blockDim.x) {
         uint32_t a, b;
@@ -210,7 +258,8 @@ __global__ void __launch_bounds__(kSBlock) sec_norm_kernel(SecDev S, double *nu,
     }
 }
 
-__global__ void __launch_bounds__(kSBlock) sec_states_kernel(SecDev S, uint32_t *out)
+template <class W>
+__global__ void __launch_bounds__(kSBlock) sec_states_kernel(SecDevT<W> S, typename W::P *out)
 {
     for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < S.n; r += (int64_t)gridDim.x * blockDim.x) {
         uint32_t a, b;
@@ -235,12 +284,13 @@ __device__ __forceinline__ int el_trans_sign(const SecDev &S, uint32_t st, int i
     return sg & 1;
 }
 
-__global__ void __launch_bounds__(kSBlock) el_flag_kernel(SecDev S, const uint16_t *__restrict__ reps, int nreps, int nup, int ndn, int64_t ncand,
-                                                          uint8_t *flag)
+__global__ void __launch_bounds__(kSBlock) el_flag_kernel(SecDev S, const uint16_t *__restrict__ reps, int nreps, int nup, int ndn, int64_t c0,
+                                                          int64_t ncand, uint8_t *flag)
 {
     const uint32_t MU = 0x5555u;
     for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < ncand; c += (int64_t)gridDim.x * blockDim.x) {
-        const uint32_t b = (uint32_t)(c / nreps), a = reps[c % nreps];
+        const int64_t cg = c0 + c;
+        const uint32_t b = (uint32_t)(cg / nreps), a = reps[cg % nreps];
         uint8_t ok = 0;
         if (__popc(a & MU) + __popc(b & MU) == nup && __popc((a >> 1) & MU) + __popc((b >> 1) & MU) == ndn && a <= S.rep[b]) {
             ok = 1;
@@ -394,7 +444,8 @@ struct SecTerms {
 };
 
 // upper bound of the stored row length: the diagonal plus one entry per antiparallel bond
-__global__ void __launch_bounds__(kSBlock) sec_cap_kernel(SecDev S, const SecTerms *Tp, int64_t *cap)
+template <class W>
+__global__ void __launch_bounds__(kSBlock) sec_cap_kernel(SecDevT<W> S, const SecTerms *Tp, int64_t *cap)
 {
     __shared__ SecTerms T;
     for (int i = threadIdx.x; i < (int)(sizeof(SecTerms) / 4); i += blockDim.x) ((int *)&T)[i] = ((const int *)Tp)[i];
@@ -406,15 +457,16 @@ __global__ void __launch_bounds__(kSBlock) sec_cap_kernel(SecDev S, const SecTer
             if (S.nu[r] != 0.0) {
                 uint32_t a, b;
                 sec_halves(S, S.keys[r], a, b);
-                const uint32_t s = spread_bits(a) | (spread_bits(b) << 1);
-                for (int t = 0; t < T.nterms; t++) c += (((s >> T.p[t]) ^ (s >> T.q[t])) & 1u);
+                const typename W::P s = spin_zip<typename W::P>(a, b);
+                for (int t = 0; t < T.nterms; t++) c += (int)(((s >> T.p[t]) ^ (s >> T.q[t])) & 1u);
             }
         }
         cap[r] = c;
     }
 }
 
-__global__ void __launch_bounds__(kSBlock) sec_rows_kernel(SecDev S, const SecTerms *Tp, const double2 *__restrict__ phase,
+template <class W>
+__global__ void __launch_bounds__(kSBlock) sec_rows_kernel(SecDevT<W> S, const SecTerms *Tp, const double2 *__restrict__ phase,
                                                            const int64_t *__restrict__ start, int64_t *row_end, int64_t *ocol, double2 *oval)
 {
     __shared__ SecTerms T;
@@ -429,9 +481,10 @@ __global__ void __launch_bounds__(kSBlock) sec_rows_kernel(SecDev S, const SecTe
             row_end[r] = start[r] + 1;
             continue;
         }
+        using P = typename W::P;
         uint32_t a, b;
         sec_halves(S, S.keys[r], a, b);
-        const uint32_t s = spread_bits(a) | (spread_bits(b) << 1);
+        const P s = spin_zip<P>(a, b);
         double dg = 0.0;
         for (int t = 0; t < T.nterms; t++)
             dg = __dadd_rn(dg, (((s >> T.p[t]) ^ (s >> T.q[t])) & 1u) ? -0.25 * T.J : 0.25 * T.J);
@@ -439,9 +492,9 @@ __global__ void __launch_bounds__(kSBlock) sec_rows_kernel(SecDev S, const SecTe
         col[0] = r; val[0] = make_double2(dg, 0.0);
         for (int t = 0; t < T.nterms; t++) {
             if (!(((s >> T.p[t]) ^ (s >> T.q[t])) & 1u)) continue;
-            const uint32_t s2 = s ^ ((1u << T.p[t]) | (1u << T.q[t]));
+            const P s2 = s ^ (((P)1 << T.p[t]) | ((P)1 << T.q[t]));
             uint32_t ca = 0, cb = 0;
-            const int i = sec_canon(S, squeeze_bits(s2), squeeze_bits(s2 >> 1), ca, cb);
+            const int i = sec_canon(S, (uint32_t)squeeze_bits(s2), (uint32_t)squeeze_bits(s2 >> 1), ca, cb);
             if (i < 0) continue;
             const int64_t j = sec_lookup(S, sec_key(S, ca, cb));
             if (j < r) continue;                                       // upper triangle (and j = -1: not in the sector)
@@ -472,13 +525,16 @@ __global__ void __launch_bounds__(kSBlock) sec_rows_kernel(SecDev S, const SecTe
 // upper-triangle filter, y[i] += x[j] * sqrt(nu_i/nu_j) * conj(c) * exp(2 pi i k.disp_i/L)), and consumed at once.  Zero-norm rows
 // carry fake_pos + i/dim on the diagonal (:1022-1025).  Nothing is stored: the sector's tables (keys, norms, sublattice tables)
 // are all that lives in HBM -- the reference's own answer to dimensions whose csr_mat does not fit.
-template <bool DOTS>
-__global__ void __launch_bounds__(kSBlock) sec_matfree_spmv_kernel(SecDev S, const SecTerms *Tp, const double2 *__restrict__ phase,
+// Blocks per SM pinned to what the 32-bit kernel has always reached (9 with the fused dots, 10 without): the launch sizes its
+// grid from the occupancy, and with the dots the grid fixes the order in which they are summed.
+template <class W, bool DOTS>
+__global__ void __launch_bounds__(kSBlock, DOTS ? 9 : 10) sec_matfree_spmv_kernel(SecDevT<W> S, const SecTerms *Tp, const double2 *__restrict__ phase,
                                                                    const double2 *__restrict__ x, const double2 *z, double2 *y,
                                                                    double2 alpha, double2 gamma, double2 beta, int scal_mode,
                                                                    const double *__restrict__ sc, double *dots_out, double *partials, unsigned *ticket)
 {
     using VT = VecTraits<double2>;
+    using P = typename W::P;
     __shared__ SecTerms T;
     for (int i = threadIdx.x; i < (int)(sizeof(SecTerms) / 4); i += blockDim.x) ((int *)&T)[i] = ((const int *)Tp)[i];
     __syncthreads();
@@ -501,16 +557,16 @@ __global__ void __launch_bounds__(kSBlock) sec_matfree_spmv_kernel(SecDev S, con
         } else {
             uint32_t a, b;
             sec_halves(S, S.keys[r], a, b);
-            const uint32_t s = spread_bits(a) | (spread_bits(b) << 1);
+            const P s = spin_zip<P>(a, b);
             double dg = 0.0;
             for (int t = 0; t < T.nterms; t++)
                 dg = __dadd_rn(dg, (((s >> T.p[t]) ^ (s >> T.q[t])) & 1u) ? -0.25 * T.J : 0.25 * T.J);
             mac(acc, dg, xi);
             for (int t = 0; t < T.nterms; t++) {
                 if (!(((s >> T.p[t]) ^ (s >> T.q[t])) & 1u)) continue;
-                const uint32_t s2 = s ^ ((1u << T.p[t]) | (1u << T.q[t]));
+                const P s2 = s ^ (((P)1 << T.p[t]) | ((P)1 << T.q[t]));
                 uint32_t ca = 0, cb = 0;
-                const int i = sec_canon(S, squeeze_bits(s2), squeeze_bits(s2 >> 1), ca, cb);
+                const int i = sec_canon(S, (uint32_t)squeeze_bits(s2), (uint32_t)squeeze_bits(s2 >> 1), ca, cb);
                 if (i < 0) continue;
                 const int64_t j = sec_lookup(S, sec_key(S, ca, cb));
                 if (j < 0) continue;                                   // not in the sector
@@ -545,7 +601,8 @@ __global__ void __launch_bounds__(kSBlock) sec_len_kernel(int64_t n, const int64
 // (S^z_q when c_r = exp(-i q.r)/sqrt(N)): only the momentum changes, the representative keeps its row index, and
 //   y[j] = sum_r  sqrt(nu_old[j] / nu_new[j]) * x[j] * (c_r * <state_j| S^z_r |state_j>)          (:1758-1761)
 // with rows skipped when |x[j]|, nu_old[j] or nu_new[j] is below lanczos_precision (:1752, :1760).
-__global__ void __launch_bounds__(kSBlock) sec_apply_sz_kernel(SecDev S, const double *__restrict__ nu_new, const double2 *__restrict__ coef,
+template <class W>
+__global__ void __launch_bounds__(kSBlock) sec_apply_sz_kernel(SecDevT<W> S, const double *__restrict__ nu_new, const double2 *__restrict__ coef,
                                                                const double2 *__restrict__ x, double2 *y)
 {
     __shared__ double2 c[kMaxTrans];
@@ -558,7 +615,7 @@ __global__ void __launch_bounds__(kSBlock) sec_apply_sz_kernel(SecDev S, const d
         if (hypot(xj.x, xj.y) >= 2e-12 && fabs(nj) >= 2e-12 && fabs(ni) > 2e-12) {
             uint32_t a, b;
             sec_halves(S, S.keys[r], a, b);
-            const uint32_t st = spread_bits(a) | (spread_bits(b) << 1);
+            const typename W::P st = spin_zip<typename W::P>(a, b);
             const double w = __dsqrt_rn(__ddiv_rn(nj, ni));
             const double2 t = make_double2(__dmul_rn(w, xj.x), __dmul_rn(w, xj.y));
             for (int site = 0; site < S.nsites; site++) {
@@ -580,7 +637,8 @@ __global__ void __launch_bounds__(kSBlock) sec_apply_sz_kernel(SecDev S, const d
 // (restated and pinned to the compiled reference in tests/repr_builders.py: apply_sminus).  Scatter with fp64 atomics:
 // the reference itself adds these contributions from several threads in no fixed order, so agreement is to rounding.
 // y must be zero on entry.
-__global__ void __launch_bounds__(kSBlock) sec_apply_ladder_kernel(SecDev So, SecDev Sn, const double2 *__restrict__ phase_new, const double2 *__restrict__ coef,
+template <class W>
+__global__ void __launch_bounds__(kSBlock) sec_apply_ladder_kernel(SecDevT<W> So, SecDevT<W> Sn, const double2 *__restrict__ phase_new, const double2 *__restrict__ coef,
                                                                    int lower, const double2 *__restrict__ x, double2 *y)
 {
     __shared__ double2 c[kMaxTrans];
@@ -590,15 +648,16 @@ __global__ void __launch_bounds__(kSBlock) sec_apply_ladder_kernel(SecDev So, Se
         const double2 xj = x[r];
         const double nj = So.nu[r];
         if (!(hypot(xj.x, xj.y) >= 2e-12) || !(nj >= 2e-12)) continue;                 // :1752
+        using P = typename W::P;
         uint32_t a, b;
         sec_halves(So, So.keys[r], a, b);
-        const uint32_t st = spread_bits(a) | (spread_bits(b) << 1);
+        const P st = spin_zip<P>(a, b);
         for (int site = 0; site < So.nsites; site++) {
-            const uint32_t bit = 1u << site;
+            const P bit = (P)1 << site;
             if (lower ? (st & bit) != 0u : (st & bit) == 0u) continue;                 // S^- needs an up spin (digit 0), S^+ a down spin
-            const uint32_t s2 = st ^ bit;
+            const P s2 = st ^ bit;
             uint32_t ca = 0, cb = 0;
-            const int i = sec_canon(Sn, squeeze_bits(s2), squeeze_bits(s2 >> 1), ca, cb);
+            const int i = sec_canon(Sn, (uint32_t)squeeze_bits(s2), (uint32_t)squeeze_bits(s2 >> 1), ca, cb);
             if (i < 0) continue;
             const int64_t tgt = sec_lookup(Sn, sec_key(Sn, ca, cb));
             if (tgt < 0) continue;
@@ -710,6 +769,8 @@ __global__ void __launch_bounds__(kSBlock) el_apply_gather_kernel(SecDev So, Sec
 static double wall_clock() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 struct FlagToInt { __host__ __device__ int operator()(uint8_t f) const { return (int)f; } };
 static int sgrid(int64_t n) { int64_t g = (n + kSBlock - 1) / kSBlock; if (g < 1) g = 1; if (g > 148 * 64) g = 148 * 64; return (int)g; }
+constexpr int64_t kChunkCand = 1ll << 30;   // candidates flagged per launch (one byte each); narrow sectors take one chunk
+static int g_sector_words = 0;              // qbgpu_debug_sector_words: 0 by size, 64 every spin sector wide
 
 }  // namespace qb
 
@@ -718,21 +779,29 @@ using namespace qb;
 struct qbgpu_sector {
     int dim = 0, L[3] = {1, 1, 1}, k[3] = {0, 0, 0}, spec = 0, nsites = 0, nsub = 0, ntrans = 0, nsubtrans = 0, ndown = 0;
     bool electron = false;                           // two bits per site (nup = ndown field, ndn below); nsub = bits of a half state
+    bool wide = false;                               // 32-bit halves, 64-bit states and keys: dev64 holds the tables, else dev
     int ndn = 0;
     uint16_t *d_invmask = nullptr;
     int64_t n = 0, zero_norm = 0;
     SecDev dev{};
-    uint16_t *d_subT = nullptr, *d_rep = nullptr;
+    SecDev64 dev64{};
+    void *d_subT = nullptr, *d_rep = nullptr, *d_keys = nullptr;
     uint8_t *d_dist = nullptr;
-    uint32_t *d_keys = nullptr, *d_seg = nullptr;
+    uint32_t *d_seg = nullptr;
     double *d_nu = nullptr;
     double2 *d_phase = nullptr;
     std::vector<std::complex<double>> phase;
     std::vector<std::vector<int>> disps;            // parent displacements, lexicographic
     std::vector<int> site_of_coor;                   // helper for bond generation / S^z_q phases
     std::vector<std::vector<int>> coor;
-    double enumerate_s = 0, norms_s = 0;
+    double enumerate_s = 0, norms_s = 0, lin_check_s = 0;
 };
+
+namespace qb {
+template <class W> SecDevT<W> &sec_dev(qbgpu_sector *S);
+template <> SecDev &sec_dev<Narrow>(qbgpu_sector *S) { return S->dev; }
+template <> SecDev64 &sec_dev<Wide>(qbgpu_sector *S) { return S->dev64; }
+}
 
 namespace {
 
@@ -768,7 +837,7 @@ struct HostLattice {
 };
 
 // does J = Ja[ia] + Jb[ib] have a solution?  (weighted union-find over the 2 * 2^nsub labels)
-bool lin_tables_exist(const std::vector<uint32_t> &keys, int nsub)
+template <class P> bool lin_tables_exist(const std::vector<P> &keys, int nsub)
 {
     const uint32_t half = 1u << nsub;
     std::vector<int32_t> parent(2 * half);
@@ -793,7 +862,9 @@ bool lin_tables_exist(const std::vector<uint32_t> &keys, int nsub)
 }
 
 struct SecMatFree {                      // what a matrix-free sector handle owns: the term list; everything else is the sector's
+    bool wide;
     SecDev dev;
+    SecDev64 dev64;
     SecTerms *d_T = nullptr;
     const double2 *phase = nullptr;
 };
@@ -807,26 +878,31 @@ void sector_free(qbgpu_sector *S)
 
 }  // namespace
 
-int qb::launch_spmv_sector_matfree(const qbgpu_matrix *A, const FusedArgs &a)
+template <class W> static int launch_sec_matfree(const SecDevT<W> &D, const SecMatFree *M, const FusedArgs &a)
 {
     Context &c = ctx();
-    const SecMatFree *M = (const SecMatFree *)A->mf_sec;
-    if (!A->api_complex) return fail(QBGPU_ERR_STATE, "matrix-free sector handle: complex vectors only");
-    auto kern = a.dots ? sec_matfree_spmv_kernel<true> : sec_matfree_spmv_kernel<false>;
+    auto kern = a.dots ? sec_matfree_spmv_kernel<W, true> : sec_matfree_spmv_kernel<W, false>;
     int blocks_per_sm = 0;
     QB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kern, kSBlock, 0));
     if (blocks_per_sm < 1) blocks_per_sm = 1;
-    const int64_t n = A->n;
+    const int64_t n = D.n;
     if (n == 0) return QBGPU_OK;
     int64_t want = (n + kSBlock - 1) / kSBlock;
     int64_t cap = (int64_t)c.num_sms * blocks_per_sm;
     if (cap > kMaxPartialBlocks) cap = kMaxPartialBlocks;
     const int grid = (int)(want < cap ? want : cap);
-    kern<<<grid, kSBlock, 0, c.stream>>>(M->dev, M->d_T, M->phase, (const double2 *)a.x, (const double2 *)a.z, (double2 *)a.y, a.alpha, a.gamma, a.beta,
+    kern<<<grid, kSBlock, 0, c.stream>>>(D, M->d_T, M->phase, (const double2 *)a.x, (const double2 *)a.z, (double2 *)a.y, a.alpha, a.gamma, a.beta,
                                          a.scal_mode, a.sc, a.dots, c.partials, c.ticket);
     QB_LAUNCH_COUNT();
     QB_CUDA(cudaGetLastError());
     return QBGPU_OK;
+}
+
+int qb::launch_spmv_sector_matfree(const qbgpu_matrix *A, const FusedArgs &a)
+{
+    const SecMatFree *M = (const SecMatFree *)A->mf_sec;
+    if (!A->api_complex) return fail(QBGPU_ERR_STATE, "matrix-free sector handle: complex vectors only");
+    return M->wide ? launch_sec_matfree<Wide>(M->dev64, M, a) : launch_sec_matfree<Narrow>(M->dev, M, a);
 }
 
 void qb::sector_matfree_destroy(qbgpu_matrix *A)
@@ -842,24 +918,20 @@ extern "C" {
 
 }  // extern "C"
 
-// spins (one bit per site, n0 = ndown) or single-orbital electrons (two bits per site, n0 = nup, n1 = ndn)
-static int sector_create_impl(qbgpu_sector_t *out, int dim, const int32_t *L, bool electron, int n0, int n1, const int32_t *k)
+// spins (one bit per site, n0 = ndown) or single-orbital electrons (two bits per site, n0 = nup, n1 = ndn); W: the word widths
+template <class W>
+static int sector_create_words(qbgpu_sector_t *out, int dim, const int32_t *L, bool electron, int n0, int n1, const int32_t *k, int spec, int N)
 {
-    QB_TRY(ensure_init());
+    using H = typename W::H;
+    using P = typename W::P;
     Context &c = ctx();
-    if (!out || !L || !k || dim < 1 || dim > 3) return fail(QBGPU_ERR_ARG, "sector_create: bad arguments");
-    *out = nullptr;
-    int spec = -1, N = 1;
-    for (int d = 0; d < dim; d++) { if (L[d] < 1) return fail(QBGPU_ERR_ARG, "sector_create: bad lattice size"); N *= L[d]; if (spec < 0 && L[d] % 2 == 0) spec = d; }
-    if (spec < 0) return fail(QBGPU_ERR_ARG, "sector_create: no even direction (the reference's divide_lattice needs one, src/lattice.cc:1076-1083)");
-    if (N > (electron ? 16 : 32) || N < 2) return fail(QBGPU_ERR_ARG, electron ? "sector_create: 2..16 sites for electrons" : "sector_create: 2..32 sites");
-    if (n0 < 0 || n0 > N || n1 < 0 || n1 > N) return fail(QBGPU_ERR_ARG, "sector_create: bad particle numbers");
     const int ndown = n0;
     const double t0 = wall_clock();
     auto *S = new qbgpu_sector;
     const int nhs = N / 2;                                              // sites of a half
     const int bps = electron ? 2 : 1;                                   // bits per site
     S->dim = dim; S->spec = spec; S->nsites = N; S->nsub = nhs * bps; S->ntrans = N; S->nsubtrans = N / 2; S->ndown = n0; S->ndn = n1; S->electron = electron;
+    S->wide = sizeof(P) == 8;
     for (int d = 0; d < dim; d++) { S->L[d] = L[d]; S->k[d] = k[d]; }
     HostLattice par(dim, S->L, spec);
     int Ls[3] = {S->L[0], S->L[1], S->L[2]};
@@ -872,23 +944,23 @@ static int sector_create_impl(qbgpu_sector_t *out, int dim, const int32_t *L, bo
     // sublattice translations of every half state, their representatives and distances
     std::vector<std::vector<int>> splans;
     for (auto &d : sub.disps) splans.push_back(sub.plan(d));
-    std::vector<uint16_t> subT((size_t)nst * half);
+    std::vector<H> subT((size_t)nst * half);
     const uint32_t dmask = (1u << bps) - 1u;
     for (int j = 0; j < nst; j++)
         for (uint32_t x = 0; x < half; x++) {
             uint32_t y = 0;
             for (int s = 0; s < nhs; s++) y |= ((x >> (bps * s)) & dmask) << (bps * splans[j][s]);
-            subT[(size_t)j * half + x] = (uint16_t)y;
+            subT[(size_t)j * half + x] = (H)y;
         }
-    std::vector<uint16_t> rep(half);
+    std::vector<H> rep(half);
     std::vector<uint8_t> dist(half), seen(half, 0);
-    std::vector<uint16_t> reps;
+    std::vector<H> reps;
     for (uint32_t x = 0; x < half; x++) {                               // src/basis.cc:1385-1419
         if (seen[x]) continue;
-        reps.push_back((uint16_t)x);
+        reps.push_back((H)x);
         for (int j = 0; j < nst; j++) {
             const uint32_t y = subT[(size_t)j * half + x];
-            if (!seen[y]) { seen[y] = 1; rep[y] = (uint16_t)x; dist[y] = (uint8_t)j; }
+            if (!seen[y]) { seen[y] = 1; rep[y] = (H)x; dist[y] = (uint8_t)j; }
         }
     }
     // each parent translation in terms of sublattice translations of the halves
@@ -906,7 +978,7 @@ static int sector_create_impl(qbgpu_sector_t *out, int dim, const int32_t *L, bo
         if (ia == sp_index.end() || ib == sp_index.end()) { sector_free(S); return fail(QBGPU_ERR_STATE, "sector_create: translation does not factor over the sublattices"); }
         fa[i] = ia->second; fb[i] = ib->second;
     }
-    SecDev &D = S->dev;
+    SecDevT<W> &D = sec_dev<W>(S);
     D.nsites = N; D.nsub = nsub; D.ntrans = N; D.shift = std::max(0, 2 * nsub - 16); D.lin_order = 1;
     D.electron = electron ? 1 : 0; D.invmask = nullptr;
     std::vector<uint16_t> invmask((size_t)N * 16, 0);
@@ -930,88 +1002,117 @@ static int sector_create_impl(qbgpu_sector_t *out, int dim, const int32_t *L, bo
         S->phase.push_back(std::exp(std::complex<double>(0.0, 2.0 * 3.1415926535897932 * e)));
     }
 
-    uint16_t *d_reps = nullptr;
+    H *d_reps = nullptr;
     uint8_t *d_flag = nullptr;
     void *d_tmp = nullptr;
     int *d_nsel = nullptr;
-    uint32_t *d_sorted = nullptr;
+    P *d_sorted = nullptr;
     unsigned long long *d_zero = nullptr;
     auto cleanup = [&]() { cudaFree(d_reps); cudaFree(d_flag); cudaFree(d_tmp); cudaFree(d_nsel); cudaFree(d_sorted); cudaFree(d_zero); };
 #define QB_CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { cleanup(); sector_free(S); return cuda_fail(e_, #call, __FILE__, __LINE__); } } while (0)
-    QB_CU(cudaMalloc(&S->d_subT, subT.size() * 2));
-    QB_CU(cudaMalloc(&S->d_rep, half * 2));
+    H *d_subT = nullptr, *d_rep = nullptr;
+    QB_CU(cudaMalloc(&d_subT, subT.size() * sizeof(H)));
+    S->d_subT = d_subT;
+    QB_CU(cudaMalloc(&d_rep, half * sizeof(H)));
+    S->d_rep = d_rep;
     QB_CU(cudaMalloc(&S->d_dist, half));
-    QB_CU(cudaMalloc(&d_reps, reps.size() * 2));
+    QB_CU(cudaMalloc(&d_reps, reps.size() * sizeof(H)));
     QB_CU(cudaMalloc(&S->d_phase, sizeof(double2) * N));
-    QB_CU(cudaMemcpyAsync(S->d_subT, subT.data(), subT.size() * 2, cudaMemcpyHostToDevice, c.stream));
-    QB_CU(cudaMemcpyAsync(S->d_rep, rep.data(), half * 2, cudaMemcpyHostToDevice, c.stream));
+    QB_CU(cudaMemcpyAsync(d_subT, subT.data(), subT.size() * sizeof(H), cudaMemcpyHostToDevice, c.stream));
+    QB_CU(cudaMemcpyAsync(d_rep, rep.data(), half * sizeof(H), cudaMemcpyHostToDevice, c.stream));
     QB_CU(cudaMemcpyAsync(S->d_dist, dist.data(), half, cudaMemcpyHostToDevice, c.stream));
-    QB_CU(cudaMemcpyAsync(d_reps, reps.data(), reps.size() * 2, cudaMemcpyHostToDevice, c.stream));
+    QB_CU(cudaMemcpyAsync(d_reps, reps.data(), reps.size() * sizeof(H), cudaMemcpyHostToDevice, c.stream));
     QB_CU(cudaMemcpyAsync(S->d_phase, S->phase.data(), sizeof(double2) * N, cudaMemcpyHostToDevice, c.stream));
     if (electron) {
         QB_CU(cudaMalloc(&S->d_invmask, invmask.size() * 2));
         QB_CU(cudaMemcpyAsync(S->d_invmask, invmask.data(), invmask.size() * 2, cudaMemcpyHostToDevice, c.stream));
         D.invmask = S->d_invmask;
     }
-    D.subT = S->d_subT; D.rep = S->d_rep; D.dist = S->d_dist;
+    D.subT = d_subT; D.rep = d_rep; D.dist = S->d_dist;
 
-    // representatives: flag the candidates (even half a sublattice representative), compact in Lin order
+    // representatives: flag the candidates (even half a sublattice representative), compact in Lin order.  Candidates go in
+    // chunks of whole odd-half ranges [b0, b1), ascending, so the selection stays in Lin order; with more than one chunk the
+    // chunks are flagged twice (once to size the key array, once to select), with one they are flagged once.
     const int nreps = (int)reps.size();
-    const int64_t ncand = (int64_t)nreps << nsub;
-    if (ncand > 2147483647LL) { cleanup(); sector_free(S); return fail(QBGPU_ERR_STATE, "sector_create: candidate count overflow"); }
-    QB_CU(cudaMalloc(&d_flag, ncand));
-    if (electron) el_flag_kernel<<<sgrid(ncand), kSBlock, 0, c.stream>>>(D, d_reps, nreps, n0, n1, ncand, d_flag);
-    else sec_flag_kernel<<<sgrid(ncand), kSBlock, 0, c.stream>>>(D, d_reps, nreps, ndown, ncand, d_flag);
-    QB_LAUNCH_COUNT();
-    QB_CU(cudaMalloc(&d_nsel, sizeof(int)));
-    uint32_t *d_all = nullptr;
+    const int64_t bstep = std::max<int64_t>(1, kChunkCand / nreps);
+    const int nchunks = (int)(((int64_t)half + bstep - 1) / bstep);
+    const int64_t chunk_cand = std::min<int64_t>(bstep, half) * nreps;
+    auto flag_chunk = [&](int q) {
+        const int64_t b0 = (int64_t)q * bstep, nc = (std::min<int64_t>(b0 + bstep, half) - b0) * nreps;
+        if (electron) el_flag_kernel<<<sgrid(nc), kSBlock, 0, c.stream>>>(sec_dev<Narrow>(S), (const uint16_t *)d_reps, nreps, n0, n1, b0 * nreps, nc, d_flag);
+        else sec_flag_kernel<W><<<sgrid(nc), kSBlock, 0, c.stream>>>(D, d_reps, nreps, ndown, b0 * nreps, nc, d_flag);
+        QB_LAUNCH_COUNT();
+        return nc;
+    };
+    QB_CU(cudaMalloc(&d_flag, chunk_cand));
+    QB_CU(cudaMalloc(&d_nsel, sizeof(int) * nchunks));
+    auto fit = thrust::make_transform_iterator((const uint8_t *)d_flag, FlagToInt());
+    thrust::counting_iterator<uint32_t> it(0u);
     {
-        // the sector size is not known before the selection: count first (a sum over the flags), then select
+        size_t tb = 0, tb2 = 0;                                         // temporary storage for the largest chunk
+        QB_CU(cub::DeviceReduce::Sum(nullptr, tb, fit, d_nsel, (int)chunk_cand, c.stream));
+        QB_CU(cub::DeviceSelect::Flagged(nullptr, tb2, it, d_flag, (P *)nullptr, d_nsel, (int)chunk_cand, c.stream));
+        QB_CU(cudaMalloc(&d_tmp, std::max<size_t>(std::max(tb, tb2), 1)));
+    }
+    // the sector size is not known before the selection: count first (a sum over the flags), then select
+    std::vector<int> cnt(nchunks);
+    for (int q = 0; q < nchunks; q++) {
+        const int64_t nc = flag_chunk(q);
         size_t tb = 0;
-        int *d_cnt = d_nsel;
-        auto fit = thrust::make_transform_iterator((const uint8_t *)d_flag, FlagToInt());
-        QB_CU(cub::DeviceReduce::Sum(nullptr, tb, fit, d_cnt, (int)ncand, c.stream));
-        QB_CU(cudaMalloc(&d_tmp, tb ? tb : 1));
-        QB_CU(cub::DeviceReduce::Sum(d_tmp, tb, fit, d_cnt, (int)ncand, c.stream));
-        int cnt = 0;
-        QB_CU(cudaMemcpyAsync(&cnt, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
-        QB_CU(cudaStreamSynchronize(c.stream));
-        cudaFree(d_tmp); d_tmp = nullptr;
-        if (cnt <= 0) { cleanup(); sector_free(S); return fail(QBGPU_ERR_ARG, "sector_create: empty sector"); }
-        S->n = cnt;
-        QB_CU(cudaMalloc(&d_all, sizeof(uint32_t) * (size_t)cnt));
-        S->d_keys = d_all;
-        thrust::counting_iterator<uint32_t> it(0u);
-        QB_CU(cub::DeviceSelect::Flagged(nullptr, tb, it, d_flag, d_all, d_nsel, (int)ncand, c.stream));
-        QB_CU(cudaMalloc(&d_tmp, tb ? tb : 1));
-        QB_CU(cub::DeviceSelect::Flagged(d_tmp, tb, it, d_flag, d_all, d_nsel, (int)ncand, c.stream));
-        sec_cand_to_key_kernel<<<sgrid(cnt), kSBlock, 0, c.stream>>>(cnt, d_reps, nreps, nsub, d_all);
+        QB_CU(cub::DeviceReduce::Sum(nullptr, tb, fit, d_nsel + q, (int)nc, c.stream));
+        QB_CU(cub::DeviceReduce::Sum(d_tmp, tb, fit, d_nsel + q, (int)nc, c.stream));
+    }
+    QB_CU(cudaMemcpyAsync(cnt.data(), d_nsel, sizeof(int) * nchunks, cudaMemcpyDeviceToHost, c.stream));
+    QB_CU(cudaStreamSynchronize(c.stream));
+    int64_t total = 0;
+    for (int q = 0; q < nchunks; q++) total += cnt[q];
+    if (total <= 0) { cleanup(); sector_free(S); return fail(QBGPU_ERR_ARG, "sector_create: empty sector"); }
+    if (total > 2147483647LL) { cleanup(); sector_free(S); return fail(QBGPU_ERR_STATE, "sector_create: more than 2^31 - 1 representatives"); }
+    S->n = total;
+    P *d_all = nullptr;
+    QB_CU(cudaMalloc(&d_all, sizeof(P) * (size_t)total));
+    S->d_keys = d_all;
+    for (int q = 0, off = 0; q < nchunks; off += cnt[q], q++) {
+        const int64_t nc = nchunks > 1 ? flag_chunk(q) : chunk_cand;
+        size_t tb = 0;
+        QB_CU(cub::DeviceSelect::Flagged(nullptr, tb, it, d_flag, d_all + off, d_nsel + q, (int)nc, c.stream));
+        QB_CU(cub::DeviceSelect::Flagged(d_tmp, tb, it, d_flag, d_all + off, d_nsel + q, (int)nc, c.stream));
+        sec_cand_to_key_kernel<W><<<sgrid(cnt[q]), kSBlock, 0, c.stream>>>(cnt[q], d_reps, nreps, nsub, (int64_t)q * bstep, d_all + off);
         QB_LAUNCH_COUNT();
     }
     // Lin tables or bisection order?  (decided on the host exactly like the reference's graph search would)
     {
-        std::vector<uint32_t> hk((size_t)S->n);
-        QB_CU(cudaMemcpyAsync(hk.data(), S->d_keys, sizeof(uint32_t) * hk.size(), cudaMemcpyDeviceToHost, c.stream));
+        std::vector<P> hk((size_t)S->n);
+        QB_CU(cudaMemcpyAsync(hk.data(), d_all, sizeof(P) * hk.size(), cudaMemcpyDeviceToHost, c.stream));
         QB_CU(cudaStreamSynchronize(c.stream));
+        const double tl = wall_clock();
         D.lin_order = lin_tables_exist(hk, nsub) ? 1 : 0;
+        S->lin_check_s = wall_clock() - tl;
     }
     if (!D.lin_order) {
-        if (electron) el_lin_to_zip_kernel<<<sgrid(S->n), kSBlock, 0, c.stream>>>(S->n, nsub, S->d_keys);
-        else sec_lin_to_zip_kernel<<<sgrid(S->n), kSBlock, 0, c.stream>>>(S->n, nsub, S->d_keys);
+        if (electron) el_lin_to_zip_kernel<<<sgrid(S->n), kSBlock, 0, c.stream>>>(S->n, nsub, (uint32_t *)d_all);
+        else sec_lin_to_zip_kernel<P><<<sgrid(S->n), kSBlock, 0, c.stream>>>(S->n, nsub, d_all);
         QB_LAUNCH_COUNT();
-        QB_CU(cudaMalloc(&d_sorted, sizeof(uint32_t) * (size_t)S->n));
+        QB_CU(cudaMalloc(&d_sorted, sizeof(P) * (size_t)S->n));
+        const int end_bit = S->wide ? 2 * nsub : 32;
         size_t tb = 0;
         cudaFree(d_tmp); d_tmp = nullptr;
-        QB_CU(cub::DeviceRadixSort::SortKeys(nullptr, tb, S->d_keys, d_sorted, (int)S->n, 0, 32, c.stream));
+        QB_CU(cub::DeviceRadixSort::SortKeys(nullptr, tb, d_all, d_sorted, (int)S->n, 0, end_bit, c.stream));
         QB_CU(cudaMalloc(&d_tmp, tb ? tb : 1));
-        QB_CU(cub::DeviceRadixSort::SortKeys(d_tmp, tb, S->d_keys, d_sorted, (int)S->n, 0, 32, c.stream));
+        QB_CU(cub::DeviceRadixSort::SortKeys(d_tmp, tb, d_all, d_sorted, (int)S->n, 0, end_bit, c.stream));
         QB_CU(cudaStreamSynchronize(c.stream));
-        std::swap(S->d_keys, d_sorted);
+        std::swap(d_all, d_sorted);
+        S->d_keys = d_all;
     }
-    D.keys = S->d_keys; D.n = S->n;
+    D.keys = d_all; D.n = S->n;
+    if (S->wide) {                                                      // about two keys per segment: a lookup is a couple of probes
+        int lg = 0;
+        while (((int64_t)1 << (lg + 1)) <= S->n) lg++;
+        D.shift = std::max(0, 2 * nsub - std::max(16, lg));
+    }
     const uint32_t nseg = 1u << (2 * nsub - D.shift);
     QB_CU(cudaMalloc(&S->d_seg, sizeof(uint32_t) * ((size_t)nseg + 1)));
-    sec_seg_kernel<<<sgrid(nseg + 1), kSBlock, 0, c.stream>>>(S->n, S->d_keys, D.shift, nseg, S->d_seg);
+    sec_seg_kernel<P><<<sgrid(nseg + 1), kSBlock, 0, c.stream>>>(S->n, d_all, D.shift, nseg, S->d_seg);
     QB_LAUNCH_COUNT();
     D.seg = S->d_seg;
     QB_CU(cudaStreamSynchronize(c.stream));
@@ -1021,8 +1122,8 @@ static int sector_create_impl(qbgpu_sector_t *out, int dim, const int32_t *L, bo
     QB_CU(cudaMalloc(&S->d_nu, sizeof(double) * (size_t)S->n));
     QB_CU(cudaMalloc(&d_zero, sizeof(unsigned long long)));
     QB_CU(cudaMemsetAsync(d_zero, 0, sizeof(unsigned long long), c.stream));
-    if (electron) el_norm_kernel<<<sgrid(S->n), kSBlock, 0, c.stream>>>(D, S->d_nu, d_zero);
-    else sec_norm_kernel<<<sgrid(S->n), kSBlock, 0, c.stream>>>(D, S->d_nu, d_zero);
+    if (electron) el_norm_kernel<<<sgrid(S->n), kSBlock, 0, c.stream>>>(sec_dev<Narrow>(S), S->d_nu, d_zero);
+    else sec_norm_kernel<W><<<sgrid(S->n), kSBlock, 0, c.stream>>>(D, S->d_nu, d_zero);
     QB_LAUNCH_COUNT();
     unsigned long long z = 0;
     QB_CU(cudaMemcpyAsync(&z, d_zero, sizeof(z), cudaMemcpyDeviceToHost, c.stream));
@@ -1035,6 +1136,23 @@ static int sector_create_impl(qbgpu_sector_t *out, int dim, const int32_t *L, bo
 #undef QB_CU
     *out = S;
     return QBGPU_OK;
+}
+
+// Spin sectors: 2..32 sites narrow, 34 and 36 sites wide (halves of at most 18 bits keep the sublattice tables in L2, about
+// 19 MB at 36 sites).  Electron sectors: 2..16 sites, narrow.
+static int sector_create_impl(qbgpu_sector_t *out, int dim, const int32_t *L, bool electron, int n0, int n1, const int32_t *k)
+{
+    QB_TRY(ensure_init());
+    if (!out || !L || !k || dim < 1 || dim > 3) return fail(QBGPU_ERR_ARG, "sector_create: bad arguments");
+    *out = nullptr;
+    int spec = -1, N = 1;
+    for (int d = 0; d < dim; d++) { if (L[d] < 1) return fail(QBGPU_ERR_ARG, "sector_create: bad lattice size"); N *= L[d]; if (spec < 0 && L[d] % 2 == 0) spec = d; }
+    if (spec < 0) return fail(QBGPU_ERR_ARG, "sector_create: no even direction (the reference's divide_lattice needs one, src/lattice.cc:1076-1083)");
+    if (N > (electron ? 16 : 36) || N < 2) return fail(QBGPU_ERR_ARG, electron ? "sector_create: 2..16 sites for electrons" : "sector_create: 2..36 sites");
+    if (n0 < 0 || n0 > N || n1 < 0 || n1 > N) return fail(QBGPU_ERR_ARG, "sector_create: bad particle numbers");
+    const bool wide = !electron && (N > 32 || g_sector_words == 64);
+    return wide ? sector_create_words<Wide>(out, dim, L, electron, n0, n1, k, spec, N)
+                : sector_create_words<Narrow>(out, dim, L, electron, n0, n1, k, spec, N);
 }
 
 extern "C" {
@@ -1053,23 +1171,53 @@ int qbgpu_sector_destroy(qbgpu_sector_t S) { sector_free(S); return QBGPU_OK; }
 int qbgpu_sector_get_info(qbgpu_sector_t S, qbgpu_sector_info *info)
 {
     if (!S || !info) return fail(QBGPU_ERR_ARG, "sector_get_info: null argument");
-    info->dim = S->n; info->zero_norm = S->zero_norm; info->nsites = S->nsites; info->lin_order = S->dev.lin_order;
+    info->dim = S->n; info->zero_norm = S->zero_norm; info->nsites = S->nsites; info->lin_order = S->wide ? S->dev64.lin_order : S->dev.lin_order;
     info->enumerate_seconds = S->enumerate_s; info->norms_seconds = S->norms_s;
+    info->lin_check_seconds = S->lin_check_s; info->state_bits = S->wide ? 64 : 32;
     return QBGPU_OK;
 }
+
+}  // extern "C"
+
+template <class W> static int sector_states_words(qbgpu_sector_t S, typename W::P *states_host)
+{
+    using P = typename W::P;
+    Context &c = ctx();
+    P *d = nullptr;
+    QB_CUDA(cudaMalloc(&d, sizeof(P) * (size_t)S->n));
+    sec_states_kernel<W><<<sgrid(S->n), kSBlock, 0, c.stream>>>(sec_dev<W>(S), d);
+    QB_LAUNCH_COUNT();
+    cudaError_t e = cudaMemcpyAsync(states_host, d, sizeof(P) * (size_t)S->n, cudaMemcpyDeviceToHost, c.stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c.stream);
+    cudaFree(d);
+    QB_CUDA(e);
+    return QBGPU_OK;
+}
+
+extern "C" {
 
 int qbgpu_sector_states(qbgpu_sector_t S, uint32_t *states_host)
 {
     if (!S || !states_host) return fail(QBGPU_ERR_ARG, "sector_states: null argument");
-    Context &c = ctx();
-    uint32_t *d = nullptr;
-    QB_CUDA(cudaMalloc(&d, sizeof(uint32_t) * (size_t)S->n));
-    sec_states_kernel<<<sgrid(S->n), kSBlock, 0, c.stream>>>(S->dev, d);
-    QB_LAUNCH_COUNT();
-    cudaError_t e = cudaMemcpyAsync(states_host, d, sizeof(uint32_t) * (size_t)S->n, cudaMemcpyDeviceToHost, c.stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c.stream);
-    cudaFree(d);
-    QB_CUDA(e);
+    if (S->wide) return fail(QBGPU_ERR_STATE, "sector_states: the states of this sector take 64 bits (qbgpu_sector_states64)");
+    return sector_states_words<Narrow>(S, states_host);
+}
+
+int qbgpu_sector_states64(qbgpu_sector_t S, uint64_t *states_host)
+{
+    if (!S || !states_host) return fail(QBGPU_ERR_ARG, "sector_states64: null argument");
+    if (S->wide) return sector_states_words<Wide>(S, states_host);
+    std::vector<uint32_t> s32((size_t)S->n);
+    const int rc = sector_states_words<Narrow>(S, s32.data());
+    if (rc != QBGPU_OK) return rc;
+    for (size_t i = 0; i < s32.size(); i++) states_host[i] = s32[i];
+    return QBGPU_OK;
+}
+
+int qbgpu_debug_sector_words(int bits)
+{
+    if (bits != 0 && bits != 64) return fail(QBGPU_ERR_ARG, "debug_sector_words: 0 (by size) or 64 (wide), not " + std::to_string(bits));
+    g_sector_words = bits;
     return QBGPU_OK;
 }
 
@@ -1087,14 +1235,16 @@ int qbgpu_sector_apply_sz(qbgpu_sector_t S_old, qbgpu_sector_t S_new, const doub
     if (!S_old || !S_new || !coef_reim || !x_old_dev || !y_new_dev) return fail(QBGPU_ERR_ARG, "sector_apply_sz: null argument");
     if (S_old->electron || S_new->electron) return fail(QBGPU_ERR_STATE, "sector_apply_sz: spin sectors only");
     if (S_old->n != S_new->n || S_old->nsites != S_new->nsites || S_old->ndown != S_new->ndown || S_old->dim != S_new->dim ||
-        memcmp(S_old->L, S_new->L, sizeof(S_old->L)) != 0 || S_old->dev.lin_order != S_new->dev.lin_order)
+        memcmp(S_old->L, S_new->L, sizeof(S_old->L)) != 0 || S_old->wide != S_new->wide ||
+        (S_old->wide ? S_old->dev64.lin_order != S_new->dev64.lin_order : S_old->dev.lin_order != S_new->dev.lin_order))
         return fail(QBGPU_ERR_ARG, "sector_apply_sz: the two sectors must share lattice and Sz (same representatives)");
     Context &c = ctx();
     double2 *d_coef = nullptr;
     QB_CUDA(cudaMalloc(&d_coef, sizeof(double2) * kMaxTrans));
     cudaError_t e = cudaMemcpyAsync(d_coef, coef_reim, sizeof(double2) * S_old->nsites, cudaMemcpyHostToDevice, c.stream);
     if (e == cudaSuccess) {
-        sec_apply_sz_kernel<<<sgrid(S_old->n), kSBlock, 0, c.stream>>>(S_old->dev, S_new->d_nu, d_coef, (const double2 *)x_old_dev, (double2 *)y_new_dev);
+        if (S_old->wide) sec_apply_sz_kernel<Wide><<<sgrid(S_old->n), kSBlock, 0, c.stream>>>(S_old->dev64, S_new->d_nu, d_coef, (const double2 *)x_old_dev, (double2 *)y_new_dev);
+        else sec_apply_sz_kernel<Narrow><<<sgrid(S_old->n), kSBlock, 0, c.stream>>>(S_old->dev, S_new->d_nu, d_coef, (const double2 *)x_old_dev, (double2 *)y_new_dev);
         QB_LAUNCH_COUNT();
         e = cudaStreamSynchronize(c.stream);
     }
@@ -1110,6 +1260,7 @@ int qbgpu_sector_apply_ladder(qbgpu_sector_t S_old, qbgpu_sector_t S_new, int lo
     if (S_old->electron || S_new->electron) return fail(QBGPU_ERR_STATE, "sector_apply_ladder: spin sectors only");
     if (S_old->nsites != S_new->nsites || S_old->dim != S_new->dim || memcmp(S_old->L, S_new->L, sizeof(S_old->L)) != 0)
         return fail(QBGPU_ERR_ARG, "sector_apply_ladder: the two sectors must share the lattice");
+    if (S_old->wide != S_new->wide) return fail(QBGPU_ERR_ARG, "sector_apply_ladder: the two sectors must have the same word width");
     if (S_new->ndown != S_old->ndown + (lower ? 1 : -1))
         return fail(QBGPU_ERR_ARG, "sector_apply_ladder: the target sector must have one more (S^-) or one fewer (S^+) down spin");
     Context &c = ctx();
@@ -1118,8 +1269,12 @@ int qbgpu_sector_apply_ladder(qbgpu_sector_t S_old, qbgpu_sector_t S_new, int lo
     cudaError_t e = cudaMemcpyAsync(d_coef, coef_reim, sizeof(double2) * S_old->nsites, cudaMemcpyHostToDevice, c.stream);
     if (e == cudaSuccess) e = cudaMemsetAsync(y_new_dev, 0, sizeof(double2) * (size_t)S_new->n, c.stream);
     if (e == cudaSuccess && S_old->n > 0) {
-        sec_apply_ladder_kernel<<<sgrid(S_old->n), kSBlock, 0, c.stream>>>(S_old->dev, S_new->dev, S_new->d_phase, d_coef, lower ? 1 : 0,
-                                                                            (const double2 *)x_old_dev, (double2 *)y_new_dev);
+        if (S_old->wide)
+            sec_apply_ladder_kernel<Wide><<<sgrid(S_old->n), kSBlock, 0, c.stream>>>(S_old->dev64, S_new->dev64, S_new->d_phase, d_coef, lower ? 1 : 0,
+                                                                                      (const double2 *)x_old_dev, (double2 *)y_new_dev);
+        else
+            sec_apply_ladder_kernel<Narrow><<<sgrid(S_old->n), kSBlock, 0, c.stream>>>(S_old->dev, S_new->dev, S_new->d_phase, d_coef, lower ? 1 : 0,
+                                                                                        (const double2 *)x_old_dev, (double2 *)y_new_dev);
         QB_LAUNCH_COUNT();
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(c.stream);
@@ -1234,7 +1389,8 @@ int qbgpu_sector_build_heisenberg(qbgpu_sector_t S, qbgpu_matrix_t *A, int nbond
     QB_CU(cudaMalloc(&d_cap, sizeof(int64_t) * (n + 1)));
     QB_CU(cudaMalloc(&d_start, sizeof(int64_t) * (n + 1)));
     QB_CU(cudaMalloc(&d_end, sizeof(int64_t) * (n + 1)));
-    sec_cap_kernel<<<sgrid(n + 1), kSBlock, 0, c.stream>>>(S->dev, d_T, d_cap);
+    if (S->wide) sec_cap_kernel<Wide><<<sgrid(n + 1), kSBlock, 0, c.stream>>>(S->dev64, d_T, d_cap);
+    else sec_cap_kernel<Narrow><<<sgrid(n + 1), kSBlock, 0, c.stream>>>(S->dev, d_T, d_cap);
     QB_LAUNCH_COUNT();
     size_t tb = 0;
     QB_CU(cub::DeviceScan::ExclusiveSum(nullptr, tb, d_cap, d_start, n + 1, c.stream));
@@ -1245,7 +1401,8 @@ int qbgpu_sector_build_heisenberg(qbgpu_sector_t S, qbgpu_matrix_t *A, int nbond
     QB_CU(cudaStreamSynchronize(c.stream));
     QB_CU(cudaMalloc(&d_col, sizeof(int64_t) * (size_t)total));
     QB_CU(cudaMalloc(&d_val, sizeof(double2) * (size_t)total));
-    sec_rows_kernel<<<sgrid(n), kSBlock, 0, c.stream>>>(S->dev, d_T, S->d_phase, d_start, d_end, d_col, d_val);
+    if (S->wide) sec_rows_kernel<Wide><<<sgrid(n), kSBlock, 0, c.stream>>>(S->dev64, d_T, S->d_phase, d_start, d_end, d_col, d_val);
+    else sec_rows_kernel<Narrow><<<sgrid(n), kSBlock, 0, c.stream>>>(S->dev, d_T, S->d_phase, d_start, d_end, d_col, d_val);
     QB_LAUNCH_COUNT();
     sec_len_kernel<<<sgrid(n), kSBlock, 0, c.stream>>>(n, d_start, d_end, d_cap);
     QB_LAUNCH_COUNT();
@@ -1289,7 +1446,7 @@ int qbgpu_sector_matfree_heisenberg(qbgpu_sector_t S, qbgpu_matrix_t *A, int nbo
     T.nterms = nbonds; T.J = J; T.fake_pos = fake_pos;
     for (int t = 0; t < nbonds; t++) { T.p[t] = (uint8_t)bs[t].first; T.q[t] = (uint8_t)bs[t].second; }
     auto *M = new SecMatFree;
-    M->dev = S->dev; M->phase = S->d_phase;
+    M->wide = S->wide; M->dev = S->dev; M->dev64 = S->dev64; M->phase = S->d_phase;
     if (cudaMalloc(&M->d_T, sizeof(SecTerms)) != cudaSuccess) { delete M; return cuda_fail(cudaGetLastError(), "cudaMalloc(terms)", __FILE__, __LINE__); }
     if (cudaMemcpyAsync(M->d_T, &T, sizeof(SecTerms), cudaMemcpyHostToDevice, c.stream) != cudaSuccess || cudaStreamSynchronize(c.stream) != cudaSuccess) {
         cudaFree(M->d_T); delete M; return cuda_fail(cudaGetLastError(), "upload(terms)", __FILE__, __LINE__);
