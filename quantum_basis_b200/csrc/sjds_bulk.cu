@@ -20,7 +20,10 @@
 //      is brought into shared memory by ONE bulk copy, the gathers become LDS.128 (a quarter-warp per wavefront, bank
 //      conflicts only), and the matrix stream keeps the register-fed path with many loads in flight.
 //
-// Both keep the arithmetic of sjds.cu: same entries, same order of accumulation per row (two alternating accumulators over
+//  (3) sjds_cross_slices_kernel -- the packed cross part of a species handle with fp64 vectors: one whole 32-row slice per
+//      warp item, register-fed, no ring; most slices are uniform (all rows of the same length) and pay no votes.
+//
+// All three keep the arithmetic of sjds.cu: same entries, same order of accumulation per row (two alternating accumulators over
 // the jagged diagonals), so products are bit-identical to spmv_sjds_kernel.
 #include "internal.hpp"
 #include <cstdlib>
@@ -396,14 +399,13 @@ static int launch_bulk_cfg(const qbgpu_matrix *A, const FusedArgs &a)
 // to L1, and L1 lines are what gathers in flight are tracked in: with fp64 vectors a fat ring (106 KB per CTA, two CTAs)
 // is best; with complex vectors (twice the lines per gather) a leaner one (profiles/r02_bulk_sweep_*.txt: 8,4,8 is 2x
 // slower than 8,3,6 there).  Packed words (4 bytes per entry, one bulk copy per segment) keep the segment length and with it
-// the gathers in flight, and take more, smaller stages (78 KB of ring per CTA with fp64 vectors instead of 106).  On BASELINE
-// config 3 the closing pass no longer follows the stream's bytes in flight: 8 x 8, 10 x 8 and 6 x 16 measured 6.77, 6.83
-// and 6.75 ms (y += H_cross x, fp64 vectors, one B200 at 1000 W).
+// the gathers in flight, and take more, smaller stages.  Packed parts with fp64 vectors take kernel (3) instead.
 template <typename ValT, typename VecT> struct BulkRing {
     static constexpr bool kPacked = std::is_same<ValT, uint32_t>::value, kCplx = sizeof(VecT) == 16;
+    static_assert(!kPacked || kCplx, "packed parts with fp64 vectors take sjds_cross_slices_kernel");
     static constexpr int NW = 8;
-    static constexpr int NST = kPacked ? (kCplx ? 6 : 8) : (kCplx ? 3 : 4);
-    static constexpr int KSEG = kPacked ? (kCplx ? 6 : 8) : (kCplx ? 6 : 8);
+    static constexpr int NST = kPacked ? 6 : (kCplx ? 3 : 4);
+    static constexpr int KSEG = kCplx ? 6 : 8;
 };
 
 template <typename ValT, typename VecT, bool DOTS, bool KEEP>
@@ -429,12 +431,200 @@ static int launch_bulk_typed(const qbgpu_matrix *A, const FusedArgs &a)
     return dots ? launch_bulk_ring<ValT, VecT, true, false>(A, a) : launch_bulk_ring<ValT, VecT, false, false>(A, a);
 }
 
+// ------------------------------------------------------------------- (3) slice-granular product of a packed cross part
+// The cross part of a species handle (hops of the up electrons, species.cu) has rows whose length is the up-hop count of
+// the row's up configuration: every 32-row slice that stays inside one block of D_dn rows is UNIFORM -- all 32 ranks have
+// the same length L, and entry (k, rank) sits at rowptr[32 s] + 32 k + rank.  Only slices that straddle two blocks (one in
+// about 400 on BASELINE config 3), the last partial slice and slices with empty rows are ragged.  So one warp takes one
+// traversal item of `order` -- a whole slice, in tile order as kernel (1) visits them -- and per trip of kXTrip diagonals
+// requests all the trip's entry words, then all its gathers of x, then accumulates.  A uniform slice pays no votes, no
+// per-segment headers and no shared-memory ring: its offsets are constants.  A ragged slice takes the same trips with a
+// per-lane predicate and the offsets of its diagonals counted by ballots (the layout of sjds.cu).
+// Same entries, same order of accumulation (diagonal k into accumulator k & 1, ascending k), same epilogue as kernel (1):
+// products, the fused way out and the running dots are bit-identical to it.
+//
+// Registers bound the trip: a word and a gathered double per diagonal in flight.  With a two-entry value table (the cross
+// part of a Hubbard model: +-t) the value is a select between two registers, and a trip keeps its codes as one bit each.
+constexpr int kXWarps = 8;              // warps per CTA: the block of the running dots' reduction tree, as in kernel (1)
+constexpr int kXTrip = 12;              // diagonals per trip (even: diagonal k + u accumulates into u & 1)
+constexpr int kXMinBlocks = 4;          // CTAs per SM the register budget is set for (64 registers a thread)
+// (BASELINE config 3, closing pass, one B200 at 1000 W: 12 diagonals at 4 CTAs per SM 6.08 ms, 16 at 3 CTAs 6.23 ms; an L2 bulk
+// prefetch of the next slice's words made both slower, 6.14 and 6.71 ms)
+// The order of the running dots depends on the grid (block_reduce_finalize): the DOTS pass keeps the grid of kernel (1)
+// with packed words -- two CTAs of 8 warps per SM -- so that Lanczos coefficients stay bit-identical.
+constexpr int kXDotsBlocksPerSm = 2;
+
+template <bool DOTS, bool KEEP, bool OUT, bool TWO>
+__global__ void __launch_bounds__(kXWarps * 32, DOTS ? kXDotsBlocksPerSm : kXMinBlocks)
+sjds_cross_slices_kernel(int64_t nslices, int64_t nrows, int64_t row_lo, const int64_t *__restrict__ rowptr,
+                         const uint32_t *__restrict__ rowinfo, const int32_t *__restrict__ words, const double *__restrict__ x,
+                         const double *z, double *y, double2 alpha, double2 gamma, double2 beta, int scal_mode,
+                         const double *__restrict__ sc, double *dots_out, double *partials, unsigned *ticket,
+                         const double *__restrict__ vdict, const int32_t *__restrict__ order, int cbits,
+                         const int32_t *__restrict__ perm_inv, double2 *y_ref, double2 out_alpha)
+{
+    static_assert(!OUT || !DOTS, "the fused way out serves the closing pass without dots");
+    using VT = VecTraits<double>;
+    __shared__ double sdict[TWO ? 1 : kPackedMaxTable];
+    if (!TWO) for (int i = threadIdx.x; i < (int)kPackedMaxTable; i += kXWarps * 32) sdict[i] = vdict[i];
+    __shared__ double2 s_scal[4];                          // [0] alpha, [1] gamma, [2] beta, [3].x the scale of the running dots
+    if (threadIdx.x == 0) {
+        double dot_scale = 1.0;
+        if (scal_mode != 0) {                              // Lanczos step a: 1 = first column block, 2 = a later one (sjds.cu)
+            const double sx = sc[0], sz = sc[1], bprev = sc[2];
+            alpha = make_double2(sx, 0.0);
+            gamma = make_double2(0.0, 0.0);
+            beta = scal_mode == 1 ? make_double2(-bprev * sz, 0.0) : make_double2(1.0, 0.0);
+            dot_scale = sx;
+        }
+        s_scal[0] = alpha; s_scal[1] = gamma; s_scal[2] = beta; s_scal[3] = make_double2(dot_scale, 0.0);
+    }
+    __syncthreads();
+    const bool use_gamma = (s_scal[1].x != 0.0 || s_scal[1].y != 0.0);
+    const bool use_beta = (s_scal[2].x != 0.0 || s_scal[2].y != 0.0);
+    const double v0 = TWO ? vdict[0] : 0.0, v1 = TWO ? vdict[1] : 0.0;
+    const uint32_t cmask = (1u << cbits) - 1u;
+    const uint64_t pol_s = pol_evict_first(), pol_x = pol_evict_last();
+    const int lane = threadIdx.x & 31;
+    double d[3] = {0.0, 0.0, 0.0};
+
+    // item `it` of this warp; the metadata of the next item and the slice of the one after are requested one item ahead
+    const int stride = (int)gridDim.x * kXWarps;           // (slice counts are < 2^31: rows < 2^31 by the int32 columns)
+    const int nsl = (int)nslices;
+    int it = (int)blockIdx.x * kXWarps + (int)(threadIdx.x >> 5);
+    auto slice_of = [&](int i) -> int { return i < nsl ? order[i] : 0; };
+    int s = slice_of(it);
+    uint32_t info = it < nsl ? rowinfo[(int64_t)s * 32 + lane] : 0u;
+    int64_t base = it < nsl ? rowptr[(int64_t)s * 32] : 0;
+    int s_next = slice_of(it + stride);
+
+#pragma unroll 1
+    for (; it < nsl; it += stride) {
+        const bool more = it + stride < nsl;
+        const uint32_t info_n = more ? rowinfo[(int64_t)s_next * 32 + lane] : 0u;
+        const int64_t base_n = more ? rowptr[(int64_t)s_next * 32] : 0;
+        const int s_after = slice_of(it + 2 * stride);
+
+        const int len = (int)(info & kLenMaskB);
+        const int maxlen = __shfl_sync(0xffffffffu, len, 0);
+        const int minlen = __shfl_sync(0xffffffffu, len, 31);
+        const int64_t row = (int64_t)s * 32 + (info >> 24);
+        const bool live = row < nrows && !(KEEP && !OUT && len == 0);      // padding ranks of the last slice point past the last row
+        double zv = 0.0, xi = 0.0;
+        int32_t rref = 0;
+        if (live) {                                        // the epilogue's operands, requested before the entries
+            if (use_beta) zv = z[row];
+            if (use_gamma || DOTS) xi = x[row_lo + row];
+            if constexpr (OUT) rref = perm_inv[row_lo + row];
+        }
+        double acc0 = 0.0, acc1 = 0.0;
+        const int32_t *wb = words + base + lane;
+        // diagonals [k, k + kXTrip): a uniform trip has the first `rem` of them on every lane at 32 (k + u) + lane; a ragged
+        // one has diagonal k + u where k + u < len, at the entries of the slice before it (`off`, counted by ballots) + lane
+        auto trip = [&](auto ragged, int k, int rem, int &off) {
+            constexpr bool RG = decltype(ragged)::value;
+            uint32_t w[kXTrip];                            // (set on every path: a value left over from the previous trip
+#pragma unroll                                         //  would stay live across it)
+            for (int u = 0; u < kXTrip; u++) {
+                bool a;
+                int o;
+                if constexpr (RG) { a = k + u < len; o = off; off += __popc(__ballot_sync(0xffffffffu, a)); }
+                else { a = u < rem; o = (k + u) * 32; }
+                w[u] = a ? (uint32_t)lds_i32(wb + o, pol_s) : 0u;
+            }
+            double xv[kXTrip];
+            uint32_t codes = 0;
+#pragma unroll
+            for (int u = 0; u < kXTrip; u++) {
+                xv[u] = 0.0;
+                if (RG ? k + u < len : u < rem) {
+                    xv[u] = ldx_hint(x + (w[u] & cmask), pol_x);
+                    if (TWO) codes |= (w[u] >> cbits) << u;
+                }
+            }
+#pragma unroll
+            for (int u = 0; u < kXTrip; u++) {
+                if (RG ? k + u < len : u < rem) {
+                    const double v = TWO ? (((codes >> u) & 1u) ? v1 : v0) : sdict[w[u] >> cbits];
+                    if (u & 1) mac(acc1, v, xv[u]); else mac(acc0, v, xv[u]);
+                }
+            }
+        };
+        int off = 0;
+        if (maxlen == minlen) {
+#pragma unroll 1
+            for (int k = 0; k < len; k += kXTrip) trip(std::false_type{}, k, min(kXTrip, len - k), off);
+        } else {
+#pragma unroll 1
+            for (int k = 0; k < maxlen; k += kXTrip) trip(std::true_type{}, k, 0, off);
+        }
+        if (live) {
+            const double acc = VT::add(acc0, acc1);
+            double out = VT::scale(s_scal[0], acc);
+            if (use_gamma) out = VT::add(out, VT::scale(s_scal[1], xi));
+            if (use_beta) out = VT::add(out, VT::scale(s_scal[2], zv));
+            if constexpr (OUT) y_ref[rref] = make_double2(out_alpha.x * out, out_alpha.y * out);
+            else y[row] = out;
+            if (DOTS) {
+                const double2 p = VT::conj_mul(xi, out);
+                d[0] += p.x; d[1] += p.y; d[2] += VT::abs2(out);
+            }
+        }
+        s = s_next; info = info_n; base = base_n; s_next = s_after;
+    }
+    if (DOTS) {
+        d[0] *= s_scal[3].x; d[1] *= s_scal[3].x;
+        block_reduce_finalize<3, kXWarps * 32>(d, partials, ticket, dots_out);
+    }
+}
+
+template <bool DOTS, bool KEEP, bool OUT, bool TWO>
+static int launch_cross_slices_cfg(const qbgpu_matrix *A, const FusedArgs &a)
+{
+    Context &c = ctx();
+    auto kern = sjds_cross_slices_kernel<DOTS, KEEP, OUT, TWO>;
+    static int blocks_per_sm = 0;
+    if (blocks_per_sm == 0) {
+        QB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kern, kXWarps * 32, 0));
+        if (blocks_per_sm < 1) return fail(QBGPU_ERR_STATE, "slice-granular cross pass: no CTA fits on an SM");
+        if (DOTS && blocks_per_sm > kXDotsBlocksPerSm) blocks_per_sm = kXDotsBlocksPerSm;
+    }
+    const int64_t nrows = A->nrows();
+    if (nrows == 0) return QBGPU_OK;
+    const int64_t nslices = (nrows + 31) / 32;
+    const int64_t want = (nslices + kXWarps - 1) / kXWarps;
+    int64_t cap = (int64_t)c.num_sms * blocks_per_sm;
+    if (cap > kMaxPartialBlocks) cap = kMaxPartialBlocks;
+    const int grid = (int)(want < cap ? want : cap);
+    kern<<<grid, kXWarps * 32, 0, c.stream>>>(nslices, nrows, A->row_lo, A->rowptr, A->rowinfo, A->col, (const double *)a.x,
+                                              (const double *)a.z, (double *)a.y, a.alpha, a.gamma, a.beta, a.scal_mode, a.sc,
+                                              a.dots, c.partials, c.ticket, A->vdict, A->slice_order, A->cbits,
+                                              OUT ? a.perm_inv : nullptr, OUT ? (double2 *)a.y_ref : nullptr, a.out_alpha);
+    QB_LAUNCH_COUNT();
+    QB_CUDA(cudaGetLastError());
+    return QBGPU_OK;
+}
+
+template <bool TWO>
+static int launch_cross_slices_typed(const qbgpu_matrix *A, const FusedArgs &a)
+{
+    const bool dots = a.dots != nullptr;
+    const bool keep = !dots && a.scal_mode == 0 && a.z == a.y && a.beta.x == 1.0 && a.beta.y == 0.0 && a.gamma.x == 0.0 && a.gamma.y == 0.0;
+    if (a.y_ref) {                                          // the closing pass of a species product writes the reference's order
+        if (keep && a.perm_inv) return launch_cross_slices_cfg<false, true, true, TWO>(A, a);
+        return fail(QBGPU_ERR_STATE, "fused way out: not the closing pass of a species handle (internal)");
+    }
+    if (keep) return launch_cross_slices_cfg<false, true, false, TWO>(A, a);
+    return dots ? launch_cross_slices_cfg<true, false, false, TWO>(A, a) : launch_cross_slices_cfg<false, false, false, TWO>(A, a);
+}
+
 // entry: tile-ordered sliced-jagged handle (slice_order set), not a ring view.  The bulk copies may read up to 15 bytes
 // before/after a slice's range inside col[] / val[]: always inside the arrays except at their very ends, where the
-// allocations keep 64 bytes of slack.
+// allocations keep 64 bytes of slack.  Packed parts with fp64 vectors take the slice-granular kernel (3).
 int launch_spmv_sjds_bulk(const qbgpu_matrix *A, const FusedArgs &a)
 {
-    if (A->cbits) return A->api_complex ? launch_bulk_typed<uint32_t, double2>(A, a) : launch_bulk_typed<uint32_t, double>(A, a);
+    if (A->cbits && !A->api_complex) return A->ndict == 2 ? launch_cross_slices_typed<true>(A, a) : launch_cross_slices_typed<false>(A, a);
+    if (A->cbits) return launch_bulk_typed<uint32_t, double2>(A, a);
     if (A->ndict) return fail(QBGPU_ERR_STATE, "bulk-streamed product: 1-byte dictionary codes are not supported (internal)");
     if (!A->api_complex) return launch_bulk_typed<double, double>(A, a);
     if (A->val_real) return launch_bulk_typed<double, double2>(A, a);
